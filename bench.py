@@ -413,6 +413,9 @@ def run_ours(args):
                 bld_p = out_p = None
         gather["headline_transport"] = transport
     t1 = time.perf_counter()
+    if args.dump_outputs and rank == 0:
+        headline_out = out_p if gather is not None and gather["headline_transport"] == "p2p" else out
+        dump_cache_sample(args.dump_outputs, headline_out, plan)
     value = F_total / (ms_per_step * 1e-3)
     kernel_only = {"value": F_total / (ko_ms * 1e-3), "unit": "frames/s", "ms_per_step": ko_ms,
                    "note": "no gather: each data-parallel rank keeps its shard resident (ResidentCache)"}
@@ -587,6 +590,23 @@ def run_ours(args):
         dist.barrier()
         dist.destroy_process_group()
     return 0
+
+
+DUMP_UTTS = 64
+
+
+def dump_cache_sample(out_dir, cache, plan):
+    """Writes ``out_dir/logmel.npy``: the log-mel rows (float32 [rows, 80], corpus order) of DUMP_UTTS utterances drawn
+    with a fixed seed from the cache the timed steps built.  The whole cache (~2 GB for cfg4) is too large to keep; the
+    sample (<= 18 MB) lets two builds of the project be compared output for output on identical inputs."""
+    import torch
+    from spev_tts_b200.cache import GatheredCache
+    n = len(plan.frames)
+    utts = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_UTTS), replace=False))
+    gc = GatheredCache(cache, plan)
+    rows = torch.cat([gc.utterance(int(u)) for u in utts]).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logmel.npy"), rows.astype(np.float32, copy=False))
 
 
 def measure_pcie(dev, host_in, host_out):
@@ -1146,7 +1166,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-gl", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of the log-mel cache they built to DIR/logmel.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)
