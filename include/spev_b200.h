@@ -194,8 +194,9 @@ SPEV_API int spev_gl_phase_update(spev_ctx* ctx, const spev_batch* batch, const 
                          int has_prev, void* stream);
 
 /* Full Griffin-Lim: ang0 = S*exp(i*phase); n_iter x (istft, stft + phase update); final istft -- executed as
- * istft once, then n_iter x (fused stft + phase update + inverse transform, pair overlap-add): see
- * spev_set_griffinlim_variant.
+ * istft once, then n_iter x (fused stft + phase update + inverse transform of the new spectra, pair overlap-add).
+ * Same arithmetic per frame as spev_istft / spev_gl_phase_update, except that the phase normalisation uses a 2-ulp
+ * rsqrt and the <= 4 overlap-add terms of a sample are summed pair by pair: agrees with those entry points to rounding.
  *   init_phase : dev float32 [n_frames, 513] radians, or NULL -> 2*pi*U[0,1) from `seed`
  *   y          : dev float32 [256*(n_frames - n_items)]
  *   workspace  : dev, >= spev_griffinlim_workspace_bytes(n_frames)
@@ -263,21 +264,6 @@ SPEV_API int spev_copy_segments_piece_bytes(void);
 SPEV_API int spev_copy_segments(const void* src, void* dst, const int64_t* src_off, const int64_t* dst_off,
                                 const int64_t* nbytes, const int64_t* piece_off, int n_segments, int64_t n_pieces,
                                 void* stream);
-
-/* A/B switch of the fused log-mel kernel: 0 (default) = the tile kernel with three CTA barriers per tile (k_stft_mel<0>);
- * 1 = decoupled warps with split-phase mbarrier synchronisation (k_stft_mel_ws; measured slower, DESIGN.md section 4).
- * Results are bit-identical. */
-SPEV_API int spev_set_logmel_variant(spev_ctx* ctx, int variant);
-/* A/B switch of the Griffin-Lim kernels (bit mask): 0 = the round-1 kernels; 1 = warp-independent phase update with
- * bulk-staged (cp.async.bulk) tprev / spectrum rows; | 2 = dynamic tile tickets in the ISTFT; | 4 = dynamic pair tickets
- * in the phase update (taken automatically for batches of >= 8 frame tiles per SM); | 8 = FUSED iteration: the phase
- * update inverse-transforms the new spectra in registers and writes pair overlap-add segments (k_gl_fused), a streaming
- * kernel finishes the overlap-add (k_ola_pairs) -- the spectra never travel through HBM; | 16 = rsqrt phase
- * normalisation in the fused kernel (2 ulp instead of IEEE sqrt + divide); | 32 = straight-line fused body (A/B of the
- * rolled two-pass body); | 64 = L2 eviction hints in the fused kernels (the momentum spectra stream through
- * evict-first, S / pair segments / y are kept evict-last).  Default 89 = 1 | 8 | 16 | 64.  Variants 0..7 are bit-identical to each other; the fused ones add
- * the <= 4 overlap-add terms in pair order and agree with them to rounding (tests/test_gpu_griffinlim.py). */
-SPEV_API int spev_set_griffinlim_variant(spev_ctx* ctx, int variant);
 
 /* Cap the number of CTAs the persistent FFT kernels launch (default: one per SM).  A multi-GPU cache build that
  * overlaps the NCCL gather of finished chunks with the kernel of the next chunk leaves a few SMs to NCCL's

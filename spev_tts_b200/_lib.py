@@ -93,8 +93,6 @@ _SIGS = {
     "spev_copy_segments": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                      C.c_int64, C.c_void_p]),
     "spev_set_sm_limit": (C.c_int, [C.c_void_p, C.c_int]),
-    "spev_set_logmel_variant": (C.c_int, [C.c_void_p, C.c_int]),
-    "spev_set_griffinlim_variant": (C.c_int, [C.c_void_p, C.c_int]),
     "spev_lr_plan": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                C.c_void_p, C.c_void_p, C.c_void_p]),
     "spev_lr_expand": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
@@ -129,9 +127,6 @@ _SIGS = {
 }
 
 EXPORTED_SYMBOLS = tuple(sorted(_SIGS))
-
-# spev_set_griffinlim_variant: the library default (bulk-staged rows | fused iteration | rsqrt phase normalisation | L2 hints)
-GL_VARIANT_DEFAULT = 89
 
 _lib = None
 _lock = threading.Lock()

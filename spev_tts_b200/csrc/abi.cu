@@ -35,7 +35,7 @@ int launch_stft_mel(spev_ctx*, const spev_batch*, const float*, float*, bool, in
 int launch_stft_phase(spev_ctx*, const spev_batch*, const float*, const float*, int64_t, void*, void*, int64_t, float, int, bool, cudaStream_t,
                       unsigned* counter = nullptr, unsigned base = 0, bool fuse = false);
 int launch_ola_pairs(spev_ctx*, const spev_batch*, const void*, int64_t, float*, cudaStream_t);
-int launch_istft(spev_ctx*, const spev_batch*, const void*, int64_t, float*, cudaStream_t, unsigned* counter = nullptr, unsigned base = 0);
+int launch_istft(spev_ctx*, const spev_batch*, const void*, int64_t, float*, cudaStream_t);
 int fft_grid(const spev_ctx*, int64_t);
 int launch_nnls_objective(spev_ctx*, const void*, int, int64_t, const float*, int, int, int64_t, int64_t, int, int, double*, double*, double*, cudaStream_t);
 int spectral_init(spev_ctx*);
@@ -223,7 +223,7 @@ int spev_create(spev_ctx** out, int device, int sr, int n_fft, int hop, int win,
 
     spev_ctx* c = new spev_ctx();
     c->device = device; c->sr = sr; c->n_fft = n_fft; c->hop = hop; c->win = kNfft; c->n_mels = n_mels;
-    c->fmin = fmin; c->fmax = fmax; c->num_sms = c->num_sms_device = prop.multiProcessorCount; c->tma = nullptr; c->use_tc = 1; c->k1_variant = 0; c->gl_variant = 89;
+    c->fmin = fmin; c->fmax = fmax; c->num_sms = c->num_sms_device = prop.multiProcessorCount; c->tma = nullptr; c->use_tc = 1;
     c->d_tw = nullptr; c->d_window = nullptr; c->d_win2048 = nullptr; c->d_tw2048 = nullptr; c->d_basis = c->d_basis_pad = c->d_basis_hi = c->d_basis_lo = nullptr; c->d_nnls_rng = nullptr;
     c->d_pinv_t = c->d_pinv_hi = c->d_pinv_lo = nullptr;
     c->d_prog_w = nullptr; c->d_prog_h = nullptr;
@@ -398,23 +398,6 @@ int spev_set_tensor_core(spev_ctx* c, int enable) {
     return SPEV_OK;
 }
 
-int spev_set_griffinlim_variant(spev_ctx* c, int variant) {
-    SPEV_REQUIRE(c, SPEV_E_INVALID, "ctx is null");
-    SPEV_REQUIRE(variant >= 0 && variant <= 127 && (variant == 0 || (variant & 1)), SPEV_E_INVALID,
-                 "spev_set_griffinlim_variant: 0 (r01 kernels) or 1 (bulk-staged rows) | 2 (dynamic ISTFT tiles) | 4 (dynamic phase-update pairs) "
-                 "| 8 (fused iteration: inverse transform inside the phase update + pair overlap-add; default 89 = 1 | 8 | 16 | 64) | 16 (rsqrt phase normalisation in the fused kernel) "
-                 "| 32 (straight-line fused body) | 64 (L2 eviction hints: momentum spectra stream, S / segments / y stay)");
-    c->gl_variant = variant;
-    return SPEV_OK;
-}
-
-int spev_set_logmel_variant(spev_ctx* c, int variant) {
-    SPEV_REQUIRE(c, SPEV_E_INVALID, "ctx is null");
-    SPEV_REQUIRE(variant == 0 || variant == 1, SPEV_E_INVALID, "spev_set_logmel_variant: 0 (tile lock-step) or 1 (decoupled warps)");
-    c->k1_variant = variant;
-    return SPEV_OK;
-}
-
 int spev_tile_frames(void) { return kTileFrames; }
 int spev_tile_chunks(void) { return kTileChunks; }
 
@@ -542,36 +525,27 @@ int spev_griffinlim(spev_ctx* c, const spev_batch* b, const float* S, int64_t ld
     uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~static_cast<uintptr_t>(255);
     float2* ang = reinterpret_cast<float2*>(base);
     float2* tprev = ang + b->n_frames * kSpecLd;
-    // ticket counters of the dynamic tile scheduler: [0] ISTFT tiles, [32] phase-update pairs (separate cache lines);
-    // they only grow during a call -- launch j starts at base j * (work + workers), see draw_ticket()
+    // ticket counter of the dynamic pair scheduler: word 32 of the 256-byte counter block (a cache line of its own);
+    // it only grows during a call -- launch j starts at base j * (work + workers), see draw_ticket()
     unsigned* counters = reinterpret_cast<unsigned*>(tprev + b->n_frames * kSpecLd);
     SPEV_CUDA(cudaMemsetAsync(counters, 0, 256, st));
-    const unsigned per_istft = static_cast<unsigned>(b->n_ctiles + fft_grid(c, b->n_ctiles));
     const unsigned per_phase = static_cast<unsigned>(static_cast<int64_t>(b->n_ftiles) * kWarps +
                                                      static_cast<int64_t>(fft_grid(c, b->n_ftiles)) * kWarps);
     // librosa: (momentum / (1 + momentum)) is a Python float applied to a complex64 array
     const float alpha = static_cast<float>(static_cast<double>(momentum) / (1.0 + static_cast<double>(momentum)));
     int rc = SPEV_OK;
     if ((rc = launch_gl_init(c, S, ld_s, init_phase, seed, ang, kSpecLd, b->n_frames, st))) return rc;
-    if ((c->gl_variant & 8) && c->gl_variant != 0) {
-        // Fused iteration (r02 default): y = istft(ang) once, then n_iter x { STFT + phase update + inverse transform of
-        // the new spectra in registers -> pair segments (in the `ang` buffer, which nothing else reads any more);
-        // overlap-add of the segments -> y }.  The new spectra never travel through HBM: 17.3 instead of 20.5 KB per
-        // frame and iteration, every FFT in the barrier-free warp-independent kernel, no halo recomputation.
-        if ((rc = launch_istft(c, b, ang, kSpecLd, y, st, counters, 0))) return rc;
-        for (int it = 0; it < n_iter; ++it) {
-            if ((rc = launch_stft_phase(c, b, y, S, ld_s, ang, tprev, kSpecLd, alpha, it > 0, true, st, counters + 32,
-                                        per_phase * static_cast<unsigned>(it), true))) return rc;
-            if ((rc = launch_ola_pairs(c, b, ang, kSpecLd, y, st))) return rc;
-        }
-        return SPEV_OK;
-    }
+    // Fused iteration: y = istft(ang) once, then n_iter x { STFT + phase update + inverse transform of the new spectra
+    // in registers -> pair segments (in the `ang` buffer, which nothing else reads any more); overlap-add of the
+    // segments -> y }.  The new spectra never travel through HBM: 17.3 instead of 20.5 KB per frame and iteration,
+    // every FFT in the barrier-free warp-independent kernel, no halo recomputation.
+    if ((rc = launch_istft(c, b, ang, kSpecLd, y, st))) return rc;
     for (int it = 0; it < n_iter; ++it) {
-        if ((rc = launch_istft(c, b, ang, kSpecLd, y, st, counters, per_istft * static_cast<unsigned>(it)))) return rc;
         if ((rc = launch_stft_phase(c, b, y, S, ld_s, ang, tprev, kSpecLd, alpha, it > 0, true, st, counters + 32,
-                                    per_phase * static_cast<unsigned>(it)))) return rc;
+                                    per_phase * static_cast<unsigned>(it), true))) return rc;
+        if ((rc = launch_ola_pairs(c, b, ang, kSpecLd, y, st))) return rc;
     }
-    return launch_istft(c, b, ang, kSpecLd, y, st, counters, per_istft * static_cast<unsigned>(n_iter));
+    return SPEV_OK;
 }
 
 int spev_frame_features(spev_ctx* c, const spev_batch* b, const float* samples, float* rms, float* centroid, void* stream) {

@@ -901,8 +901,7 @@ int spev_pyin_cmnd(spev_pyin* c, const spev_batch* b, const float* samples, floa
         const int L8 = 8 * octets, need = c->win_length + L8, zmax = (kCmndGroup - 1) * kHop + need, nplane = (zmax + 7) / 8 + 4;
         const size_t smem = sizeof(float) * (((zmax + 3) & ~3) + 4 * (2 * nplane + 4) + (2 * kCmndGroup + 6) * L8 +
                                              kCmndGroup * (need + 1) + 8);
-        static const bool use_shared = std::getenv("SPEV_PYIN_CMND_PER_FRAME") == nullptr;
-        if (use_shared && c->win_length == 1024 && c->frame_length == 2048 && smem <= 232448) {
+        if (c->win_length == 1024 && c->frame_length == 2048 && smem <= 232448) {
             const int64_t groups = static_cast<int64_t>(b->n_ftiles) * ((kTileFrames + kCmndGroup - 1) / kCmndGroup);
             SPEV_CUDA(cudaFuncSetAttribute(k_yin_cmnd_shared, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
             k_yin_cmnd_shared<<<static_cast<int>(std::min<int64_t>(groups, 148 * 32)), kCmndThreads, smem, static_cast<cudaStream_t>(stream)>>>(

@@ -8,26 +8,26 @@
 //                   gather overlap-add (each output sample owner sums its <= 4 frames in
 //                   ascending frame order, no atomics) fused with window-sum-square
 //                   normalisation.            Replaces librosa.istft under :730-733.
-// K5 k_stft_phase : STFT of the rebuilt signal fused with Griffin-Lim's momentum / phase
-//                   normalisation update.     Replaces librosa.stft + the angle update lines of
-//                   librosa.griffinlim under :730-733.
+// K5 k_stft_phase_w : STFT of the rebuilt signal fused with Griffin-Lim's momentum / phase
+//                   normalisation update, one frame pair per warp.  Replaces librosa.stft + the angle
+//                   update lines of librosa.griffinlim under :730-733.
 // K5f k_gl_fused  : the Griffin-Lim ITERATION as the driver runs it (round 2): STFT + phase update + inverse transform of
 //                   the new spectra in registers; leaves one overlap-add segment per frame pair.  K4p k_ola_pairs sums the
 //                   segments into y.  (K4 / K5 above stay the stand-alone spev_istft / spev_stft / spev_gl_phase_update.)
 // K3 k_mel_to_mag : S = sqrt(max(pinv . exp(logmel), 0)) (FFMA version; the tcgen05 version
 //                   lives in gemm_tc.cu).     Replaces librosa mel_to_stft under :730.
 //
-// All three FFT kernels are persistent (grid = #SMs, one 16-warp CTA per SM, static round-robin
-// over host-built 48-byte tile descriptors).  Nothing on the per-tile critical path waits on
+// All FFT kernels are persistent (grid = #SMs, one 16-warp CTA per SM).  K1 and K4 go round-robin
+// over host-built 48-byte tile descriptors, and nothing on their per-tile critical path waits on
 // global memory: tile descriptors travel through a 4-slot cp.async ring three tiles ahead, and
 // the samples of tile i+1 are cp.async-staged into the second half of a double buffer while
-// tile i is transformed.
+// tile i is transformed.  K5 and K5f hand out frame pairs to warps instead (see k_stft_phase_w).
 //
-// Shared-memory plan per CTA:
+// Shared-memory plan per CTA (K1 / K4):
 //   s_tw    float2[32*32]   inter-stage twiddles                       8,192 B
 //   s_win   float [1024]    periodic Hann                              4,096 B
 //   s_ring  spev_tile[4]    descriptor ring                              192 B
-//   s_stage float [2][8960] double-buffered tile samples (K1/K5)      71,680 B
+//   s_stage float [2][8960] double-buffered tile samples (K1)         71,680 B
 //   s_x     16 x 2114 words warp-private transpose tiles; reused for
 //                           |X|^2 (K1) / windowed frames (K4)        135,296 B
 //   bands   CSR form of the mel basis (K1)                            ~5,000 B
@@ -105,7 +105,7 @@ __device__ __forceinline__ void load_frame_pair(float2 (&v)[32], const float* s_
 }
 
 // ---------------------------------------------------------------------------------------
-// Mel phase shared by the fused kernels: lane <-> frame (pf = the lane's |X|^2 row, conflict-free LDS.128),
+// Mel phase of the fused log-mel kernel: lane <-> frame (pf = the lane's |X|^2 row, conflict-free LDS.128),
 // warp <-> its NB bands.  Per float4 group: one broadcast LDS.128 of weights, one LDS.128 of |X|^2, four FFMA --
 // no index loads, no per-group branch (a band is a run of consecutive bins); the NB results stay in registers
 // until all bands are done, so nothing orders the loads behind a store and they pipeline freely.
@@ -259,7 +259,7 @@ k_stft_mel(BatchView bv, const float* __restrict__ samples, float* __restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------
-// K5: STFT (+ Griffin-Lim phase update)
+// Griffin-Lim phase update of one bin: a = reb - alpha * tprev (unless has_prev == 0), S * a / (|a| + tiny)
 // ---------------------------------------------------------------------------------------
 __device__ __forceinline__ float2 phase_of(float2 reb, float s, float2 tp, float alpha, int has_prev) {
     float2 a = reb;
@@ -270,112 +270,6 @@ __device__ __forceinline__ float2 phase_of(float2 reb, float s, float2 tp, float
     const float den = sqrtf(fmaf(a.x, a.x, a.y * a.y)) + kTiny;
     const float r = 1.0f / den;   // numpy complex/real division multiplies by the reciprocal
     return make_float2(a.x * r * s, a.y * r * s);
-}
-
-template <int MODE>   // 0: plain STFT into `ang`; 1: Griffin-Lim phase update
-__global__ void __launch_bounds__(kThreads, 1)
-k_stft_phase(BatchView bv, const float* __restrict__ y, const float* __restrict__ S, int64_t ld_s,
-             float2* __restrict__ ang, float2* tprev, int64_t ld, float alpha,
-             int has_prev, const float2* __restrict__ g_tw, const float* __restrict__ g_win) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    float2* s_tw = reinterpret_cast<float2*>(smem_raw);
-    float* s_win = reinterpret_cast<float*>(s_tw + 1024);
-    spev_tile* s_ring = reinterpret_cast<spev_tile*>(s_win + 1024);
-    float* s_stage = reinterpret_cast<float*>(s_ring + kRing);
-    float* s_x = s_stage + 2 * kStageSamples;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    load_tables(s_tw, s_win, g_tw, g_win, 0.5f);
-    float2* xw = reinterpret_cast<float2*>(s_x + warp * kWarpRegionWords);
-
-    const int stride = gridDim.x;
-    pdl_launch_dependents();
-    const int my_n = ring_prologue(s_ring, bv.ftiles, bv.n_ftiles);
-    pdl_wait();   // y (and ang/tprev) come from the previous kernel
-    if (my_n > 0) stage_async(s_stage, y, s_ring[0]);
-    cp_async_commit();
-
-    for (int i = 0; i < my_n; ++i) {
-        cp_async_wait_all();
-        __syncthreads();
-        const int nf = s_ring[i & 3].n;
-        const int64_t row0 = s_ring[i & 3].row0;
-        if (i + 1 < my_n) stage_async(s_stage + ((i + 1) & 1) * kStageSamples, y, s_ring[(i + 1) & 3]);
-        if (i + 3 < my_n) fetch_desc(s_ring + ((i + 3) & 3), bv.ftiles + blockIdx.x + (i + 3) * stride);
-        cp_async_commit();
-        const float* stage = s_stage + (i & 1) * kStageSamples;
-
-        const int fa = 2 * warp;
-        if (fa < nf) {
-            const bool b_valid = fa + 1 < nf;
-            if (MODE == 1) {   // start pulling this pair's epilogue operands into L2 now
-                const int rows = b_valid ? 2 : 1;
-                warp_prefetch_l2(S + (row0 + fa) * ld_s, static_cast<int>((rows - 1) * ld_s + kBins) * 4, lane);
-                if (has_prev)
-                    warp_prefetch_l2(tprev + (row0 + fa) * ld, static_cast<int>((rows - 1) * ld + kBins) * 8, lane);
-            }
-            float2 v[32];
-            load_frame_pair(v, stage, s_win, fa, b_valid, lane);
-            warp_fft1024<-1>(v, xw, s_tw, lane);
-            float2 p[16];
-            fetch_mirror(v, p, lane);
-            const int64_t ra = (row0 + fa) * ld;        // row of frame a in ang / tprev
-            const int64_t rb = ra + ld;
-            const float* sa = S + (row0 + fa) * ld_s;
-            const float* sb = sa + ld_s;
-            // four groups of four bins-per-lane: all loads of a group are issued before its
-            // arithmetic so that 16 independent requests per thread are in flight (eight-bin groups
-            // were measured: no gain, and they spill)
-            static_for<0, 4>([&](auto gc) {
-                constexpr int g = decltype(gc)::value;
-                float2 tpa[4], tpb[4];
-                float s_a[4], s_b[4];
-                if (MODE == 1) {
-                    static_for<0, 4>([&](auto qc) {
-                        constexpr int q = decltype(qc)::value;
-                        const int k = lane + 32 * (4 * g + q);
-                        s_a[q] = sa[k];
-                        s_b[q] = b_valid ? sb[k] : 0.f;
-                        tpa[q] = has_prev ? tprev[ra + k] : make_float2(0.f, 0.f);
-                        tpb[q] = (has_prev && b_valid) ? tprev[rb + k] : make_float2(0.f, 0.f);
-                    });
-                }
-                static_for<0, 4>([&](auto qc) {
-                    constexpr int q = decltype(qc)::value;
-                    constexpr int k2 = 4 * g + q;
-                    const int k = lane + 32 * k2;
-                    float2 xa, xb;
-                    split_pair_prescaled(v[k2], p[k2], xa, xb);
-                    if (MODE == 0) {
-                        ang[ra + k] = xa;
-                        if (b_valid) ang[rb + k] = xb;
-                    } else {
-                        ang[ra + k] = phase_of(xa, s_a[q], tpa[q], alpha, has_prev);
-                        tprev[ra + k] = xa;
-                        if (b_valid) {
-                            ang[rb + k] = phase_of(xb, s_b[q], tpb[q], alpha, has_prev);
-                            tprev[rb + k] = xb;
-                        }
-                    }
-                });
-            });
-            if (lane == 0) {
-                // the window carries a factor 1/2: X[512] = 2 * Z'[512]
-                const float2 xa = make_float2(2.f * v[16].x, 0.f), xb = make_float2(2.f * v[16].y, 0.f);
-                if (MODE == 0) {
-                    ang[ra + 512] = xa;
-                    if (b_valid) ang[rb + 512] = xb;
-                } else {
-                    const float2 z = make_float2(0.f, 0.f);
-                    ang[ra + 512] = phase_of(xa, sa[512], has_prev ? tprev[ra + 512] : z, alpha, has_prev);
-                    tprev[ra + 512] = xa;
-                    if (b_valid) {
-                        ang[rb + 512] = phase_of(xb, sb[512], has_prev ? tprev[rb + 512] : z, alpha, has_prev);
-                        tprev[rb + 512] = xb;
-                    }
-                }
-            }
-        }
-    }
 }
 
 // ---------------------------------------------------------------------------------------
@@ -428,19 +322,18 @@ __device__ __forceinline__ PairInfo stage_pair(float* region, const float* __res
     return pi;
 }
 
-// Work distribution: with `counter` the warps draw (tile, slot) pairs dynamically (draw_ticket) -- cfg3 has 2.7 pairs
-// per warp, which a static stride pays as 3 --, else they stride statically.
+// Work distribution: warp w of CTA c takes pairs w + 16 c, then strides by 16 * grid.
 // STAGE_T (phase update only): the pair's `tprev` rows are pulled into the warp's transpose tile by ONE bulk
 // asynchronous copy (cp.async.bulk, 8,272 B) as soon as the exchange has been read back; it lands during the second
 // 32-point DFT, so the epilogue reads them from shared memory instead of waiting on 32 global loads per lane
 // (ncu before: long_scoreboard 2.5 warps per issue cycle on exactly those loads).
 constexpr int kWsRegionWords = kXWords + kNfft + kHop;   // transpose tile + 1280 staged samples of the NEXT pair
 
-template <int MODE, bool STAGE_T, bool FUSE = false>   // MODE 0: plain STFT into `ang`; 1: Griffin-Lim phase update
+template <int MODE, bool STAGE_T>   // MODE 0: plain STFT into `ang`; 1: Griffin-Lim phase update
 __global__ void __launch_bounds__(kThreads, 1)
 k_stft_phase_w(BatchView bv, const float* __restrict__ y, const float* __restrict__ S, int64_t ld_s,
                float2* __restrict__ ang, float2* tprev, int64_t ld, float alpha, int has_prev,
-               const float2* __restrict__ g_tw, const float* __restrict__ g_win, unsigned* counter, unsigned base) {
+               const float2* __restrict__ g_tw, const float* __restrict__ g_win) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2* s_tw = reinterpret_cast<float2*>(smem_raw);
     float* s_win = reinterpret_cast<float*>(s_tw + 1024);
@@ -457,35 +350,22 @@ k_stft_phase_w(BatchView bv, const float* __restrict__ y, const float* __restric
     float2* xb = reinterpret_cast<float2*>(tile);
     uint64_t* tbar = s_bar + warp;
     unsigned tphase = 0;
-    const int pl = (32 - lane) & 31;
 
     const int64_t n_pairs = static_cast<int64_t>(bv.n_ftiles) * kWarps;
     const int64_t stride = static_cast<int64_t>(gridDim.x) * kWarps;
-    int64_t p_static = static_cast<int64_t>(blockIdx.x) * kWarps + warp;
-    bool drained = false;
-    unsigned pend = 0;                                   // lane 0: a ticket drawn one call ahead (hides the atomic's latency)
-    auto draw_ahead = [&]() { if (lane == 0) pend = draw_ticket(counter, base); };
-    // next (tile, slot) pair of this warp: >= n_pairs when the work is exhausted (a drained warp draws no more)
-    auto next_pair = [&]() -> int64_t {
-        if (counter == nullptr) { const int64_t p = p_static; p_static += stride; return p; }
-        if (drained) return n_pairs;
-        const unsigned t = __shfl_sync(0xffffffffu, pend, 0);
-        if (t >= static_cast<unsigned>(n_pairs)) { drained = true; return n_pairs; }
-        draw_ahead();
-        return static_cast<int64_t>(t);
-    };
+    int64_t p_next = static_cast<int64_t>(blockIdx.x) * kWarps + warp;
     // stage the samples of this warp's next pair that has frames (slots past a partial tile's end have none)
     auto stage_next = [&]() -> PairInfo {
         PairInfo pi{0, 0, 0};
         for (;;) {
-            const int64_t p = next_pair();
+            const int64_t p = p_next;
+            p_next += stride;
             if (p >= n_pairs) return pi;
             pi = stage_pair(xs, y, bv.ftiles, p, n_pairs, lane);
             if (pi.valid) return pi;
         }
     };
     pdl_wait();                                          // y / ang / tprev come from the previous kernel
-    if (counter != nullptr) draw_ahead();                // (tickets only after the wait: see k_istft)
     PairInfo cur = stage_next();
     cp_async_commit();
 
@@ -537,7 +417,6 @@ k_stft_phase_w(BatchView bv, const float* __restrict__ y, const float* __restric
         fetch_mirror(v, pm, lane);
         const float2* tsm = reinterpret_cast<const float2*>(tile);   // staged rows: a at [0, 514), b at [ld, ld + 514)
         if (staged) { bar_wait(tbar, tphase); tphase ^= 1; }
-        float nyq_a = 0.f, nyq_b = 0.f;                  // FUSE: Re(ang[512]) of the two frames (lane 0)
         static_for<0, 4>([&](auto gc) {
             constexpr int g = decltype(gc)::value;
             float2 tpa[4], tpb[4];
@@ -566,26 +445,13 @@ k_stft_phase_w(BatchView bv, const float* __restrict__ y, const float* __restric
                 if (MODE == 0) {
                     ang[ra + k] = xa;
                     if (b_valid) ang[rb + k] = xbv;
-                } else if (!FUSE) {
+                } else {
                     ang[ra + k] = phase_of(xa, s_a[q], tpa[q], alpha, has_prev);
                     tprev[ra + k] = xa;
                     if (b_valid) {
                         ang[rb + k] = phase_of(xbv, s_b[q], tpb[q], alpha, has_prev);
                         tprev[rb + k] = xbv;
                     }
-                } else {
-                    // the new spectra never leave the registers: pack them (A + iB, and conj(A) + i conj(B) for the
-                    // mirror half) exactly as k_istft packs the rows it loads
-                    float2 a = phase_of(xa, s_a[q], tpa[q], alpha, has_prev);
-                    float2 b = make_float2(0.f, 0.f);
-                    tprev[ra + k] = xa;
-                    if (b_valid) {
-                        b = phase_of(xbv, s_b[q], tpb[q], alpha, has_prev);
-                        tprev[rb + k] = xbv;
-                    }
-                    if (k2 == 0 && lane == 0) { a.y = 0.f; b.y = 0.f; }   // irfft ignores Im(DC)
-                    v[k2] = make_float2(a.x - b.y, a.y + b.x);
-                    pm[k2] = make_float2(a.x + b.y, b.x - a.y);
                 }
             });
         });
@@ -598,47 +464,14 @@ k_stft_phase_w(BatchView bv, const float* __restrict__ y, const float* __restric
             } else {
                 const float2 z = make_float2(0.f, 0.f);
                 const float2 ta = !has_prev ? z : (staged ? tsm[512] : tprev[ra + 512]);
-                const float2 na = phase_of(xa, sa[512], ta, alpha, has_prev);
-                if (FUSE) nyq_a = na.x; else ang[ra + 512] = na;
+                ang[ra + 512] = phase_of(xa, sa[512], ta, alpha, has_prev);
                 tprev[ra + 512] = xa;
                 if (b_valid) {
                     const float2 tb = !has_prev ? z : (staged ? tsm[ld + 512] : tprev[rb + 512]);
-                    const float2 nb = phase_of(xbv, sb[512], tb, alpha, has_prev);
-                    if (FUSE) nyq_b = nb.x; else ang[rb + 512] = nb;
+                    ang[rb + 512] = phase_of(xbv, sb[512], tb, alpha, has_prev);
                     tprev[rb + 512] = xbv;
                 }
             }
-        }
-        if (FUSE) {
-            // ---- inverse transform of the pair straight from the registers, Hann, and the overlap-add of the
-            // pair's two frames (frame b = frame a shifted by 8 rows of 32 samples: the same lane) ----
-            static_for<0, 16>([&](auto ic) {
-                constexpr int ii = decltype(ic)::value;
-                float2 r;
-                r.x = __shfl_sync(0xffffffffu, pm[15 - ii].x, pl);
-                r.y = __shfl_sync(0xffffffffu, pm[15 - ii].y, pl);
-                if (lane == 0) {
-                    if constexpr (ii == 0) r = make_float2(nyq_a, nyq_b);
-                    else r = pm[16 - ii];
-                }
-                v[16 + ii] = r;
-            });
-            __syncwarp();                                // staged tprev rows consumed: the tile is free for the exchange
-            warp_fft1024<1>(v, xb, s_tw, lane);
-            // s_win holds Hann / 2 (forward scaling); Hann / 1024 = s_win / 512 exactly
-            static_for<0, 32>([&](auto kc) {
-                constexpr int k2 = decltype(kc)::value;
-                const float w = s_win[lane + 32 * k2] * (1.0f / 512.0f);
-                v[k2].x *= w;
-                v[k2].y = b_valid ? v[k2].y * w : 0.f;
-            });
-            float* seg = reinterpret_cast<float*>(ang + ra) + lane;
-            static_for<0, 40>([&](auto jc) {
-                constexpr int j = decltype(jc)::value;
-                if constexpr (j < 8) seg[32 * j] = v[j].x;
-                else if constexpr (j < 32) seg[32 * j] = v[j].x + v[j - 8].y;
-                else { if (b_valid) seg[32 * j] = v[j - 8].y; }
-            });
         }
         __syncwarp();                                    // staged rows consumed: the tile is free for the next exchange
         cur = nxt;
@@ -650,18 +483,18 @@ k_stft_phase_w(BatchView bv, const float* __restrict__ y, const float* __restric
 // the INVERSE transform of the new spectra without leaving the registers; what goes back to HBM is the pair's
 // 1280-sample overlap-add segment (k_ola_pairs finishes the overlap-add) and the rebuilt spectra for the momentum term.
 //
-// Same work distribution and staging as k_stft_phase_w (warp-independent pairs, cp.async samples one pair ahead, bulk-
-// staged tprev rows), but the body is written ONCE and run twice per pair: pass 0 transforms the samples, pass 1 the
-// new spectra.  The inverse transform is the forward one on swapped components (swap(z) = i conj(z):
-// ifft(V) = swap(fft(swap(V)))), so both passes -- and, inside a pass, both 32-point stages -- execute the same
-// instructions.  The straight-line version (k_stft_phase_w<1, *, true>: four inlined 32-point DFTs, ~75 KB of code)
-// lost 1.3 warps per issue cycle to instruction fetch (ncu `no_instruction`) because its 16 drifting warps walk the
-// whole body at different places; this body is less than half of that.
-// FAST: |a| normalisation by MUFU.RSQ (2 ulp) instead of IEEE sqrt + divide.
+// Same staging as k_stft_phase_w (warp-independent pairs, cp.async samples one pair ahead, bulk-staged tprev rows),
+// but the body is written ONCE and run twice per pair: pass 0 transforms the samples, pass 1 the new spectra.  The
+// inverse transform is the forward one on swapped components (swap(z) = i conj(z): ifft(V) = swap(fft(swap(V)))), so
+// both passes -- and, inside a pass, both 32-point stages -- execute the same instructions.  A straight-line body (four
+// inlined 32-point DFTs, ~75 KB of code) was measured: it lost 1.3 warps per issue cycle to instruction fetch (ncu
+// `no_instruction`) because its 16 drifting warps walk the whole body at different places; this body is less than
+// half of that.
+// Work distribution: with `counter` the warps draw (tile, slot) pairs dynamically (draw_ticket) -- worth it once a
+// warp has many pairs, see launch_stft_phase --, else they stride statically like k_stft_phase_w.
 // ---------------------------------------------------------------------------------------
-template <bool FAST>
-__device__ __forceinline__ float2 phase_of_t(float2 reb, float s, float2 tp, float alpha, int has_prev) {
-    if constexpr (!FAST) return phase_of(reb, s, tp, alpha, has_prev);
+// phase_of with the |a| normalisation by MUFU.RSQ (2 ulp) instead of IEEE sqrt + divide
+__device__ __forceinline__ float2 phase_of_rsqrt(float2 reb, float s, float2 tp, float alpha, int has_prev) {
     float2 a = reb;
     if (has_prev) {
         a.x = a.x - alpha * tp.x;
@@ -675,11 +508,11 @@ __device__ __forceinline__ float2 phase_of_t(float2 reb, float s, float2 tp, flo
     return make_float2(a.x * r, a.y * r);
 }
 
-template <bool STAGE_T, bool FAST>
+template <bool STAGE_T>
 __global__ void __launch_bounds__(kThreads, 1)
 k_gl_fused(BatchView bv, const float* __restrict__ y, const float* __restrict__ S, int64_t ld_s,
            float* __restrict__ seg_base, float2* tprev, int64_t ld, float alpha, int has_prev,
-           const float2* __restrict__ g_tw, const float* __restrict__ g_win, unsigned* counter, unsigned base, int l2_hints) {
+           const float2* __restrict__ g_tw, const float* __restrict__ g_win, unsigned* counter, unsigned base) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2* s_tw = reinterpret_cast<float2*>(smem_raw);
     float* s_win = reinterpret_cast<float*>(s_tw + 1024);
@@ -698,8 +531,11 @@ k_gl_fused(BatchView bv, const float* __restrict__ y, const float* __restrict__ 
     uint64_t* sbar = s_bar + kWarps + warp;
     unsigned tphase = 0, sphase = 0;
     const int pl = (32 - lane) & 31;
-    // tprev streams through (read once, rewritten, next use a whole iteration away); S and the segments are re-used soon
-    const uint64_t pol_stream = l2_policy(l2_hints ? 1 : 0), pol_keep = l2_policy(l2_hints ? 2 : 0);
+    // tprev streams through (read once, rewritten, next use a whole iteration away); S and the segments are re-used soon.
+    // The broadcast from lane 0 keeps the policies in uniform registers: without it ptxas moves them to per-thread
+    // registers and converts them back before each of the ~50 hinted stores (measured 1 % slower at cfg3).
+    const uint64_t pol_stream = __shfl_sync(0xffffffffu, l2_policy_evict_first(), 0);
+    const uint64_t pol_keep = __shfl_sync(0xffffffffu, l2_policy_evict_last(), 0);
 
     const int64_t n_pairs = static_cast<int64_t>(bv.n_ftiles) * kWarps;
     const int64_t stride = static_cast<int64_t>(gridDim.x) * kWarps;
@@ -725,6 +561,9 @@ k_gl_fused(BatchView bv, const float* __restrict__ y, const float* __restrict__ 
         }
     };
     pdl_wait();                                          // y / tprev come from the previous kernels
+    // Tickets may only be drawn once every earlier launch of this kernel has finished drawing: with programmatic
+    // dependent launch the prologue above can run while the launch before the previous kernel is still at work, and
+    // its tickets would interleave with ours.  griddepcontrol.wait returns when the whole chain behind us is complete.
     if (counter != nullptr) draw_ahead();
     PairInfo cur = stage_next();
     cp_async_commit();
@@ -802,11 +641,11 @@ k_gl_fused(BatchView bv, const float* __restrict__ y, const float* __restrict__ 
                     const float2 xa = make_float2(2.f * v[16].x, 0.f), xbv = make_float2(2.f * v[16].y, 0.f);
                     const float2 z = make_float2(0.f, 0.f);
                     const float2 ta = !has_prev ? z : (staged ? tsm[512] : tprev[ra + 512]);
-                    nyq_a = phase_of_t<FAST>(xa, ssa[512], ta, alpha, has_prev).x;
+                    nyq_a = phase_of_rsqrt(xa, ssa[512], ta, alpha, has_prev).x;
                     st_hint(tprev + ra + 512, xa, pol_stream);
                     if (b_valid) {
                         const float2 tb = !has_prev ? z : (staged ? tsm[ld + 512] : tprev[rb + 512]);
-                        nyq_b = phase_of_t<FAST>(xbv, ssb[512], tb, alpha, has_prev).x;
+                        nyq_b = phase_of_rsqrt(xbv, ssb[512], tb, alpha, has_prev).x;
                         st_hint(tprev + rb + 512, xbv, pol_stream);
                     }
                 }
@@ -833,11 +672,11 @@ k_gl_fused(BatchView bv, const float* __restrict__ y, const float* __restrict__ 
                         const int k = lane + 32 * k2;
                         float2 xa, xbv;
                         split_pair_prescaled(v[k2], pm[k2], xa, xbv);
-                        float2 a = phase_of_t<FAST>(xa, s_a[q], tpa[q], alpha, has_prev);
+                        float2 a = phase_of_rsqrt(xa, s_a[q], tpa[q], alpha, has_prev);
                         float2 b = make_float2(0.f, 0.f);
                         st_hint(tprev + ra + k, xa, pol_stream);
                         if (b_valid) {
-                            b = phase_of_t<FAST>(xbv, s_b[q], tpb[q], alpha, has_prev);
+                            b = phase_of_rsqrt(xbv, s_b[q], tpb[q], alpha, has_prev);
                             st_hint(tprev + rb + k, xbv, pol_stream);
                         }
                         if (k2 == 0 && lane == 0) { a.y = 0.f; b.y = 0.f; }   // irfft ignores Im(DC)
@@ -886,166 +725,15 @@ k_gl_fused(BatchView bv, const float* __restrict__ y, const float* __restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------
-// K1 (default): fused STFT -> power -> mel -> log with DECOUPLED warps
-//
-// Same arithmetic as k_stft_mel<0> (bit-identical results), different schedule.  In the tile kernel above every
-// warp of the CTA walks through "stage / FFT / mel / copy-out" in lock-step, separated by three CTA barriers per
-// 32-frame tile: the four warps of a scheduler hit the shared-memory bursts, the latency-bound mel chains and the
-// barriers together (ncu: issue-active 65 %).  Here a warp owns one frame pair per tile end to end:
-//   * it stages its own 1280 samples with cp.async into its warp-private region (which is also its transpose
-//     tile), one pair ahead -- no CTA-wide staging buffer, no CTA barrier for the samples;
-//   * |X|^2 goes to a dedicated CTA buffer P (32 frames x 516 words) because the mel phase needs all 32 frames
-//     (lane <-> frame) -- the only cross-warp exchange;
-//   * all synchronisation is SPLIT-PHASE on four mbarriers (FULL: P written, EMPTY: P consumed, OUT: mel rows
-//     staged, COPIED: rows stored): a warp arrives as soon as its share is done and waits only where it needs the
-//     others', with the copy-out of the previous tile and the register-only first half of its next transform
-//     (frame loads, 32-point DFTs, twiddles) in between.  Warps drift apart by up to about a third of a tile, so
-//     the mel chains and exchanges of some overlap the FFT arithmetic of others.
-// Shared memory: twiddles 8 KB, window 4 KB, 16 regions x 8,480 B, P 66,048 B, staged rows 10,368 B, mel program.
-// ---------------------------------------------------------------------------------------
-constexpr int kPRow2 = 2 * kPSlot;               // words per frame PAIR in P: 1032 == 2 (mod 8) in 16-byte units
-constexpr int kPWords = kWarps * kPRow2;         // 16,512 words
-
-template <int NB>
-__global__ void __launch_bounds__(kThreads, 1)
-k_stft_mel_ws(BatchView bv, const float* __restrict__ samples, float* __restrict__ out,
-              const float2* __restrict__ g_tw, const float* __restrict__ g_win, MelProgram mb,
-              int log_mode, float floor_v, float lo, float hi) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    float2* s_tw = reinterpret_cast<float2*>(smem_raw);
-    float* s_win = reinterpret_cast<float*>(s_tw + 1024);
-    uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_win + 1024);          // [4] FULL, EMPTY, OUT, COPIED (+4 pad)
-    float* s_x = reinterpret_cast<float*>(s_bar + 8);                     // 16 warp regions
-    float* s_p = s_x + kWarps * kXWords;                                  // |X|^2 of the tile
-    float* s_out = s_p + kPWords;                                         // [32][n_mels + 1]
-    float4* s_gw = reinterpret_cast<float4*>(s_out + kTileFrames * (mb.n_mels + 1) + ((4 - (kTileFrames * (mb.n_mels + 1)) % 4) % 4));
-    int4* s_hdr = reinterpret_cast<int4*>(s_gw + mb.n_groups);
-    uint64_t* b_full = s_bar, *b_empty = s_bar + 1, *b_out = s_bar + 2, *b_copied = s_bar + 3;
-
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    load_tables(s_tw, s_win, g_tw, g_win, 0.5f);
-    for (int i = threadIdx.x; i < mb.n_groups; i += blockDim.x) s_gw[i] = mb.gw[i];
-    for (int i = threadIdx.x; i < kWarps * mb.nb; i += blockDim.x) s_hdr[i] = mb.hdr[i];
-    if (threadIdx.x == 0) {
-        bar_init(b_full, kWarps); bar_init(b_empty, kWarps); bar_init(b_out, kWarps); bar_init(b_copied, kWarps);
-        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-    }
-    __syncthreads();                                                      // the only CTA-wide barrier
-
-    float* region = s_x + warp * kXWords;
-    float2* xb = reinterpret_cast<float2*>(region);
-    const int n_mels = mb.n_mels, out_pitch = n_mels + 1;
-    const int rows_per_pass = kThreads / n_mels;
-    const int cp_m = threadIdx.x % n_mels, cp_f0 = threadIdx.x / n_mels;
-    const float* pf = s_p + (lane >> 1) * kPRow2 + (lane & 1) * kPSlot;   // mel phase: lane <-> frame
-    float* pw = s_p + warp * kPRow2;                                      // this warp's two rows of P
-    const int4* hdr = s_hdr + warp * mb.nb;
-
-    const int first = blockIdx.x, stride = gridDim.x;
-    const int my_n = first < bv.n_ftiles ? (bv.n_ftiles - first + stride - 1) / stride : 0;
-    const int64_t n_pairs = static_cast<int64_t>(bv.n_ftiles) * kWarps;
-
-    // mel projection + log of tile j (all 32 frames, this warp's bands) into s_out
-    auto mel_phase = [&](int j) {
-        bar_wait(b_full, j & 1);                       // everybody's |X|^2 of tile j is in P
-        if (j >= 1) bar_wait(b_copied, (j - 1) & 1);   // tile j-1's rows have left s_out
-        mel_bands<NB>(pf, s_gw, hdr, mb.nb, s_out + lane * out_pitch, log_mode, floor_v, lo, hi);
-        __syncwarp();
-        if (lane == 0) { bar_arrive(b_out); bar_arrive(b_empty); }
-    };
-    // store the staged rows of tile j (this thread's share)
-    auto copy_out = [&](int j) {
-        const spev_tile* d = bv.ftiles + first + static_cast<int64_t>(j) * stride;
-        const int nf = __ldg(&d->n);
-        const int64_t row0 = __ldg(&d->row0);
-        bar_wait(b_out, j & 1);                        // everybody's bands of tile j are in s_out
-        float* o = out + row0 * n_mels;
-        if (cp_f0 < rows_per_pass)
-            for (int f = cp_f0; f < nf; f += rows_per_pass) o[f * n_mels + cp_m] = s_out[f * out_pitch + cp_m];
-        __syncwarp();
-        if (lane == 0) bar_arrive(b_copied);
-    };
-
-    PairInfo cur{0, 0, 0};
-    if (my_n > 0) cur = stage_pair(region, samples, bv.ftiles, static_cast<int64_t>(first) * kWarps + warp, n_pairs, lane);
-    cp_async_commit();
-
-    for (int i = 0; i < my_n; ++i) {
-        // ---- front half of tile i's transform: registers only ----
-        float2 v[32];
-        cp_async_wait_all();
-        __syncwarp();
-        if (cur.valid) {
-            load_frame_pair(v, region, s_win, 0, cur.b_valid != 0, lane);
-            dft32<-1>(v);
-            static_for<1, 32>([&](auto k1c) {
-                constexpr int k1 = decltype(k1c)::value;
-                v[k1] = cmul(v[k1], s_tw[k1 * 32 + lane]);
-            });
-        }
-        __syncwarp();                                  // staged samples consumed: the region may be overwritten
-        // ---- previous tile: mel phase (needs all warps' P; they had the whole front half above to get there) ----
-        if (i >= 1) mel_phase(i - 1);
-        // ---- back half: exchange, second DFT, Hermitian split, |X|^2 -> P ----
-        PairInfo nxt{0, 0, 0};
-        if (cur.valid) {
-            static_for<0, 32>([&](auto k1c) {
-                constexpr int k1 = decltype(k1c)::value;
-                xb[k1 * kXPitch + lane] = v[k1];
-            });
-            __syncwarp();
-            static_for<0, 32>([&](auto n2c) {
-                constexpr int n2 = decltype(n2c)::value;
-                v[n2] = xb[lane * kXPitch + n2];
-            });
-            __syncwarp();                              // tile read back: free for the next pair's samples
-        }
-        if (i + 1 < my_n)
-            nxt = stage_pair(region, samples, bv.ftiles, (static_cast<int64_t>(first) + static_cast<int64_t>(i + 1) * stride) * kWarps + warp,
-                             n_pairs, lane);
-        cp_async_commit();
-        if (cur.valid) {
-            dft32<-1>(v);
-            float2 p[16];
-            fetch_mirror(v, p, lane);
-            if (i >= 1) bar_wait(b_empty, (i - 1) & 1);   // everybody has finished reading P of tile i-1
-            const float pa512 = 4.f * v[16].x * v[16].x, pb512 = 4.f * v[16].y * v[16].y;
-            static_for<0, 16>([&](auto kc) {
-                constexpr int k2 = decltype(kc)::value;
-                float2 xa, xb2;
-                split_pair_prescaled(v[k2], p[k2], xa, xb2);
-                pw[lane + 32 * k2] = fmaf(xa.x, xa.x, xa.y * xa.y);
-                pw[kPSlot + lane + 32 * k2] = fmaf(xb2.x, xb2.x, xb2.y * xb2.y);
-            });
-            if (lane < 4) {   // bin 512 + three zero words so that padded float4 band reads stay clean
-                pw[512 + lane] = lane == 0 ? pa512 : 0.f;
-                pw[kPSlot + 512 + lane] = lane == 0 ? pb512 : 0.f;
-            }
-        } else if (i >= 1) {
-            bar_wait(b_empty, (i - 1) & 1);            // keep the phase bookkeeping uniform
-        }
-        __syncwarp();
-        if (lane == 0) bar_arrive(b_full);
-        // ---- the previous tile's staged rows (everybody's bands arrived before their own back half) ----
-        if (i >= 1) copy_out(i - 1);
-        cur = nxt;
-    }
-    // ---- drain: the last tile ----
-    if (my_n >= 1) { mel_phase(my_n - 1); copy_out(my_n - 1); }
-}
-
-// ---------------------------------------------------------------------------------------
 // K4: ISTFT with gather overlap-add and window-sum-square normalisation
 // ---------------------------------------------------------------------------------------
-// With `counter` the CTAs draw their tiles dynamically (draw_ticket; thread 0 draws three tiles ahead, like the static
-// ring): cfg3's 448 chunk tiles are 3.03 rounds of work on 148 SMs, which the static round-robin pays as 4.
 // BULK: a warp's two spectrum rows (8,272 B) arrive in its region by ONE bulk asynchronous copy instead of 34 scattered
 // 8-byte loads per lane (ncu r01: lg_throttle 1.2 + long_scoreboard 1.7 warps per issue cycle on those loads): no LSU
 // queue pressure, and all 16 warps' rows are in flight at once.
 template <bool BULK>
 __global__ void __launch_bounds__(kThreads, 1)
 k_istft(BatchView bv, const float2* __restrict__ spec, int64_t ld, float* __restrict__ y,
-        const float2* __restrict__ g_tw, const float* __restrict__ g_win, unsigned* counter, unsigned base) {
+        const float2* __restrict__ g_tw, const float* __restrict__ g_win) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float2* s_tw = reinterpret_cast<float2*>(smem_raw);
     float* s_win = reinterpret_cast<float*>(s_tw + 1024);
@@ -1072,25 +760,15 @@ k_istft(BatchView bv, const float2* __restrict__ spec, int64_t ld, float* __rest
 
     const int stride = gridDim.x;
     pdl_launch_dependents();
-    // slot j of the ring <- the CTA's j-th tile: static (blockIdx.x + j * grid) or the next ticket (thread 0 only;
-    // it stops drawing at its first ticket past the end, so a launch consumes exactly n_ctiles + grid tickets)
-    bool drained = false;
+    // slot j of the ring <- the CTA's j-th tile, blockIdx.x + j * grid (thread 0 only)
     auto claim = [&](int j) {
         if (threadIdx.x != 0) return;
         int t = -1;
-        if (counter == nullptr) {
-            const int64_t q = blockIdx.x + static_cast<int64_t>(j) * stride;
-            if (q < bv.n_ctiles) t = static_cast<int>(q);
-        } else if (!drained) {
-            const unsigned q = draw_ticket(counter, base);
-            if (q < static_cast<unsigned>(bv.n_ctiles)) t = static_cast<int>(q); else drained = true;
-        }
+        const int64_t q = blockIdx.x + static_cast<int64_t>(j) * stride;
+        if (q < bv.n_ctiles) t = static_cast<int>(q);
         s_tick[j & 3] = t;
         if (t >= 0) fetch_desc(s_ring + (j & 3), bv.ctiles + t);
     };
-    // Tickets may only be drawn once every earlier launch of this kernel has finished drawing: with programmatic
-    // dependent launch the prologue above can run while the launch before the previous kernel is still at work, and
-    // its tickets would interleave with ours.  griddepcontrol.wait returns when the whole chain behind us is complete.
     pdl_wait();   // the spectra come from the previous kernel
     for (int j = 0; j < 3; ++j) claim(j);
     cp_async_commit();
@@ -1208,7 +886,7 @@ k_istft(BatchView bv, const float2* __restrict__ spec, int64_t ld, float* __rest
 // ---------------------------------------------------------------------------------------
 // K4p: overlap-add of PAIR segments (the fused Griffin-Lim iteration)
 //
-// k_stft_phase_w<1, *, true> leaves, for every frame pair (2j, 2j+1) of an item, the 1280-sample sum of its two
+// k_gl_fused leaves, for every frame pair (2j, 2j+1) of an item, the 1280-sample sum of its two
 // windowed inverse-transform frames at row (item row + 2j) of the `ang` workspace (float view, 2 * ld floats per row;
 // a lone last frame leaves its 1024 samples).  Padded chunk q = c + 2 of output chunk c lies in the segments of pairs
 // j with 0 <= q - 2j <= 4 -- two or three of them --, summed here in ascending pair order and normalised by the
@@ -1221,7 +899,7 @@ constexpr int kOlaParts = (kTileChunks + kOlaWarps * kOlaPerWarp - 1) / (kOlaWar
 
 __global__ void __launch_bounds__(kOlaWarps * 32)
 k_ola_pairs(BatchView bv, const float* __restrict__ seg, int64_t ld_f, float* __restrict__ y,
-            const float* __restrict__ g_win /* [1024] Hann, then [256] 1 / sum_q w^2 (ctx table) */, int l2_hints) {
+            const float* __restrict__ g_win /* [1024] Hann, then [256] 1 / sum_q w^2 (ctx table) */) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const float* g_iw = g_win + kNfft;
     pdl_launch_dependents();
@@ -1282,17 +960,12 @@ k_ola_pairs(BatchView bv, const float* __restrict__ seg, int64_t ld_f, float* __
             r1 = make_float4(norm(r1.x, s1), norm(r1.y, s1 + 1), norm(r1.z, s1 + 2), norm(r1.w, s1 + 3));
         }
         float* yo = yo0 + static_cast<int64_t>(cl0 + e) * kHop;
-        if ((reinterpret_cast<uintptr_t>(yo) & 15) == 0) {
-            if (l2_hints) {   // y is read back by the next kernel: keep it in L2
-                const uint64_t pol = l2_policy(2);
-                asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %2, %3, %4}, %5;\n" ::"l"(reinterpret_cast<float4*>(yo) + lane),
-                             "f"(r0.x), "f"(r0.y), "f"(r0.z), "f"(r0.w), "l"(pol) : "memory");
-                asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %2, %3, %4}, %5;\n" ::"l"(reinterpret_cast<float4*>(yo) + 32 + lane),
-                             "f"(r1.x), "f"(r1.y), "f"(r1.z), "f"(r1.w), "l"(pol) : "memory");
-            } else {
-                reinterpret_cast<float4*>(yo)[lane] = r0;
-                reinterpret_cast<float4*>(yo)[32 + lane] = r1;
-            }
+        if ((reinterpret_cast<uintptr_t>(yo) & 15) == 0) {   // y is read back by the next kernel: keep it in L2
+            const uint64_t pol = l2_policy_evict_last();
+            asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %2, %3, %4}, %5;\n" ::"l"(reinterpret_cast<float4*>(yo) + lane),
+                         "f"(r0.x), "f"(r0.y), "f"(r0.z), "f"(r0.w), "l"(pol) : "memory");
+            asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %2, %3, %4}, %5;\n" ::"l"(reinterpret_cast<float4*>(yo) + 32 + lane),
+                         "f"(r1.x), "f"(r1.y), "f"(r1.z), "f"(r1.w), "l"(pol) : "memory");
         } else {
             yo[s0] = r0.x; yo[s0 + 1] = r0.y; yo[s0 + 2] = r0.z; yo[s0 + 3] = r0.w;
             yo[s1] = r1.x; yo[s1 + 1] = r1.y; yo[s1 + 2] = r1.z; yo[s1 + 3] = r1.w;
@@ -1441,24 +1114,18 @@ int launch_stft_mel(spev_ctx* ctx, const spev_batch* b, const float* samples, fl
                  "(%zu B > 232448); bands wider than ~128 bins (n_mels below ~24 at 22 kHz) are not supported",
                  ctx->n_mels, ctx->prog_groups, smem);
     const int grid = std::min<int64_t>(b->n_ftiles, ctx->num_sms);
-    const size_t out_words = (static_cast<size_t>(kTileFrames) * (ctx->n_mels + 1) + 3) & ~static_cast<size_t>(3);
-    const size_t smem_ws = sizeof(float2) * 1024 + sizeof(float) * 1024 + sizeof(uint64_t) * 8 +
-                           sizeof(float) * kWarps * kXWords + sizeof(float) * kPWords + sizeof(float) * out_words +
-                           smem_prog(ctx);
-    const bool ws = !power_only && ctx->k1_variant == 1 && smem_ws <= 232448;
-    const size_t bytes = ws ? smem_ws : smem;
     auto go = [&](auto kernel, bool mel) -> int {
-        kernel<<<grid, kThreads, bytes, st>>>(view_of(b), samples, out, ctx->d_tw, ctx->d_window, mb, mel ? log_mode : 0,
-                                              mel ? floor_v : 0.f, mel ? lo : 0.f, mel ? hi : 0.f);
+        kernel<<<grid, kThreads, smem, st>>>(view_of(b), samples, out, ctx->d_tw, ctx->d_window, mb, mel ? log_mode : 0,
+                                             mel ? floor_v : 0.f, mel ? lo : 0.f, mel ? hi : 0.f);
         SPEV_CUDA(cudaGetLastError());
         return SPEV_OK;
     };
     if (power_only) return go(k_stft_mel<1, 0>, false);
-#define SPEV_K1_CASE(NBV) case NBV: return ws ? go(k_stft_mel_ws<NBV>, true) : go(k_stft_mel<0, NBV>, true)
+#define SPEV_K1_CASE(NBV) case NBV: return go(k_stft_mel<0, NBV>, true)
     switch (mb.nb) {
         SPEV_K1_CASE(1); SPEV_K1_CASE(2); SPEV_K1_CASE(3); SPEV_K1_CASE(4);
         SPEV_K1_CASE(5); SPEV_K1_CASE(6); SPEV_K1_CASE(7); SPEV_K1_CASE(8);
-        default: return ws ? go(k_stft_mel_ws<0>, true) : go(k_stft_mel<0, 0>, true);
+        default: return go(k_stft_mel<0, 0>, true);
     }
 #undef SPEV_K1_CASE
 }
@@ -1481,17 +1148,11 @@ int launch_stft_phase(spev_ctx* ctx, const spev_batch* b, const float* y, const 
     if (!phase) {
         // plain STFT: warp-independent kernel (r01: 18.0 vs 19.9 us at cfg3, 128 vs 156 us on 120 k frames)
         return launch_pdl(k_stft_phase_w<0, false>, grid, kThreads, smem_ws_phase(), st, view_of(b), y, static_cast<const float*>(nullptr),
-                          static_cast<int64_t>(0), static_cast<float2*>(ang), static_cast<float2*>(nullptr), ld, 0.f, 0, tw, win,
-                          counter, base);
+                          static_cast<int64_t>(0), static_cast<float2*>(ang), static_cast<float2*>(nullptr), ld, 0.f, 0, tw, win);
     }
     SPEV_REQUIRE(S && tprev && ld_s >= kBins, SPEV_E_INVALID, "phase update: null S/tprev");
-    if (ctx->gl_variant == 0)   // r01 tile kernel: CTA-staged samples, direct tprev loads, static round-robin
-        return launch_pdl(k_stft_phase<1>, grid, kThreads, smem_stft(0), st, view_of(b), y, S, ld_s, static_cast<float2*>(ang),
-                          static_cast<float2*>(tprev), ld, alpha, has_prev, tw, win);
     // bulk staging of the tprev rows needs 16-byte aligned rows with one readable pad column, and both rows of a pair
     // must fit the warp's transpose tile
-    unsigned* const counter_in = counter;
-    if (!(ctx->gl_variant & 4)) counter = nullptr;
     const bool stage_t = (reinterpret_cast<uintptr_t>(tprev) & 15) == 0 && ld % 2 == 0 && ld > kBins &&
                          static_cast<size_t>(ld) * 8 + (kBins + 1) * 8 <= sizeof(float) * kXWords;
     if (fuse) {
@@ -1500,28 +1161,15 @@ int launch_stft_phase(spev_ctx* ctx, const spev_batch* b, const float* y, const 
                      "fused phase update: segment rows need 16-byte alignment and >= 1024 floats per row");
         // dynamic pair tickets pay once a warp has many pairs (measured: 0.72 vs 0.67 of the roofline on 138 k frames,
         // 0.635 vs 0.65 at cfg3's 2.7 pairs per warp): chosen from the batch alone, so every launch of a call agrees
-        if (!(ctx->gl_variant & 4) && b->n_ftiles >= 8 * grid) counter = counter_in;
-        float* seg = static_cast<float*>(ang);
-        const bool fast = (ctx->gl_variant & 16) != 0;
-#define SPEV_GLF(ST, FA) launch_pdl(k_gl_fused<ST, FA>, grid, kThreads, smem_gl_fused(), st, view_of(b), y, S, ld_s, seg, \
-                                    static_cast<float2*>(tprev), ld, alpha, has_prev, tw, win, counter, base, (ctx->gl_variant & 64) ? 1 : 0)
-        if (ctx->gl_variant & 32)   // straight-line body (A/B: instruction-fetch bound)
-            return stage_t ? launch_pdl(k_stft_phase_w<1, true, true>, grid, kThreads, smem_ws_phase(), st, view_of(b), y, S, ld_s,
-                                        static_cast<float2*>(ang), static_cast<float2*>(tprev), ld, alpha, has_prev, tw, win, counter, base)
-                           : launch_pdl(k_stft_phase_w<1, false, true>, grid, kThreads, smem_ws_phase(), st, view_of(b), y, S, ld_s,
-                                        static_cast<float2*>(ang), static_cast<float2*>(tprev), ld, alpha, has_prev, tw, win, counter, base);
+        if (b->n_ftiles < 8 * grid) counter = nullptr;
         // bulk staging of the S rows: 16-byte aligned rows, both rows (+ 3 pad columns) inside the 1280-float sample region
         const bool stage_s = stage_t && (reinterpret_cast<uintptr_t>(S) & 15) == 0 && ld_s % 4 == 0 && ld_s >= kPSlot &&
                              ld_s + kPSlot <= kNfft + kHop;
-        if (stage_s) return fast ? SPEV_GLF(true, true) : SPEV_GLF(true, false);
-        return fast ? SPEV_GLF(false, true) : SPEV_GLF(false, false);
-#undef SPEV_GLF
+        return launch_pdl(stage_s ? k_gl_fused<true> : k_gl_fused<false>, grid, kThreads, smem_gl_fused(), st, view_of(b), y, S,
+                          ld_s, static_cast<float*>(ang), static_cast<float2*>(tprev), ld, alpha, has_prev, tw, win, counter, base);
     }
-    if (stage_t)
-        return launch_pdl(k_stft_phase_w<1, true>, grid, kThreads, smem_ws_phase(), st, view_of(b), y, S, ld_s, static_cast<float2*>(ang),
-                          static_cast<float2*>(tprev), ld, alpha, has_prev, tw, win, counter, base);
-    return launch_pdl(k_stft_phase_w<1, false>, grid, kThreads, smem_ws_phase(), st, view_of(b), y, S, ld_s, static_cast<float2*>(ang),
-                      static_cast<float2*>(tprev), ld, alpha, has_prev, tw, win, counter, base);
+    return launch_pdl(stage_t ? k_stft_phase_w<1, true> : k_stft_phase_w<1, false>, grid, kThreads, smem_ws_phase(), st, view_of(b),
+                      y, S, ld_s, static_cast<float2*>(ang), static_cast<float2*>(tprev), ld, alpha, has_prev, tw, win);
 }
 
 // Overlap-add of the pair segments the fused phase update left in `seg` (rows of 2 * ld floats) into y.
@@ -1531,24 +1179,19 @@ int launch_ola_pairs(spev_ctx* ctx, const spev_batch* b, const void* seg, int64_
     if (b->n_ctiles == 0) return SPEV_OK;
     SPEV_REQUIRE(seg && y, SPEV_E_INVALID, "ola: null buffer");
     return launch_pdl(k_ola_pairs, b->n_ctiles * kOlaParts, kOlaWarps * 32, 0, st, view_of(b), static_cast<const float*>(seg),
-                      2 * ld, y, static_cast<const float*>(ctx->d_window), (ctx->gl_variant & 64) ? 1 : 0);
+                      2 * ld, y, static_cast<const float*>(ctx->d_window));
 }
 
-int launch_istft(spev_ctx* ctx, const spev_batch* b, const void* spec, int64_t ld, float* y,
-                 cudaStream_t st, unsigned* counter, unsigned base) {
+int launch_istft(spev_ctx* ctx, const spev_batch* b, const void* spec, int64_t ld, float* y, cudaStream_t st) {
     int rc = check_batch(ctx, b, true);
     if (rc) return rc;
     if (b->n_ctiles == 0) return SPEV_OK;
     SPEV_REQUIRE(spec && y && ld >= kBins, SPEV_E_INVALID, "istft: null buffer or ld < 513");
     // bulk staging needs 16-byte aligned rows with one readable pad column, two rows per warp region
-    const bool bulk = ctx->gl_variant != 0 && (reinterpret_cast<uintptr_t>(spec) & 15) == 0 && ld % 2 == 0 && ld > kBins &&
+    const bool bulk = (reinterpret_cast<uintptr_t>(spec) & 15) == 0 && ld % 2 == 0 && ld > kBins &&
                       static_cast<size_t>(ld) * 8 + (kBins + 1) * 8 <= sizeof(float) * kWarpRegionWords;
-    unsigned* ctr = (ctx->gl_variant & 2) ? counter : nullptr;
-    if (bulk)
-        return launch_pdl(k_istft<true>, fft_grid(ctx, b->n_ctiles), kThreads, smem_istft(), st, view_of(b), static_cast<const float2*>(spec),
-                          ld, y, static_cast<const float2*>(ctx->d_tw), static_cast<const float*>(ctx->d_window), ctr, base);
-    return launch_pdl(k_istft<false>, fft_grid(ctx, b->n_ctiles), kThreads, smem_istft(), st, view_of(b), static_cast<const float2*>(spec),
-                      ld, y, static_cast<const float2*>(ctx->d_tw), static_cast<const float*>(ctx->d_window), ctr, base);
+    return launch_pdl(bulk ? k_istft<true> : k_istft<false>, fft_grid(ctx, b->n_ctiles), kThreads, smem_istft(), st, view_of(b),
+                      static_cast<const float2*>(spec), ld, y, static_cast<const float2*>(ctx->d_tw), static_cast<const float*>(ctx->d_window));
 }
 
 // Opt every FFT kernel into the full shared-memory carve-out ONCE per ctx (per device) -- r01 re-issued
@@ -1557,15 +1200,11 @@ int spectral_init(spev_ctx*) {
     const int kMax = 232448;
     int rc = SPEV_OK;
     auto opt = [&](auto kernel) { if (!rc) rc = set_smem(kernel, kMax); };
-    opt(k_stft_mel<1, 0>); opt(k_stft_mel<0, 0>); opt(k_stft_mel_ws<0>);
+    opt(k_stft_mel<1, 0>); opt(k_stft_mel<0, 0>);
     opt(k_stft_mel<0, 1>); opt(k_stft_mel<0, 2>); opt(k_stft_mel<0, 3>); opt(k_stft_mel<0, 4>);
     opt(k_stft_mel<0, 5>); opt(k_stft_mel<0, 6>); opt(k_stft_mel<0, 7>); opt(k_stft_mel<0, 8>);
-    opt(k_stft_mel_ws<1>); opt(k_stft_mel_ws<2>); opt(k_stft_mel_ws<3>); opt(k_stft_mel_ws<4>);
-    opt(k_stft_mel_ws<5>); opt(k_stft_mel_ws<6>); opt(k_stft_mel_ws<7>); opt(k_stft_mel_ws<8>);
-    opt(k_stft_phase<0>); opt(k_stft_phase<1>);
     opt(k_stft_phase_w<0, false>); opt(k_stft_phase_w<1, false>); opt(k_stft_phase_w<1, true>);
-    opt(k_stft_phase_w<1, false, true>); opt(k_stft_phase_w<1, true, true>);
-    opt(k_gl_fused<true, true>); opt(k_gl_fused<true, false>); opt(k_gl_fused<false, true>); opt(k_gl_fused<false, false>);
+    opt(k_gl_fused<true>); opt(k_gl_fused<false>);
     opt(k_istft<true>); opt(k_istft<false>);
     return rc;
 }

@@ -78,6 +78,4 @@ struct spev_ctx {
     int band_max_len;
     void* tma;           // opaque: tensor-map cache (gemm_tc.cu)
     int use_tc;          // mel->magnitude on frame-major input uses the tcgen05 GEMM
-    int gl_variant;      // Griffin-Lim kernels, bit set (spev_set_griffinlim_variant): default 89 = bulk-staged rows | fused iteration | rsqrt | L2 hints; 0 = r01 static tile kernels
-    int k1_variant;      // fused log-mel kernel: 1 = decoupled warps (k_stft_mel_ws, default), 0 = tile lock-step (k_stft_mel<0>)
 };

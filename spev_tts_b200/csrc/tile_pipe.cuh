@@ -61,16 +61,12 @@ __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepc
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;\n" ::: "memory"); }
 
 // ---------------------------------------------------------------------------------------
-// split-phase CTA synchronisation on shared-memory mbarriers: a warp ARRIVES when its part of a
-// phase is done and WAITS only where it needs everybody's part -- with useful work in between.
-// (one elected lane arrives after __syncwarp(); waits are bounded: a protocol bug traps instead of hanging)
+// shared-memory mbarriers, completed by the bulk asynchronous copies below
+// (waits are bounded: a protocol bug traps instead of hanging)
 // ---------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_addr(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
 __device__ __forceinline__ void bar_init(uint64_t* bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;\n" ::"r"(smem_addr(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void bar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.release.cta.shared::cta.b64 _, [%0];\n" ::"r"(smem_addr(bar)) : "memory");
 }
 __device__ __forceinline__ void bar_wait(uint64_t* bar, uint32_t parity) {
     const uint32_t addr = smem_addr(bar);
@@ -97,11 +93,14 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gsrc, uint3
 }
 // L2 eviction policies (createpolicy): the Griffin-Lim loop streams 106 MB of momentum spectra per iteration through
 // an L2 that could otherwise keep its 73 MB producer -> consumer working set (S, pair segments, y) resident.
-__device__ __forceinline__ uint64_t l2_policy(int kind) {   // 0: normal, 1: evict first (streaming), 2: evict last (keep)
+__device__ __forceinline__ uint64_t l2_policy_evict_first() {   // streaming data
     uint64_t p;
-    if (kind == 1) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;\n" : "=l"(p));
-    else if (kind == 2) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;\n" : "=l"(p));
-    else asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;\n" : "=l"(p));
+    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;\n" : "=l"(p));
+    return p;
+}
+__device__ __forceinline__ uint64_t l2_policy_evict_last() {    // data read again soon
+    uint64_t p;
+    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;\n" : "=l"(p));
     return p;
 }
 __device__ __forceinline__ void bulk_g2s_hint(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar, uint64_t pol) {

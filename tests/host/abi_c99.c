@@ -15,7 +15,7 @@ int spev_c99_probe(void) {
     USE(spev_duration_rule); USE(spev_bucketize_embed); USE(spev_frame_features); USE(spev_segment_pool); USE(spev_segment_pool_log); USE(spev_pcm16_to_f32); USE(spev_collate); USE(spev_variance_fuse);
     USE(spev_pyin_create); USE(spev_pyin_destroy); USE(spev_pyin_info); USE(spev_pyin_host_tables);
     USE(spev_pyin_cmnd); USE(spev_pyin_observe); USE(spev_pyin_decode_workspace_bytes); USE(spev_pyin_decode); USE(spev_pitch_pool);
-    USE(spev_lr_expand_backward); USE(spev_copy_segments_piece_bytes); USE(spev_copy_segments); USE(spev_set_sm_limit); USE(spev_set_logmel_variant); USE(spev_set_griffinlim_variant); USE(spev_nnls_objective); USE(spev_transpose_batched); USE(spev_variance_fuse_backward_workspace_bytes); USE(spev_variance_fuse_backward);
+    USE(spev_lr_expand_backward); USE(spev_copy_segments_piece_bytes); USE(spev_copy_segments); USE(spev_set_sm_limit); USE(spev_nnls_objective); USE(spev_transpose_batched); USE(spev_variance_fuse_backward_workspace_bytes); USE(spev_variance_fuse_backward);
     t.n = 0; b.n_items = 0;
     return (int)sizeof(spev_tile) + t.n + b.n_items;   /* 48 */
 }

@@ -245,66 +245,126 @@ def test_griffinlim_24khz_cfg5(cuda):
         assert abs(lr.spectral_convergence(y, S) - ref[b][0]) <= 1e-3
 
 
-def test_griffinlim_kernel_variants_agree(cuda):
-    """The r02 Griffin-Lim kernels (dynamic tile tickets, bulk-staged tprev rows) and the r01 static tile kernels
-    perform the same arithmetic: bit-identical waveforms, ragged batch included."""
+def _two_kernel_griffinlim(ctx, fb, S, ph, n_iter, momentum=0.99):
+    """librosa.griffinlim's loop from the stand-alone entry points: ang0 = S e^{i phase} (built in torch), n_iter x
+    (spev_istft, spev_gl_phase_update), a final spev_istft.  The new spectra go through HBM and the phase normalisation
+    is IEEE sqrt + divide."""
+    from spev_tts_b200 import _lib
+    st = torch.cuda.current_stream(S.device).cuda_stream
+    ang = torch.zeros(fb.n_frames, _lib.SPEC_LD, dtype=torch.complex64, device=S.device)
+    ang[:, :513] = torch.polar(S[:, :513].contiguous(), ph)
+    tprev = torch.zeros_like(ang)
+    y = torch.empty(fb.n_out_samples, dtype=torch.float32, device=S.device)
+    m = float(np.float32(momentum))                 # spev_griffinlim takes a float and forms alpha in double
+    alpha = float(np.float32(m / (1.0 + m)))
+    for it in range(n_iter):
+        _lib.check(ctx.lib.spev_istft(ctx.handle, fb.desc, ang.data_ptr(), _lib.SPEC_LD, y.data_ptr(), st))
+        _lib.check(ctx.lib.spev_gl_phase_update(ctx.handle, fb.desc, y.data_ptr(), S.data_ptr(), S.shape[1], ang.data_ptr(),
+                                                tprev.data_ptr(), _lib.SPEC_LD, alpha, int(it > 0), st))
+    _lib.check(ctx.lib.spev_istft(ctx.handle, fb.desc, ang.data_ptr(), _lib.SPEC_LD, y.data_ptr(), st))
+    return y
+
+
+def test_griffinlim_static_and_dynamic_pair_tickets_agree(cuda):
+    """The fused phase update draws (tile, slot) pairs from a ticket counter once a batch has >= 8 frame tiles per CTA,
+    else it strides statically.  Capping the CTA count (spev_set_sm_limit) moves every batch across that line; both
+    schedules perform the same arithmetic: bit-identical waveforms, ragged batch included."""
     import spev_tts_b200 as sp
     from spev_tts_b200 import _lib
     ctx = sp.Context.get(cuda, fmin=0.0, fmax=8000.0)
+    n_sms = torch.cuda.get_device_properties(cuda).multi_processor_count
+    limits = (0, 1, 3, 16)                                      # 0: one CTA per SM
     # a ragged batch, a small single item (grids far below the SM count: successive launches overlap under programmatic
-    # dependent launch, which the ticket scheme must survive) and a batch larger than one round of tiles
+    # dependent launch, which the ticket bases must survive) and a batch larger than one round of tiles
     for frames, n_iter in (([800, 33, 1, 2, 64, 517, 95], 7), ([300], 25), ([40] * 7, 25), ([800] * 16, 3)):
         fb = sp.make_batch(ctx, n_frames=frames, with_chunks=True)
+        grids = [min(fb.n_ftiles, lim or n_sms) for lim in limits]
+        assert fb.n_ftiles < 8 * grids[0], frames               # static pairs without a limit ...
+        assert any(fb.n_ftiles >= 8 * grid for grid in grids[1:]), frames   # ... dynamic pairs under some limit
         g = torch.Generator(device=cuda).manual_seed(5)
         S = torch.rand(fb.n_frames, _lib.SPEC_LD, generator=g, device=cuda)
         ph = torch.rand(fb.n_frames, 513, generator=g, device=cuda) * 6.2831853
         outs = []
         try:
-            for variant in (0, 1, 7):
-                _lib.check(ctx.lib.spev_set_griffinlim_variant(ctx.handle, variant))
+            for lim in limits:
+                _lib.check(ctx.lib.spev_set_sm_limit(ctx.handle, lim))
                 outs.append(sp.griffinlim_flat(S, fb, ctx, n_iter=n_iter, init_phase=ph).clone())
         finally:
-            _lib.check(ctx.lib.spev_set_griffinlim_variant(ctx.handle, _lib.GL_VARIANT_DEFAULT))
-        assert torch.isfinite(outs[1]).all(), frames
-        assert torch.equal(outs[0], outs[1]) and torch.equal(outs[1], outs[2]), frames
+            _lib.check(ctx.lib.spev_set_sm_limit(ctx.handle, 0))   # the ctx is cached and shared
+        assert torch.isfinite(outs[0]).all(), frames
+        for lim, out in zip(limits[1:], outs[1:]):
+            assert torch.equal(outs[0], out), (frames, lim)
 
 
 def test_griffinlim_fused_iteration_matches_two_kernel_path(cuda):
-    """The fused iteration (default, variant 89 = 9 + rsqrt phase normalisation + L2 hints; 9: the new spectra are inverse-transformed in registers inside the phase
-    update and leave as pair segments; k_ola_pairs overlap-adds them) against the two-kernel path (variant 1: spectra
-    through HBM, k_istft): same arithmetic per frame, only the order of the <= 4 overlap-add terms differs (pairs first),
-    so a few iterations agree to rounding; static and dynamic pair scheduling are bit-identical to each other."""
+    """spev_griffinlim runs the fused iteration (the new spectra are inverse-transformed in registers inside the phase
+    update and leave as pair segments; k_ola_pairs overlap-adds them, rsqrt phase normalisation).  The two-kernel loop
+    from the stand-alone entry points (spectra through HBM, k_istft) does the same arithmetic per frame up to the phase
+    normalisation (2 ulp) and the order of the <= 4 overlap-add terms (pairs first), so a few iterations agree to
+    rounding.  n_iter = 0 is one ISTFT of ang0 on both sides; only torch's cos / sin and sincosf may differ there."""
     import spev_tts_b200 as sp
     from spev_tts_b200 import _lib
     ctx = sp.Context.get(cuda, fmin=0.0, fmax=8000.0)
     for frames, n_iter, tol in (([800, 33, 1, 2, 3, 4, 5, 64, 517, 95, 31], 1, 2e-6), ([800, 33, 1, 2, 3, 4, 5, 64, 517, 95, 31], 3, 1e-5),
-                                ([7] * 40, 2, 1e-5), ([800] * 16, 2, 1e-5), ([301], 0, 0.0)):
+                                ([7] * 40, 2, 1e-5), ([800] * 16, 2, 1e-5), ([301], 0, 1e-6)):
         fb = sp.make_batch(ctx, n_frames=frames, with_chunks=True)
         g = torch.Generator(device=cuda).manual_seed(11)
         S = torch.rand(fb.n_frames, _lib.SPEC_LD, generator=g, device=cuda)
         ph = torch.rand(fb.n_frames, 513, generator=g, device=cuda) * 6.2831853
-        outs = {}
-        try:
-            for variant in (1, 9, 13, 25, 41, 89):
-                _lib.check(ctx.lib.spev_set_griffinlim_variant(ctx.handle, variant))
-                outs[variant] = sp.griffinlim_flat(S, fb, ctx, n_iter=n_iter, init_phase=ph).clone()
-        finally:
-            _lib.check(ctx.lib.spev_set_griffinlim_variant(ctx.handle, _lib.GL_VARIANT_DEFAULT))
-        assert torch.isfinite(outs[9]).all(), frames
-        assert torch.equal(outs[9], outs[13]), frames
-        a = outs[1].double()
-        # 9 / 13: rolled body, static / dynamic pairs; 25: the default (rsqrt normalisation); 41: straight-line body
-        assert torch.equal(outs[25], outs[89]), frames      # L2 eviction hints change no arithmetic
-        for variant in (9, 25, 41):
-            b = outs[variant].double()
-            off = 0   # per item (a short item must not hide behind a long one)
-            for T in frames:
-                n = (T - 1) * 256
-                if n:
-                    ia, ib = a[off:off + n], b[off:off + n]
-                    err = float((ia - ib).norm() / ia.norm().clamp_min(1e-30))
-                    assert err <= tol, (frames, n_iter, variant, T, err)
-                off += n
+        fused = sp.griffinlim_flat(S, fb, ctx, n_iter=n_iter, init_phase=ph)
+        assert torch.isfinite(fused).all(), frames
+        a = _two_kernel_griffinlim(ctx, fb, S, ph, n_iter).double()
+        b = fused.double()
+        off = 0   # per item (a short item must not hide behind a long one)
+        for T in frames:
+            n = (T - 1) * 256
+            if n:
+                ia, ib = a[off:off + n], b[off:off + n]
+                err = float((ia - ib).norm() / ia.norm().clamp_min(1e-30))
+                assert err <= tol, (frames, n_iter, T, err)
+            off += n
+
+
+def test_unaligned_rows_take_the_unstaged_kernels(cuda):
+    """Rows at ld = 513 (not 16-byte aligned) cannot be bulk-staged into shared memory: spev_griffinlim (S rows),
+    spev_istft (spectrum rows) and spev_gl_phase_update (tprev rows) then take the kernels that read those operands
+    from global memory.  Staging changes where the operands are read from, not the arithmetic: every result is
+    bit-identical to the same rows at ld = 520."""
+    import spev_tts_b200 as sp
+    from spev_tts_b200 import _lib
+    ctx = sp.Context.get(cuda, fmin=0.0, fmax=8000.0)
+    fb = sp.make_batch(ctx, n_frames=[800, 33, 1, 2, 64, 517, 95], with_chunks=True)
+    F, ld = fb.n_frames, _lib.SPEC_LD
+    g = torch.Generator(device=cuda).manual_seed(23)
+    S = torch.rand(F, ld, generator=g, device=cuda)
+    ph = torch.rand(F, 513, generator=g, device=cuda) * 6.2831853
+    X = torch.view_as_complex(torch.randn(F, ld, 2, generator=g, device=cuda))
+    tprev = torch.view_as_complex(torch.randn(F, ld, 2, generator=g, device=cuda))
+
+    def narrow(t):
+        return t[:, :513].contiguous()
+
+    y_s = sp.griffinlim_flat(S, fb, ctx, n_iter=5, init_phase=ph).clone()
+    y_u = sp.griffinlim_flat(narrow(S), fb, ctx, n_iter=5, init_phase=ph).clone()
+    assert torch.isfinite(y_s).all()
+    assert torch.equal(y_s, y_u)
+
+    st = torch.cuda.current_stream(cuda).cuda_stream
+    y = {}
+    for w, spec in ((ld, X), (513, narrow(X))):
+        y[w] = torch.empty(fb.n_out_samples, dtype=torch.float32, device=cuda)
+        _lib.check(ctx.lib.spev_istft(ctx.handle, fb.desc, spec.data_ptr(), w, y[w].data_ptr(), st))
+    assert torch.equal(y[ld], y[513])
+
+    alpha = float(np.float32(0.99 / 1.99))
+    ang, tp = {}, {}
+    for w, s_w, tp_w in ((ld, S, tprev.clone()), (513, narrow(S), narrow(tprev))):
+        ang[w] = torch.zeros(F, w, dtype=torch.complex64, device=cuda)
+        tp[w] = tp_w
+        _lib.check(ctx.lib.spev_gl_phase_update(ctx.handle, fb.desc, y[ld].data_ptr(), s_w.data_ptr(), w, ang[w].data_ptr(),
+                                                tp[w].data_ptr(), w, alpha, 1, st))
+    assert torch.equal(ang[ld][:, :513], ang[513])
+    assert torch.equal(tp[ld][:, :513], tp[513])
 
 
 def test_griffinlim_fused_silent_bins_and_items(cuda):

@@ -16,9 +16,6 @@ S = torch.rand(F, 520, generator=g, device=dev)
 y = torch.zeros(fb.n_out_samples, device=dev)
 st = torch.cuda.current_stream(dev).cuda_stream
 lib = ctx.lib
-variant = int(os.environ.get("GL_VARIANT", "89"))
-_lib.check(lib.spev_set_griffinlim_variant(ctx.handle, variant))
-print("griffinlim variant", variant)
 def t_loop(fn, n=60, reps=5):
     for _ in range(2): 
         for _ in range(n): fn()
@@ -43,11 +40,6 @@ kb = t_loop(both)
 ws = torch.empty(lib.spev_griffinlim_workspace_bytes(F), dtype=torch.uint8, device=dev)
 def full():
     _lib.check(lib.spev_griffinlim(ctx.handle, fb.desc, S.data_ptr(), 520, None, 7, 60, 0.99, y.data_ptr(), ws.data_ptr(), ws.numel(), st))
-for v in (25, 89, 25, 89):
-    _lib.check(lib.spev_set_griffinlim_variant(ctx.handle, v))
-    kv = t_loop(full, n=1, reps=8)
-    print(f"  variant {v}: spev_griffinlim 60 it {kv/1e3:7.3f} ms  {kv/60:6.2f} us/iter  roofline {F*(20516*60+5128)/kv/1e3/6542.1:.3f}")
-_lib.check(lib.spev_set_griffinlim_variant(ctx.handle, variant))
 kf = t_loop(full, n=1, reps=8)
 print(f"B={B} T={T} frames={F} ftiles={fb.n_ftiles} ctiles={fb.n_ctiles}")
 print(f"spev_griffinlim 60 it: {kf/1e3:8.3f} ms  -> {kf/60:6.2f} us/iter  roofline {F*(20516*60+5128)/kf/1e3/6542.1:.3f}")

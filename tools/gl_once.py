@@ -3,14 +3,11 @@ import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 import spev_tts_b200 as sp
-from spev_tts_b200 import _lib
 dev = torch.device("cuda", 0)
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 16
 T = int(sys.argv[2]) if len(sys.argv) > 2 else 800
 n_iter = int(sys.argv[3]) if len(sys.argv) > 3 else 6
 ctx = sp.Context.get(dev, fmin=0.0, fmax=8000.0)
-if "GL_VARIANT" in os.environ:
-    _lib.check(ctx.lib.spev_set_griffinlim_variant(ctx.handle, int(os.environ["GL_VARIANT"])))
 fb = sp.make_batch(ctx, n_frames=[T] * B, with_chunks=True)
 g = torch.Generator(device=dev).manual_seed(0)
 S = torch.rand(fb.n_frames, 520, generator=g, device=dev)
