@@ -59,7 +59,19 @@ typedef struct spev_ctx spev_ctx;
  *     src0 = absolute index in y of the first output sample of chunk t0
  *     row0 = global row of item frame (t0 - 1): the first of the n+3 frames the tile gathers
  *            (one before the item's first row when t0 == 0; never dereferenced then)
- *     lo, hi unused. */
+ *     lo, hi = 0, 0 (what spev_plan_chunk_tiles writes): whole chunks, the item's output is
+ *            (T-1)*hop samples.  hi > lo: absolute bounds of the item's output in y; the ISTFT
+ *            kernels write every sample of [lo, hi) and nothing outside it.
+ *
+ * Output-length layout (librosa's istft / griffinlim `length=`): item i has L_i samples at
+ * absolute offset out_off[i] of y.  Its chunk tiles cover chunks 0 .. ceil(L_i/hop)-1 with
+ * src0 = out_off[i] + hop*t0, lo = out_off[i], hi = out_off[i] + L_i; only the last chunk can be
+ * partial.  Chunk c sums the item frames c-1 .. c+2 that exist: chunk T-1 has frames T-2, T-1,
+ * chunk T has frame T-1, later chunks have none and are written as 0 (librosa's zero padding).
+ * The frame tiles of the same layout (spev_plan_frame_tiles with sample_lo = out_off,
+ * n_samples = L) make spev_stft / spev_gl_phase_update / spev_griffinlim re-analyse exactly
+ * these samples.  Griffin-Lim needs 1 + L_i/hop == T_i, i.e. (T_i-1)*hop <= L_i < T_i*hop.
+ * out_off[i] a multiple of 4 keeps the 16-byte load and store paths. */
 typedef struct spev_tile {
     int64_t src0, lo, hi, row0;
     int32_t n, t0, T /* frames in the item */, item;
@@ -177,7 +189,8 @@ SPEV_API int spev_nnls_objective(spev_ctx* ctx, const void* x, int x_mode, int64
 
 /* ISTFT (irFFT-1024, Hann, gather overlap-add, window-sum-square normalisation).
  *   spec : dev float2 [n_frames, ld] ; y : dev float32, item i at 256*(frame_off[i]-i),
- *   length (T_i-1)*256.   Replaces librosa.istft inside griffinlim (:730-733). */
+ *   length (T_i-1)*256 -- or, with bounded chunk tiles, the output-length layout above.
+ *   Replaces librosa.istft inside griffinlim (:730-733). */
 SPEV_API int spev_istft(spev_ctx* ctx, const spev_batch* batch, const void* spec, int64_t ld, float* y,
                void* stream);
 
@@ -198,7 +211,9 @@ SPEV_API int spev_gl_phase_update(spev_ctx* ctx, const spev_batch* batch, const 
  * Same arithmetic per frame as spev_istft / spev_gl_phase_update, except that the phase normalisation uses a 2-ulp
  * rsqrt and the <= 4 overlap-add terms of a sample are summed pair by pair: agrees with those entry points to rounding.
  *   init_phase : dev float32 [n_frames, 513] radians, or NULL -> 2*pi*U[0,1) from `seed`
- *   y          : dev float32 [256*(n_frames - n_items)]
+ *   y          : dev float32 [256*(n_frames - n_items)]; with bounded chunk tiles (and frame tiles of
+ *                the same layout) item i is [out_off[i], out_off[i] + L_i) instead: librosa's
+ *                griffinlim(length=L_i), every inner istft included; samples between items are not touched
  *   workspace  : dev, >= spev_griffinlim_workspace_bytes(n_frames)
  * Replaces librosa.griffinlim under spev_real_metrics.py:730-733 (n_iter default 32 there,
  * momentum 0.99). */

@@ -12,7 +12,7 @@ CPU, PyTorch-eager or Triton fallback: without the library or without an sm_100 
 raise ``RuntimeError``.
 """
 from ._lib import EXPORTED_SYMBOLS, LIB_PATH, load  # noqa: F401
-from .batch import Context, FlatBatch, make_batch, plan_chunk_tiles, plan_frame_tiles  # noqa: F401
+from .batch import Context, FlatBatch, make_batch, out_layout, plan_chunk_tiles, plan_frame_tiles  # noqa: F401
 from .dataset import (ResidentCache, read_reference_cache, write_metadata, write_records,  # noqa: F401
                       write_reference_cache)
 from .features import frame_features_flat, rms, segment_pool, spectral_centroid  # noqa: F401

@@ -57,20 +57,55 @@ def plan_frame_tiles(frames, sample_lo=None, n_samples=None, tile_frames: int = 
     return out
 
 
-def plan_chunk_tiles(frames, tile_chunks: int = 29) -> np.ndarray:
-    """numpy twin of ``spev_plan_chunk_tiles``: one ``spev_tile`` per <=29-chunk ISTFT tile."""
+def plan_chunk_tiles(frames, tile_chunks: int = 29, *, out_off=None, out_len=None) -> np.ndarray:
+    """numpy twin of ``spev_plan_chunk_tiles``: one ``spev_tile`` per <=29-chunk ISTFT tile.
+
+    With ``out_off`` / ``out_len`` the tiles describe an explicit output layout instead (librosa's ``length=``): item i
+    writes ``out_len[i]`` samples at ``out_off[i]``, ``ceil(out_len[i] / 256)`` chunks, ``lo`` / ``hi`` set to those
+    bounds (see ``include/spev_b200.h``).  Without them ``lo = hi = 0``: the (T-1)*256-sample layout."""
     frames = np.asarray(frames, dtype=np.int64)
     fo = np.concatenate([[0], np.cumsum(frames)])[:-1]
-    nc = np.maximum(frames - 1, 0)
+    if (out_off is None) != (out_len is None):
+        raise ValueError("out_off and out_len go together")
+    if out_len is None:
+        nc = np.maximum(frames - 1, 0)
+        start = HOP * (fo - np.arange(len(frames)))
+    else:
+        lens = np.asarray(out_len, dtype=np.int64).reshape(-1)
+        start = np.asarray(out_off, dtype=np.int64).reshape(-1)
+        nc = (lens + HOP - 1) // HOP
     item, c0 = _split(nc, tile_chunks)
     out = np.zeros(len(item), dtype=TILE_DTYPE)
-    out["src0"] = HOP * (fo[item] - item) + HOP * c0
+    out["src0"] = start[item] + HOP * c0
+    if out_len is not None:
+        out["lo"], out["hi"] = start[item], start[item] + lens[item]
     out["row0"] = fo[item] + c0 - 1
     out["n"] = np.minimum(tile_chunks, nc[item] - c0)
     out["t0"], out["T"], out["item"] = c0, frames[item], item
     # full tiles first, partial tiles last (same order as the C planner): tile j runs on CTA j mod grid, so the
     # cheap tiles fall into the last, incomplete round
     return out[np.argsort(out["n"] < tile_chunks, kind="stable")]
+
+
+def out_layout(frames, out_len, out_off=None):
+    """Output layout of a batch with explicit per-item output lengths -> (``out_off`` int64 [n_items], ``out_len`` int64
+    [n_items]).  ``out_len`` is one length per item (or one for all).  Default offsets pack the items in order, each
+    starting at a multiple of 4 samples (the kernels' 16-byte paths); given offsets must keep the items apart."""
+    frames = np.asarray(frames, dtype=np.int64).reshape(-1)
+    lens = np.broadcast_to(np.asarray(out_len, dtype=np.int64), frames.shape).copy()
+    if (lens < 0).any():
+        raise ValueError("output lengths must be >= 0")
+    if out_off is None:
+        padded = (lens + 3) // 4 * 4
+        off = np.concatenate([[0], np.cumsum(padded)])[:-1].astype(np.int64)
+    else:
+        off = np.asarray(out_off, dtype=np.int64).reshape(-1)
+        if off.shape != frames.shape:
+            raise ValueError(f"out_off needs one offset per item ({len(frames)}), got {off.shape}")
+        order = np.argsort(off, kind="stable")
+        if (off < 0).any() or (off[order][1:] < (off + lens)[order][:-1]).any():
+            raise ValueError("out_off: item outputs must not be negative or overlap")
+    return off, lens
 
 
 class Context:
@@ -114,16 +149,19 @@ class Context:
                 cls._cache[key] = ctx
         return ctx
 
-    def uniform_batch(self, n_items: int, n_frames: int, with_chunks: bool = True) -> "FlatBatch":
+    def uniform_batch(self, n_items: int, n_frames: int, with_chunks: bool = True,
+                      out_len: Optional[int] = None) -> "FlatBatch":
         """Descriptor of ``n_items`` equal-length spectrogram items, cached: the vocoder is called over and over with
-        the same shapes, and planning + pinned staging + upload cost more than the kernels of a short utterance."""
-        key = (int(n_items), int(n_frames), bool(with_chunks))
+        the same shapes, and planning + pinned staging + upload cost more than the kernels of a short utterance.
+        ``out_len``: output samples per item (librosa's ``length=``; default layout when None)."""
+        key = (int(n_items), int(n_frames), bool(with_chunks), None if out_len is None else int(out_len))
         cache = self.__dict__.setdefault("_uniform", {})
         fb = cache.get(key)
         if fb is None:
             if len(cache) >= 64:
                 cache.pop(next(iter(cache)))
-            fb = cache[key] = make_batch(self, n_frames=[n_frames] * n_items, with_chunks=with_chunks)
+            fb = cache[key] = make_batch(self, n_frames=[n_frames] * n_items, with_chunks=with_chunks,
+                                         out_len=None if out_len is None else [out_len] * n_items)
         return fb
 
     def side_stream(self) -> "torch.cuda.Stream":
@@ -178,25 +216,47 @@ class FlatBatch:
     table: torch.Tensor         # device uint8 buffer holding frame_off + tile tables
     desc: _lib.SpevBatch
     device: torch.device
+    out_off: Optional[np.ndarray] = None   # int64 [n_items] ISTFT output starts (explicit output layout), else None
+    out_len: Optional[np.ndarray] = None   # int64 [n_items] ISTFT output lengths (explicit output layout), else None
 
     @property
     def n_out_samples(self) -> int:
-        """total ISTFT output length: sum (T_i - 1) * hop"""
+        """size of the flat ISTFT output buffer: sum (T_i - 1) * hop, or the end of the last item of an explicit
+        output layout"""
+        if self.out_len is not None:
+            return int((self.out_off + self.out_len).max(initial=0))
         return int((self.n_frames - self.n_items) * HOP)
 
     def out_sample_off(self) -> np.ndarray:
+        """[n_items + 1]: item i's output starts at entry i; the last entry is ``n_out_samples``.  Items are back to
+        back in the default layout; an explicit layout (``out_len``) may leave gaps, which no kernel writes."""
+        if self.out_len is not None:
+            return np.append(self.out_off, self.n_out_samples).astype(np.int64)
         return (self.frame_off - np.arange(self.n_items + 1)) * HOP
+
+    def out_lengths(self) -> np.ndarray:
+        """[n_items] ISTFT output samples per item: (T_i - 1) * hop, or the explicit lengths."""
+        if self.out_len is not None:
+            return self.out_len.copy()
+        return np.maximum(self.frames - 1, 0) * HOP
 
 
 def make_batch(ctx: Context, *, n_samples: Optional[Sequence[int]] = None,
                n_frames: Optional[Sequence[int]] = None, sample_off: Optional[np.ndarray] = None,
-               with_chunks: bool = False, pinned: bool = True) -> FlatBatch:
+               with_chunks: bool = False, pinned: bool = True, out_len=None,
+               out_off: Optional[Sequence[int]] = None) -> FlatBatch:
     """Build the descriptor for items given by sample counts (waveform inputs) or frame counts
     (spectrogram inputs; sample tiles then describe the implicit ISTFT-output layout).
     ``sample_off[i]`` is the absolute start of item i in the flat sample buffer (default: items
     packed back to back).  Starts that are multiples of 4 samples take the 16-byte cp.async path;
-    whatever lies between items is never read as signal (explicit [lo, hi) bounds per item)."""
+    whatever lies between items is never read as signal (explicit [lo, hi) bounds per item).
+    ``out_len`` (spectrogram inputs only): item i's ISTFT output has ``out_len[i]`` samples at ``out_off[i]``
+    (librosa's ``length=``; see ``out_layout`` for the default offsets); frame and chunk tiles follow that layout."""
     dev = torch.device("cuda", ctx.device)
+    if out_off is not None and out_len is None:
+        raise ValueError("out_off needs out_len")
+    if out_len is not None and n_samples is not None:
+        raise ValueError("out_len describes ISTFT outputs: give n_frames, not n_samples")
     if n_samples is not None:
         ns = np.asarray(n_samples, dtype=np.int64).reshape(-1)
         frames = 1 + ns // HOP
@@ -208,10 +268,13 @@ def make_batch(ctx: Context, *, n_samples: Optional[Sequence[int]] = None,
     else:
         frames = np.asarray(n_frames, dtype=np.int64).reshape(-1)
         sample_off = None
-        ftiles = plan_frame_tiles(frames, None, None, ctx.tile_frames)
+        if out_len is not None:
+            out_off, out_len = out_layout(frames, out_len, out_off)
+        ftiles = plan_frame_tiles(frames, out_off, out_len, ctx.tile_frames)
     n_items = int(len(frames))
     frame_off = np.concatenate([[0], np.cumsum(frames)]).astype(np.int64)
-    ctiles = plan_chunk_tiles(frames, ctx.tile_chunks) if with_chunks else np.zeros(0, dtype=TILE_DTYPE)
+    ctiles = (plan_chunk_tiles(frames, ctx.tile_chunks, out_off=out_off, out_len=out_len) if with_chunks
+              else np.zeros(0, dtype=TILE_DTYPE))
 
     # one staging buffer: [ftiles | ctiles | frame_off]; tile tables first (16-byte aligned)
     parts = [ftiles.view(np.uint8).reshape(-1), ctiles.view(np.uint8).reshape(-1),
@@ -233,6 +296,6 @@ def make_batch(ctx: Context, *, n_samples: Optional[Sequence[int]] = None,
     d.frame_off = base + sizes[0] + sizes[1]
     fb = FlatBatch(n_items=n_items, n_frames=int(frame_off[-1]), frames=frames,
                    sample_off=sample_off, frame_off=frame_off, n_ftiles=len(ftiles),
-                   n_ctiles=len(ctiles), table=table, desc=d, device=dev)
+                   n_ctiles=len(ctiles), table=table, desc=d, device=dev, out_off=out_off, out_len=out_len)
     fb._host = host   # keep the pinned staging buffer alive until the async copy is consumed
     return fb

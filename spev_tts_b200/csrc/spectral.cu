@@ -8,6 +8,8 @@
 //                   gather overlap-add (each output sample owner sums its <= 4 frames in
 //                   ascending frame order, no atomics) fused with window-sum-square
 //                   normalisation.            Replaces librosa.istft under :730-733.
+//                   Chunk tiles with hi > lo bound the output explicitly (librosa's istft(length=)):
+//                   every sample of [lo, hi) is written, nothing outside it.
 // K5 k_stft_phase_w : STFT of the rebuilt signal fused with Griffin-Lim's momentum / phase
 //                   normalisation update, one frame pair per warp.  Replaces librosa.stft + the angle
 //                   update lines of librosa.griffinlim under :730-733.
@@ -726,6 +728,11 @@ k_gl_fused(BatchView bv, const float* __restrict__ y, const float* __restrict__ 
 
 // ---------------------------------------------------------------------------------------
 // K4: ISTFT with gather overlap-add and window-sum-square normalisation
+//
+// Output chunk c (samples [256c, 256c + 256) of the item) sums frames c-1 .. c+2 that exist.  Without an explicit
+// bound an item has chunks 0 .. T-2.  With one (hi > lo: librosa's istft(length=L), ceil(L / 256) chunks) it may also
+// have chunk T-1 (frames T-2, T-1), chunk T (frame T-1) and later chunks with no frame, written as 0; all of them take
+// the per-sample edge normalisation.  Only the item's last chunk can be partial, and only its stores are masked.
 // ---------------------------------------------------------------------------------------
 // BULK: a warp's two spectrum rows (8,272 B) arrive in its region by ONE bulk asynchronous copy instead of 34 scattered
 // 8-byte loads per lane (ncu r01: lg_throttle 1.2 + long_scoreboard 1.7 warps per issue cycle on those loads): no LSU
@@ -845,10 +852,13 @@ k_istft(BatchView bv, const float2* __restrict__ spec, int64_t ld, float* __rest
             });
         }
         __syncthreads();
-        // gather: chunk c = c0 + cl receives frames c-1, c, c+1, c+2 (ascending), local cl..cl+3
+        // gather: chunk c = c0 + cl receives frames c-1, c, c+1, c+2 (ascending), local cl..cl+3.  An explicit output
+        // bound (hi > lo) may end inside the item's last chunk: only that chunk stores fewer than kHop samples.
         for (int cl = warp; cl < nchunks; cl += kWarps) {
             const int c = c0 + cl;
             float* yo_c = y + d.src0 + static_cast<int64_t>(cl) * kHop;
+            const int nv = d.hi > d.lo ? static_cast<int>(min(static_cast<int64_t>(kHop), d.hi - d.src0 - static_cast<int64_t>(cl) * kHop))
+                                       : kHop;
             if (c >= 1 && c + 2 < T) {   // all four frames exist: table-driven normalisation
                 const float* f0 = s_x + (cl >> 1) * kWarpRegionWords + (cl & 1) * kNfft + lane;
                 const float* f1 = s_x + ((cl + 1) >> 1) * kWarpRegionWords + ((cl + 1) & 1) * kNfft + lane;
@@ -858,7 +868,7 @@ k_istft(BatchView bv, const float2* __restrict__ spec, int64_t ld, float* __rest
                 for (int ii = 0; ii < kHop / 32; ++ii) {
                     const int o = 32 * ii;
                     const float sum = ((f0[768 + o] + f1[512 + o]) + f2[256 + o]) + f3[o];
-                    yo_c[lane + o] = sum * s_iw[lane + o];
+                    if (lane + o < nv) yo_c[lane + o] = sum * s_iw[lane + o];
                 }
                 continue;
             }
@@ -877,7 +887,7 @@ k_istft(BatchView bv, const float2* __restrict__ spec, int64_t ld, float* __rest
                         wss = fmaf(w, w, wss);
                     }
                 }
-                yo_c[s] = wss > kTiny ? sum / wss : sum;
+                if (s < nv) yo_c[s] = wss > kTiny ? sum / wss : sum;
             }
         }
     }
@@ -892,6 +902,9 @@ k_istft(BatchView bv, const float2* __restrict__ spec, int64_t ld, float* __rest
 // j with 0 <= q - 2j <= 4 -- two or three of them --, summed here in ascending pair order and normalised by the
 // window-sum-square exactly as k_istft does (table for interior chunks, per-sample sum over the existing frames at
 // the item edges).  One warp per chunk, 16-byte loads and stores, no shared-memory staging: a pure streaming kernel.
+// With an explicit output bound (chunk tiles with hi > lo) an item may also have chunk T-1 (frames T-2, T-1: pairs
+// covering them are selected by the same rule, a lone last frame included) and chunk T (frame T-1 alone); later chunks
+// meet no segment and are written as 0.  Only the item's last chunk can be partial; it stores sample by sample.
 // ---------------------------------------------------------------------------------------
 constexpr int kOlaWarps = 8;
 constexpr int kOlaPerWarp = 1;                                           // chunks per warp (2 measured: no gain)
@@ -909,11 +922,14 @@ k_ola_pairs(BatchView bv, const float* __restrict__ seg, int64_t ld_f, float* __
     if (cl0 >= n) return;
     const int t0 = __ldg(&d->t0), T = __ldg(&d->T);
     const int64_t item_row = __ldg(&d->row0) - t0 + 1;
-    float* yo0 = y + __ldg(&d->src0);
+    const int64_t src0 = __ldg(&d->src0);
+    float* yo0 = y + src0;
+    // an explicit output bound (hi > lo) that ends inside this warp's chunks: kept as one predicate, the exact count is
+    // re-read from the descriptor only on that path
+    const bool bounded_tail = __ldg(&d->hi) > __ldg(&d->lo) &&
+                              __ldg(&d->hi) - src0 - static_cast<int64_t>(cl0) * kHop < kOlaPerWarp * kHop;
     const int n_pairs = (T + 1) >> 1;
     const int s0 = 4 * lane, s1 = 128 + 4 * lane;
-    // constant tables before the wait: they do not depend on the previous kernel
-    const float4 w0 = __ldg(reinterpret_cast<const float4*>(g_iw + s0)), w1 = __ldg(reinterpret_cast<const float4*>(g_iw + s1));
     pdl_wait();   // the segments come from the previous kernel
     float4 p0[kOlaPerWarp][3], p1[kOlaPerWarp][3];
 #pragma unroll
@@ -944,6 +960,9 @@ k_ola_pairs(BatchView bv, const float* __restrict__ seg, int64_t ld_f, float* __
         const int c = t0 + cl0 + e;
         float4 r0 = add3(p0[e]), r1 = add3(p1[e]);
         if (c >= 1 && c + 2 < T) {
+            // 1 / sum w^2 (constant table) read here, not before the wait: held across the segment loads it would take the
+            // registers the masked tail stores need, and 52 instead of 48 registers cost one 256-thread CTA per SM
+            const float4 w0 = __ldg(reinterpret_cast<const float4*>(g_iw + s0)), w1 = __ldg(reinterpret_cast<const float4*>(g_iw + s1));
             r0 = make_float4(r0.x * w0.x, r0.y * w0.y, r0.z * w0.z, r0.w * w0.w);
             r1 = make_float4(r1.x * w1.x, r1.y * w1.y, r1.z * w1.z, r1.w * w1.w);
         } else {
@@ -960,15 +979,27 @@ k_ola_pairs(BatchView bv, const float* __restrict__ seg, int64_t ld_f, float* __
             r1 = make_float4(norm(r1.x, s1), norm(r1.y, s1 + 1), norm(r1.z, s1 + 2), norm(r1.w, s1 + 3));
         }
         float* yo = yo0 + static_cast<int64_t>(cl0 + e) * kHop;
-        if ((reinterpret_cast<uintptr_t>(yo) & 15) == 0) {   // y is read back by the next kernel: keep it in L2
+        if (!bounded_tail && (reinterpret_cast<uintptr_t>(yo) & 15) == 0) {   // y is read back by the next kernel: keep it in L2
             const uint64_t pol = l2_policy_evict_last();
             asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %2, %3, %4}, %5;\n" ::"l"(reinterpret_cast<float4*>(yo) + lane),
                          "f"(r0.x), "f"(r0.y), "f"(r0.z), "f"(r0.w), "l"(pol) : "memory");
             asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %2, %3, %4}, %5;\n" ::"l"(reinterpret_cast<float4*>(yo) + 32 + lane),
                          "f"(r1.x), "f"(r1.y), "f"(r1.z), "f"(r1.w), "l"(pol) : "memory");
-        } else {
-            yo[s0] = r0.x; yo[s0 + 1] = r0.y; yo[s0 + 2] = r0.z; yo[s0 + 3] = r0.w;
-            yo[s1] = r1.x; yo[s1 + 1] = r1.y; yo[s1 + 2] = r1.z; yo[s1 + 3] = r1.w;
+        } else {   // unaligned, or the item's partial last chunk
+            int nv = kHop;                       // samples of this chunk inside the item's output
+            if (bounded_tail) {
+                const spev_tile* dt = bv.ctiles + blockIdx.x / kOlaParts;
+                nv = static_cast<int>(max(static_cast<int64_t>(0), min(static_cast<int64_t>(kHop),
+                                                                      __ldg(&dt->hi) - __ldg(&dt->src0) - static_cast<int64_t>(cl0 + e) * kHop)));
+            }
+            if (s0 < nv) yo[s0] = r0.x;
+            if (s0 + 1 < nv) yo[s0 + 1] = r0.y;
+            if (s0 + 2 < nv) yo[s0 + 2] = r0.z;
+            if (s0 + 3 < nv) yo[s0 + 3] = r0.w;
+            if (s1 < nv) yo[s1] = r1.x;
+            if (s1 + 1 < nv) yo[s1 + 1] = r1.y;
+            if (s1 + 2 < nv) yo[s1 + 2] = r1.z;
+            if (s1 + 3 < nv) yo[s1 + 3] = r1.w;
         }
     }
 }

@@ -185,23 +185,48 @@ def stft(y: ArrayLike, *, n_fft=2048, hop_length=None, win_length=None, window="
     return _ret(out, was_numpy)
 
 
+def _check_length(length) -> Optional[int]:
+    if length is None:
+        return None
+    if isinstance(length, (bool, np.bool_)) or not isinstance(length, (int, np.integer)) or length < 0:
+        raise ValueError(f"length must be a non-negative integer or None, got {length!r}")
+    return int(length)
+
+
+def _gl_length(length, T: int) -> Optional[int]:
+    """librosa's Griffin-Lim loop re-analyses each istft(length=L) output and needs T frames back: 1 + L // hop == T."""
+    length = _check_length(length)
+    if length is not None and 1 + length // HOP != T:
+        raise ValueError(f"length={length} is outside [{(T - 1) * HOP}, {T * HOP - 1}], the lengths whose STFT has the "
+                         f"T={T} frames of the input (librosa's Griffin-Lim loop needs 1 + length // {HOP} == T)")
+    return length
+
+
+def _unpack_items(y: torch.Tensor, b: int, L: int, pitch: int) -> torch.Tensor:
+    """Uniform items of ``L`` samples, item i at ``i * pitch`` of the flat buffer ``y`` (>= b * pitch) -> ``[b, L]``."""
+    out = y[: b * pitch].view(b, pitch)
+    return out if pitch == L else out[:, :L].contiguous()
+
+
 def istft(X: ArrayLike, *, hop_length=None, win_length=None, n_fft=None, window="hann", center=True,
           dtype=None, length=None, device=None):
-    """Drop-in for ``librosa.istft`` -> float32 ``[..., (T-1)*hop]``."""
+    """Drop-in for ``librosa.istft`` -> float32 ``[..., (T-1)*hop]``, or ``[..., length]`` with librosa's crop / zero
+    padding (any ``length >= 0``).  The kernels write exactly ``length`` samples per item."""
     nb = X.shape[-2]
     _check_fixed(n_fft or 2 * (nb - 1), hop_length, win_length, window, center, "constant")
-    if length is not None:
-        raise NotImplementedError("istft(length=...) is not on the reference path")
+    length = _check_length(length)
     t, was_numpy = _to_device(X, device, dtype=torch.complex64)
     lead, T = t.shape[:-2], t.shape[-1]
     b = int(np.prod(lead)) if lead else 1
     ctx = Context.get(t.device)
-    batch = make_batch(ctx, n_frames=[T] * b, with_chunks=True)
+    L = (T - 1) * HOP if length is None else length
+    batch = make_batch(ctx, n_frames=[T] * b, with_chunks=True, out_len=None if length is None else [L] * b)
     spec = _spec_to_internal(t.reshape(b, nb, T))
-    y = torch.empty(batch.n_out_samples, dtype=torch.float32, device=t.device)
+    pitch = int(batch.out_sample_off()[1] - batch.out_sample_off()[0]) if b > 1 else L
+    y = torch.empty(max(batch.n_out_samples, b * pitch), dtype=torch.float32, device=t.device)
     _lib.check(ctx.lib.spev_istft(ctx.handle, batch.desc, spec.data_ptr(), _lib.SPEC_LD, y.data_ptr(),
                                   stream_ptr(t.device)), "spev_istft")
-    return _ret(y.view(*lead, (T - 1) * HOP), was_numpy)
+    return _ret(_unpack_items(y, b, L, pitch).view(*lead, L), was_numpy)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -346,8 +371,15 @@ def griffinlim_flat(S: torch.Tensor, batch: FlatBatch, ctx: Context, *, n_iter=3
                     init_phase: Optional[torch.Tensor] = None, seed: int = 0,
                     out: Optional[torch.Tensor] = None, workspace: Optional[torch.Tensor] = None):
     """``S``: ``[F, 520]`` float32 magnitudes; ``init_phase``: ``[F, 513]`` float32 radians or None.
-    Returns the flat waveform buffer (item i at ``batch.out_sample_off()[i]``)."""
+    Returns the flat waveform buffer (item i at ``batch.out_sample_off()[i]``, ``batch.out_lengths()[i]`` samples).
+    A batch built with ``out_len`` runs librosa's ``griffinlim(length=out_len[i])`` per item: every inner ISTFT writes
+    those samples and the next STFT re-analyses them; each length must satisfy ``1 + out_len[i] // 256 == T_i``."""
     lib = ctx.lib
+    if batch.out_len is not None:
+        bad = np.flatnonzero(1 + batch.out_len // HOP != batch.frames)
+        if len(bad):
+            i = int(bad[0])
+            _gl_length(int(batch.out_len[i]), int(batch.frames[i]))      # raises, naming the valid range
     need = lib.spev_griffinlim_workspace_bytes(batch.n_frames)
     if workspace is None or workspace.numel() < need:
         workspace = torch.empty(need, dtype=torch.uint8, device=S.device)
@@ -369,24 +401,30 @@ def _phase_to_internal(init_phase: ArrayLike, b: int, T: int, device) -> torch.T
 def griffinlim(S: ArrayLike, *, n_iter=32, hop_length=None, win_length=None, n_fft=None, window="hann",
                center=True, dtype=None, length=None, pad_mode="constant", momentum=0.99, init="random",
                random_state=None, init_phase: Optional[ArrayLike] = None, device=None):
-    """Drop-in for ``librosa.griffinlim`` (``[..., 513, T]`` magnitudes -> ``[..., (T-1)*hop]``).
+    """Drop-in for ``librosa.griffinlim`` (``[..., 513, T]`` magnitudes -> ``[..., (T-1)*hop]``, or ``[..., length]``
+    for ``(T-1)*hop <= length < T*hop``: librosa passes ``length`` to every inner istft, so the tail samples are
+    rebuilt and re-analysed in each iteration).
     ``init_phase`` (radians, same shape as S) pins the starting phases for parity tests;
     otherwise phases are drawn on the device from ``random_state`` (None -> OS entropy, like
     librosa)."""
     nb = S.shape[-2]
     _check_fixed(n_fft or 2 * (nb - 1), hop_length, win_length, window, center, pad_mode)
-    if length is not None or init not in ("random",):
-        raise NotImplementedError("griffinlim: only init='random', length=None are on the reference path")
+    if init not in ("random",):
+        raise NotImplementedError("griffinlim: only init='random' is on the reference path")
+    length = _gl_length(length, S.shape[-1])
     t, was_numpy = _to_device(S, device)
     lead, T = t.shape[:-2], t.shape[-1]
     b = int(np.prod(lead)) if lead else 1
     ctx = Context.get(t.device)
-    batch = make_batch(ctx, n_frames=[T] * b, with_chunks=True)
+    L = (T - 1) * HOP if length is None else length
+    batch = make_batch(ctx, n_frames=[T] * b, with_chunks=True, out_len=None if length is None else [L] * b)
     Sf = items_to_rows(t.reshape(b, nb, T), _lib.SPEC_LD, out=torch.zeros((b * T, _lib.SPEC_LD), dtype=torch.float32, device=t.device))
     ph = _phase_to_internal(init_phase, b, T, t.device) if init_phase is not None else None
     seed = int(np.random.SeedSequence(random_state).generate_state(2, dtype=np.uint32).view(np.uint64)[0])
-    y = griffinlim_flat(Sf, batch, ctx, n_iter=n_iter, momentum=momentum, init_phase=ph, seed=seed)
-    return _ret(y.view(*lead, (T - 1) * HOP), was_numpy)
+    pitch = int(batch.out_sample_off()[1] - batch.out_sample_off()[0]) if b > 1 else L
+    y = torch.empty(max(batch.n_out_samples, b * pitch), dtype=torch.float32, device=t.device)
+    y = griffinlim_flat(Sf, batch, ctx, n_iter=n_iter, momentum=momentum, init_phase=ph, seed=seed, out=y)
+    return _ret(_unpack_items(y, b, L, pitch).view(*lead, L), was_numpy)
 
 
 def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_length=None, window="hann",
@@ -394,19 +432,21 @@ def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_len
                  fmin=0.0, fmax=None, momentum=0.99, init_phase: Optional[ArrayLike] = None,
                  random_state=None, is_log=False, nnls="librosa", device=None):
     """Drop-in for ``librosa.feature.inverse.mel_to_audio`` (call site
-    ``spev_real_metrics.py:730-733``): ``[..., n_mels, T]`` mel power -> ``[..., (T-1)*hop]``.
+    ``spev_real_metrics.py:730-733``): ``[..., n_mels, T]`` mel power -> ``[..., (T-1)*hop]``, or ``[..., length]``
+    for ``(T-1)*hop <= length < T*hop`` (copy-synthesis: ``length=len(y)`` of the source signal; see ``griffinlim``).
     ``is_log=True`` fuses the reference's ``np.exp`` (``:729``) into the first kernel.  ``nnls``: see ``mel_to_stft``
     (``"pinv"`` keeps the whole call free of host synchronisation)."""
     _check_fixed(n_fft, hop_length, win_length, window, center, pad_mode, power)
     if nnls not in ("librosa", "pinv"):
         raise ValueError("nnls must be 'librosa' or 'pinv'")
-    if length is not None:
-        raise NotImplementedError("mel_to_audio(length=...) is not on the reference path")
+    length = _gl_length(length, M.shape[-1])
     t, was_numpy = _to_device(M, device)
     lead, n_mels, T = t.shape[:-2], t.shape[-2], t.shape[-1]
     b = int(np.prod(lead)) if lead else 1
     ctx = Context.get(t.device, sr=sr, n_mels=n_mels, fmin=fmin, fmax=fmax)
-    batch = ctx.uniform_batch(b, T, with_chunks=True)
+    L = (T - 1) * HOP if length is None else length
+    batch = ctx.uniform_batch(b, T, with_chunks=True, out_len=length)
+    pitch = int(batch.out_sample_off()[1] - batch.out_sample_off()[0]) if b > 1 else L
     tm = items_to_rows(t.reshape(b, n_mels, T)).view(-1)                  # frame-major -> tensor-core GEMM
     S = mel_to_mag_flat(tm, batch, ctx, layout=0, is_log=is_log)
     ph = _phase_to_internal(init_phase, b, T, t.device) if init_phase is not None else None
@@ -414,7 +454,9 @@ def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_len
     out = {}
 
     def run_gl():
-        out["y"] = griffinlim_flat(S, batch, ctx, n_iter=n_iter, momentum=momentum, init_phase=ph, seed=seed, out=out.get("y"))
+        if "y" not in out:
+            out["y"] = torch.empty(max(batch.n_out_samples, b * pitch), dtype=torch.float32, device=t.device)
+        griffinlim_flat(S, batch, ctx, n_iter=n_iter, momentum=momentum, init_phase=ph, seed=seed, out=out["y"])
     if nnls == "librosa" and b * T > 0:
         # Griffin-Lim is enqueued on the warm start while the host fetches the screening result; in the (rare: short
         # utterances, short remainder blocks) case that librosa's solver iterates, S is refined and the loop redone
@@ -422,5 +464,4 @@ def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_len
             run_gl()
     else:
         run_gl()
-    y = out["y"]
-    return _ret(y.view(*lead, (T - 1) * HOP), was_numpy)
+    return _ret(_unpack_items(out["y"], b, L, pitch).view(*lead, L), was_numpy)

@@ -1,0 +1,139 @@
+"""CPU tests of ``length=`` (librosa's exact-length inverse transforms): the restated istft against torch.istft, the
+Griffin-Lim loop with ``length`` against torchaudio, and the host planner of the output-length layout."""
+import numpy as np
+import pytest
+import torch
+
+from oracle import librosa_restated as lr
+from spev_tts_b200 import batch as B
+from tests import length_ref, synth
+
+
+def _lengths(T):
+    """Shorter than (T-1)*256 (frames drop), (T-1)*256, +1, T*256 - 1, and longer than the signal (zero padding)."""
+    full = (T - 1) * 256
+    out = [full - 300, full - 1, full, full + 1, T * 256 - 1, (T + 1) * 256, (T + 3) * 256 + 17]
+    return sorted({L for L in out if L > 0})
+
+
+@pytest.mark.parametrize("T", [1, 2, 3, 33, 100])
+def test_istft_length_vs_torch_float64(T):
+    rng = np.random.default_rng(T)
+    X = rng.standard_normal((513, T)) + 1j * rng.standard_normal((513, T))
+    w = torch.hann_window(1024, periodic=True, dtype=torch.float64)
+    for L in _lengths(T):
+        got = lr.istft(X, hop_length=256, n_fft=1024, dtype=np.float64, length=L)
+        ref = torch.istft(torch.from_numpy(X), 1024, 256, 1024, w, center=True, length=L).numpy()
+        assert got.shape == ref.shape == (L,)
+        assert np.abs(got - ref).max() <= 1e-6 * max(1.0, np.abs(ref).max()), (T, L)
+        if L > (T + 1) * 256:
+            assert not got[(T + 1) * 256:].any()                 # zero padding past the last frame
+
+
+def test_istft_length_zero_is_empty():
+    rng = np.random.default_rng(0)
+    X = (rng.standard_normal((2, 513, 5)) + 1j * rng.standard_normal((2, 513, 5))).astype(np.complex64)
+    y = lr.istft(X, hop_length=256, n_fft=1024, length=0)
+    assert y.shape == (2, 0) and y.dtype == np.float32
+
+
+def test_griffinlim_length_loop_against_torchaudio(monkeypatch):
+    """The loop with ``length`` against torchaudio's griffinlim(length=...), which also passes the length to every
+    inner istft.  As in test_oracle.py's loop test, the re-analysis is swapped for a reflect-padded stft (torchaudio's
+    padding) for this comparison only."""
+    import torchaudio
+    T, n_iter = 60, 8
+    plain_stft = lr.stft
+
+    def stft_reflect(y, *, n_fft=2048, hop_length=None, **kw):
+        pad = [(0, 0)] * (np.ndim(y) - 1) + [(n_fft // 2, n_fft // 2)]
+        return plain_stft(np.pad(y, pad, mode="reflect"), n_fft=n_fft, hop_length=hop_length, center=False)
+    for L in ((T - 1) * 256, (T - 1) * 256 + 1, (T - 1) * 256 + 100, T * 256 - 1):
+        y0 = synth.speechy(seed=78, n=L)
+        S = np.abs(plain_stft(y0, n_fft=1024, hop_length=256)).astype(np.float32)
+        assert S.shape == (513, T)
+        monkeypatch.setattr(lr, "stft", stft_reflect)
+        got = length_ref.griffinlim(S, n_iter=n_iter, init_phase=np.zeros(S.shape), length=L)
+        monkeypatch.setattr(lr, "stft", plain_stft)
+        ref = torchaudio.functional.griffinlim(torch.from_numpy(S).double(), torch.hann_window(1024, periodic=True, dtype=torch.float64),
+                                               n_fft=1024, hop_length=256, win_length=1024, power=1.0, n_iter=n_iter,
+                                               momentum=0.99, length=L, rand_init=False).numpy()
+        assert got.shape == ref.shape == (L,)
+        err = np.linalg.norm(got - ref) / np.linalg.norm(ref)
+        assert err <= 1e-4, (L, err)
+
+
+def test_griffinlim_length_of_whole_chunks_is_the_default():
+    g = synth.speechy(seed=79, n=40 * 256)
+    S = np.abs(lr.stft(g, n_fft=1024, hop_length=256)).astype(np.float32)        # [513, 41]
+    ph = synth.init_phase(S.shape, seed=80)
+    plain = lr.griffinlim(S, n_iter=4, hop_length=256, n_fft=1024, init_phase=ph)
+    assert np.array_equal(length_ref.griffinlim(S, n_iter=4, init_phase=ph), plain)
+    assert np.array_equal(length_ref.griffinlim(S, n_iter=4, init_phase=ph, length=40 * 256), plain)
+    tail = length_ref.griffinlim(S, n_iter=4, init_phase=ph, length=40 * 256 + 200)
+    assert tail.shape == (40 * 256 + 200,) and np.abs(tail[40 * 256:]).max() > 0
+    assert not np.array_equal(tail[: 40 * 256], plain)         # the tail is re-analysed in every iteration
+
+
+def test_length_planner_covers_every_sample_once():
+    rng = np.random.default_rng(5)
+    for trial in range(20):
+        n = int(rng.integers(1, 12))
+        frames = rng.integers(1, 200, n)
+        lens = rng.integers(0, 260 * 200, n) if trial % 2 else (frames - 1) * 256 + rng.integers(0, 256, n)
+        if trial % 4 == 3:          # explicit, unaligned offsets with gaps
+            gaps = rng.integers(0, 50, n)
+            offs = np.cumsum(np.concatenate([[0], lens[:-1] + gaps[:-1]])) + gaps[0]
+            off, L = B.out_layout(frames, lens, offs)
+            assert np.array_equal(off, offs)
+        else:
+            off, L = B.out_layout(frames, lens)
+            assert (off % 4 == 0).all() and off[0] == 0
+        tiles = B.plan_chunk_tiles(frames, 29, out_off=off, out_len=L)
+        end = int((off + L).max(initial=0)) + 300
+        count = np.zeros(end + 29 * 256, dtype=np.int64)
+        for t in tiles:
+            i = t["item"]
+            assert t["lo"] == off[i] and t["hi"] == off[i] + L[i] and t["T"] == frames[i]
+            assert t["src0"] == off[i] + 256 * t["t0"] and 1 <= t["n"] <= 29
+            assert t["row0"] == frames[:i].sum() + t["t0"] - 1
+            a = int(t["src0"])
+            b = min(a + 256 * int(t["n"]), int(t["hi"]))
+            assert b > a + 256 * (int(t["n"]) - 1)            # only the last chunk of an item may be partial
+            count[a:b] += 1
+        want = np.zeros_like(count)
+        for i in range(n):
+            want[off[i]: off[i] + L[i]] += 1
+        assert np.array_equal(count, want), trial
+        full = tiles["n"] == 29
+        assert not (full[1:] & ~full[:-1]).any()               # full tiles first
+        ft = B.plan_frame_tiles(frames, off, L)
+        assert np.array_equal(ft["lo"], off[ft["item"]]) and np.array_equal(ft["hi"], (off + L)[ft["item"]])
+    # without a layout: byte-identical to the plain planner (lo = hi = 0)
+    frames = np.array([800, 33, 1, 2, 64])
+    assert B.plan_chunk_tiles(frames, 29).tobytes() == B.plan_chunk_tiles(frames).tobytes()
+    assert not B.plan_chunk_tiles(frames)["hi"].any()
+
+
+def test_out_layout_rejects_bad_layouts():
+    with pytest.raises(ValueError):
+        B.out_layout([3, 3], [-1, 5])
+    with pytest.raises(ValueError):
+        B.out_layout([3, 3], [600, 600], [0, 599])             # overlapping items
+    with pytest.raises(ValueError):
+        B.out_layout([3, 3], [600, 600], [0])
+    assert B.out_layout([3, 3, 3], 513)[0].tolist() == [0, 516, 1032]
+
+
+def test_griffinlim_length_outside_the_frame_range_is_a_value_error():
+    """librosa's loop needs the re-analysis to return T frames: 1 + length // 256 == T.  Checked before any device
+    work, naming the valid range."""
+    import spev_tts_b200 as sp
+    S = np.zeros((513, 10), np.float32)
+    for L in (9 * 256 - 1, 10 * 256, -1):
+        with pytest.raises(ValueError, match="2304" if L >= 0 else "non-negative"):
+            sp.griffinlim(S, n_iter=1, length=L)
+        with pytest.raises(ValueError):
+            sp.mel_to_audio(np.zeros((80, 10), np.float32), sr=22050, n_fft=1024, hop_length=256, length=L)
+    with pytest.raises(ValueError):
+        sp.istft(np.zeros((513, 4), np.complex64), length=-3)
