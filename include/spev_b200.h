@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SPEV_ABI_VERSION 1
+#define SPEV_ABI_VERSION 2
 
 #if defined(__GNUC__)
 #define SPEV_API __attribute__((visibility("default")))
@@ -59,12 +59,13 @@ typedef struct spev_ctx spev_ctx;
  *     src0 = absolute index in y of the first output sample of chunk t0
  *     row0 = global row of item frame (t0 - 1): the first of the n+3 frames the tile gathers
  *            (one before the item's first row when t0 == 0; never dereferenced then)
- *     lo, hi = 0, 0 (what spev_plan_chunk_tiles writes): whole chunks, the item's output is
- *            (T-1)*hop samples.  hi > lo: absolute bounds of the item's output in y; the ISTFT
- *            kernels write every sample of [lo, hi) and nothing outside it.
+ *     lo, hi = 0, 0 (what spev_plan_chunk_tiles writes without out_off / out_len): whole chunks,
+ *            the item's output is (T-1)*hop samples.  hi > lo: absolute bounds of the item's output
+ *            in y; the ISTFT kernels write every sample of [lo, hi) and nothing outside it.
  *
  * Output-length layout (librosa's istft / griffinlim `length=`): item i has L_i samples at
- * absolute offset out_off[i] of y.  Its chunk tiles cover chunks 0 .. ceil(L_i/hop)-1 with
+ * absolute offset out_off[i] of y.  Its chunk tiles (spev_plan_chunk_tiles with out_off,
+ * out_len = L) cover chunks 0 .. ceil(L_i/hop)-1 with
  * src0 = out_off[i] + hop*t0, lo = out_off[i], hi = out_off[i] + L_i; only the last chunk can be
  * partial.  Chunk c sums the item frames c-1 .. c+2 that exist: chunk T-1 has frames T-2, T-1,
  * chunk T has frame T-1, later chunks have none and are written as 0 (librosa's zero padding).
@@ -122,10 +123,16 @@ SPEV_API int spev_host_pinv(const float* a, int m, int n, float* pinv);
  *   sample_lo[i]  : absolute start of item i's samples in the flat buffer, n_samples[i] its
  *                   length (waveform batches: spev_logmel / spev_stft_power); pass NULL for both
  *                   to describe the implicit ISTFT-output layout (spev_stft, spev_gl_*, where
- *                   item i has (T_i-1)*hop samples at hop*(frame_off[i]-i)). */
+ *                   item i has (T_i-1)*hop samples at hop*(frame_off[i]-i)).
+ *   out_off[i], out_len[i] : the output-length layout above (chunk tiles); pass NULL for both
+ *                   for the implicit ISTFT-output layout.  Offsets must keep the items apart.
+ * Chunk tiles are listed full tiles first, then the partial ones, each in item order.
+ * Returns the tile count, or SPEV_E_INVALID (a null frames, n_items < 0, only one of a
+ * pointer pair given, a negative out_len). */
 SPEV_API int64_t spev_plan_frame_tiles(const int64_t* frames, const int64_t* sample_lo,
                                        const int64_t* n_samples, int n_items, spev_tile* out);
-SPEV_API int64_t spev_plan_chunk_tiles(const int64_t* frames, int n_items, spev_tile* out);
+SPEV_API int64_t spev_plan_chunk_tiles(const int64_t* frames, const int64_t* out_off,
+                                       const int64_t* out_len, int n_items, spev_tile* out);
 
 /* STFT -> |.|^2 -> mel -> (optional) log compression, fused, one launch.
  *   samples : dev float32, flat buffer the frame tiles index into

@@ -56,7 +56,7 @@ _SIGS = {
     "spev_host_mel_basis": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_void_p]),
     "spev_host_pinv": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "spev_plan_frame_tiles": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
-    "spev_plan_chunk_tiles": (C.c_int64, [C.c_void_p, C.c_int, C.c_void_p]),
+    "spev_plan_chunk_tiles": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "spev_logmel": (C.c_int, [C.c_void_p, C.POINTER(SpevBatch), C.c_void_p, C.c_void_p, C.c_int,
                               C.c_float, C.c_float, C.c_float, C.c_void_p]),
     "spev_pcm16_to_f32": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),

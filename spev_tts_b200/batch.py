@@ -1,9 +1,9 @@
 """Device context and flat (ragged) batch descriptors for the C ABI.
 
 A *flat batch* concatenates items (utterances or spectrograms) and describes them with prefix
-offsets + per-CTA tile tables, all built on the host with numpy and uploaded in ONE
-host->device copy.  Framing follows librosa ``center=True``: an item of ``N`` samples has
-``T = 1 + N // hop`` frames and an ISTFT output of ``(T-1)*hop`` samples
+offsets + per-CTA tile tables (planned by the library's ``spev_plan_*_tiles``), all built on
+the host and uploaded in ONE host->device copy.  Framing follows librosa ``center=True``: an
+item of ``N`` samples has ``T = 1 + N // hop`` frames and an ISTFT output of ``(T-1)*hop`` samples
 (reference call sites: ``spev_real_metrics.py:363`` and ``:730-733``).
 """
 from __future__ import annotations
@@ -27,77 +27,56 @@ TILE_DTYPE = np.dtype([("src0", "<i8"), ("lo", "<i8"), ("hi", "<i8"), ("row0", "
 assert TILE_DTYPE.itemsize == 48
 
 
-def _split(counts: np.ndarray, per_tile: int):
-    """(tile_item, tile_start) for items with ``counts[i]`` units cut into ``per_tile``-unit tiles."""
-    counts = np.asarray(counts, dtype=np.int64)
-    nt = (counts + per_tile - 1) // per_tile
-    tile_item = np.repeat(np.arange(len(counts), dtype=np.int64), nt)
-    first = np.cumsum(nt) - nt
-    tile_start = (np.arange(int(nt.sum()), dtype=np.int64) - np.repeat(first, nt)) * per_tile
-    return tile_item, tile_start
-
-
-def plan_frame_tiles(frames, sample_lo=None, n_samples=None, tile_frames: int = 32) -> np.ndarray:
-    """numpy twin of ``spev_plan_frame_tiles`` (vectorised): one ``spev_tile`` per <=32-frame tile."""
-    frames = np.asarray(frames, dtype=np.int64)
-    fo = np.concatenate([[0], np.cumsum(frames)])[:-1]
-    if sample_lo is None:
-        lo = HOP * (fo - np.arange(len(frames)))
-        hi = lo + (frames - 1) * HOP
-    else:
-        lo = np.asarray(sample_lo, dtype=np.int64)
-        hi = lo + np.asarray(n_samples, dtype=np.int64)
-    item, t0 = _split(frames, tile_frames)
-    out = np.zeros(len(item), dtype=TILE_DTYPE)
-    out["src0"] = lo[item] + HOP * t0 - N_FFT // 2
-    out["lo"], out["hi"] = lo[item], hi[item]
-    out["row0"] = fo[item] + t0
-    out["n"] = np.minimum(tile_frames, frames[item] - t0)
-    out["t0"], out["T"], out["item"] = t0, frames[item], item
+def _plan(fn, frames, pair):
+    """Count query, then fill, of a C tile planner ``fn(frames, a, b, n_items, out)``; ``pair`` is ``(a, b)``: two
+    per-item int64 arrays, or ``(None, None)`` for the implicit ISTFT-output layout."""
+    frames = np.ascontiguousarray(frames, dtype=np.int64).reshape(-1)
+    pair = [None if a is None else np.ascontiguousarray(a, dtype=np.int64).reshape(-1) for a in pair]
+    if any(a is not None and a.shape != frames.shape for a in pair):
+        raise ValueError(f"{fn.__name__}: needs one entry per item ({len(frames)}) in every array")
+    args = [frames.ctypes.data] + [None if a is None else a.ctypes.data for a in pair] + [len(frames)]
+    n = fn(*args, None)
+    if n < 0:
+        raise ValueError(_lib.load().spev_last_error().decode(errors="replace"))
+    out = np.empty(n, dtype=TILE_DTYPE)
+    fn(*args, out.ctypes.data)
     return out
 
 
-def plan_chunk_tiles(frames, tile_chunks: int = 29, *, out_off=None, out_len=None) -> np.ndarray:
-    """numpy twin of ``spev_plan_chunk_tiles``: one ``spev_tile`` per <=29-chunk ISTFT tile.
+def plan_frame_tiles(frames, sample_lo=None, n_samples=None) -> np.ndarray:
+    """``spev_plan_frame_tiles``: one ``spev_tile`` per <=32-frame tile.  Item i's samples are ``n_samples[i]`` at
+    ``sample_lo[i]``, or, without both, its ISTFT output in the implicit layout."""
+    return _plan(_lib.load().spev_plan_frame_tiles, frames, (sample_lo, n_samples))
+
+
+def plan_chunk_tiles(frames, *, out_off=None, out_len=None) -> np.ndarray:
+    """``spev_plan_chunk_tiles``: one ``spev_tile`` per <=29-chunk ISTFT tile, full tiles first.
 
     With ``out_off`` / ``out_len`` the tiles describe an explicit output layout instead (librosa's ``length=``): item i
     writes ``out_len[i]`` samples at ``out_off[i]``, ``ceil(out_len[i] / 256)`` chunks, ``lo`` / ``hi`` set to those
     bounds (see ``include/spev_b200.h``).  Without them ``lo = hi = 0``: the (T-1)*256-sample layout."""
-    frames = np.asarray(frames, dtype=np.int64)
-    fo = np.concatenate([[0], np.cumsum(frames)])[:-1]
-    if (out_off is None) != (out_len is None):
-        raise ValueError("out_off and out_len go together")
-    if out_len is None:
-        nc = np.maximum(frames - 1, 0)
-        start = HOP * (fo - np.arange(len(frames)))
-    else:
-        lens = np.asarray(out_len, dtype=np.int64).reshape(-1)
-        start = np.asarray(out_off, dtype=np.int64).reshape(-1)
-        nc = (lens + HOP - 1) // HOP
-    item, c0 = _split(nc, tile_chunks)
-    out = np.zeros(len(item), dtype=TILE_DTYPE)
-    out["src0"] = start[item] + HOP * c0
-    if out_len is not None:
-        out["lo"], out["hi"] = start[item], start[item] + lens[item]
-    out["row0"] = fo[item] + c0 - 1
-    out["n"] = np.minimum(tile_chunks, nc[item] - c0)
-    out["t0"], out["T"], out["item"] = c0, frames[item], item
-    # full tiles first, partial tiles last (same order as the C planner): tile j runs on CTA j mod grid, so the
-    # cheap tiles fall into the last, incomplete round
-    return out[np.argsort(out["n"] < tile_chunks, kind="stable")]
+    return _plan(_lib.load().spev_plan_chunk_tiles, frames, (out_off, out_len))
+
+
+def aligned_offsets(n_samples: Sequence[int], align: int = 4) -> np.ndarray:
+    """Item starts ``[U+1]`` (last entry = buffer size) with every start a multiple of ``align``
+    samples, so that the kernels take the 16-byte cp.async staging path.  The <= align-1 filler
+    samples between items are never read as signal."""
+    ns = np.asarray(n_samples, dtype=np.int64)
+    padded = (ns + align - 1) // align * align
+    return np.concatenate([[0], np.cumsum(padded)]).astype(np.int64)
 
 
 def out_layout(frames, out_len, out_off=None):
     """Output layout of a batch with explicit per-item output lengths -> (``out_off`` int64 [n_items], ``out_len`` int64
     [n_items]).  ``out_len`` is one length per item (or one for all).  Default offsets pack the items in order, each
-    starting at a multiple of 4 samples (the kernels' 16-byte paths); given offsets must keep the items apart."""
+    starting at a multiple of 4 samples (``aligned_offsets``); given offsets must keep the items apart."""
     frames = np.asarray(frames, dtype=np.int64).reshape(-1)
     lens = np.broadcast_to(np.asarray(out_len, dtype=np.int64), frames.shape).copy()
     if (lens < 0).any():
         raise ValueError("output lengths must be >= 0")
     if out_off is None:
-        padded = (lens + 3) // 4 * 4
-        off = np.concatenate([[0], np.cumsum(padded)])[:-1].astype(np.int64)
+        off = aligned_offsets(lens)[:-1]
     else:
         off = np.asarray(out_off, dtype=np.int64).reshape(-1)
         if off.shape != frames.shape:
@@ -125,8 +104,6 @@ class Context:
         self.sr, self.n_fft, self.hop, self.win, self.n_mels = sr, n_fft, hop, win, n_mels
         self.fmin = float(fmin)
         self.fmax = float(fmax) if fmax is not None else 0.5 * sr
-        self.tile_frames = lib.spev_tile_frames()
-        self.tile_chunks = lib.spev_tile_chunks()
         h = C.c_void_p()
         _lib.check(lib.spev_create(C.byref(h), self.device, sr, n_fft, hop, win, n_mels,
                                    self.fmin, self.fmax), "spev_create")
@@ -240,6 +217,19 @@ class FlatBatch:
             return self.out_len.copy()
         return np.maximum(self.frames - 1, 0) * HOP
 
+    def output_items(self, y: torch.Tensor) -> torch.Tensor:
+        """``[n_items, L]`` items of an equal-length batch from its flat ISTFT output ``y`` (``n_out_samples``
+        samples): a view when the items are back to back, a contiguous copy when starts are padded apart."""
+        off, lens = self.out_sample_off()[:-1], self.out_lengths()
+        L = int(lens[0]) if self.n_items else 0
+        pitch = int(off[1] - off[0]) if self.n_items > 1 else L
+        if (lens != L).any() or (np.diff(off) != pitch).any() or pitch < L:
+            raise ValueError("output_items needs items of one length at one spacing")
+        if y.dim() != 1 or not y.is_contiguous() or y.numel() < self.n_out_samples:
+            raise ValueError(f"output_items: y must be a flat buffer of >= {self.n_out_samples} samples")
+        items = y.as_strided((self.n_items, L), (pitch, 1), y.storage_offset() + (int(off[0]) if self.n_items else 0))
+        return items if pitch == L else items.contiguous()
+
 
 def make_batch(ctx: Context, *, n_samples: Optional[Sequence[int]] = None,
                n_frames: Optional[Sequence[int]] = None, sample_off: Optional[np.ndarray] = None,
@@ -264,16 +254,16 @@ def make_batch(ctx: Context, *, n_samples: Optional[Sequence[int]] = None,
             sample_off = np.concatenate([[0], np.cumsum(ns)])[:-1].astype(np.int64)
         else:
             sample_off = np.asarray(sample_off, dtype=np.int64).reshape(-1)[: len(ns)]
-        ftiles = plan_frame_tiles(frames, sample_off, ns, ctx.tile_frames)
+        ftiles = plan_frame_tiles(frames, sample_off, ns)
     else:
         frames = np.asarray(n_frames, dtype=np.int64).reshape(-1)
         sample_off = None
         if out_len is not None:
             out_off, out_len = out_layout(frames, out_len, out_off)
-        ftiles = plan_frame_tiles(frames, out_off, out_len, ctx.tile_frames)
+        ftiles = plan_frame_tiles(frames, out_off, out_len)
     n_items = int(len(frames))
     frame_off = np.concatenate([[0], np.cumsum(frames)]).astype(np.int64)
-    ctiles = (plan_chunk_tiles(frames, ctx.tile_chunks, out_off=out_off, out_len=out_len) if with_chunks
+    ctiles = (plan_chunk_tiles(frames, out_off=out_off, out_len=out_len) if with_chunks
               else np.zeros(0, dtype=TILE_DTYPE))
 
     # one staging buffer: [ftiles | ctiles | frame_off]; tile tables first (16-byte aligned)

@@ -19,7 +19,7 @@ import numpy as np
 import torch
 
 from . import _lib, spectral
-from .batch import HOP, Context, make_batch
+from .batch import HOP, Context, aligned_offsets, make_batch
 
 
 # ---------------------------------------------------------------------------------------------
@@ -81,15 +81,6 @@ def shard_utterances(n_samples: Sequence[int], world_size: int) -> List[np.ndarr
         owner[i] = r
         loads[r] += fr[i]
     return [np.sort(np.nonzero(owner == r)[0]) for r in range(world_size)]
-
-
-def aligned_offsets(n_samples: Sequence[int], align: int = 4) -> np.ndarray:
-    """Item starts ``[U+1]`` (last entry = buffer size) with every start a multiple of ``align``
-    samples, so that the kernels take the 16-byte cp.async staging path.  The <= align-1 filler
-    samples between items are never read as signal."""
-    ns = np.asarray(n_samples, dtype=np.int64)
-    padded = (ns + align - 1) // align * align
-    return np.concatenate([[0], np.cumsum(padded)]).astype(np.int64)
 
 
 @dataclass

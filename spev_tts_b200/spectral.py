@@ -202,12 +202,6 @@ def _gl_length(length, T: int) -> Optional[int]:
     return length
 
 
-def _unpack_items(y: torch.Tensor, b: int, L: int, pitch: int) -> torch.Tensor:
-    """Uniform items of ``L`` samples, item i at ``i * pitch`` of the flat buffer ``y`` (>= b * pitch) -> ``[b, L]``."""
-    out = y[: b * pitch].view(b, pitch)
-    return out if pitch == L else out[:, :L].contiguous()
-
-
 def istft(X: ArrayLike, *, hop_length=None, win_length=None, n_fft=None, window="hann", center=True,
           dtype=None, length=None, device=None):
     """Drop-in for ``librosa.istft`` -> float32 ``[..., (T-1)*hop]``, or ``[..., length]`` with librosa's crop / zero
@@ -222,11 +216,10 @@ def istft(X: ArrayLike, *, hop_length=None, win_length=None, n_fft=None, window=
     L = (T - 1) * HOP if length is None else length
     batch = make_batch(ctx, n_frames=[T] * b, with_chunks=True, out_len=None if length is None else [L] * b)
     spec = _spec_to_internal(t.reshape(b, nb, T))
-    pitch = int(batch.out_sample_off()[1] - batch.out_sample_off()[0]) if b > 1 else L
-    y = torch.empty(max(batch.n_out_samples, b * pitch), dtype=torch.float32, device=t.device)
+    y = torch.empty(batch.n_out_samples, dtype=torch.float32, device=t.device)
     _lib.check(ctx.lib.spev_istft(ctx.handle, batch.desc, spec.data_ptr(), _lib.SPEC_LD, y.data_ptr(),
                                   stream_ptr(t.device)), "spev_istft")
-    return _ret(_unpack_items(y, b, L, pitch).view(*lead, L), was_numpy)
+    return _ret(batch.output_items(y).view(*lead, L), was_numpy)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -421,10 +414,8 @@ def griffinlim(S: ArrayLike, *, n_iter=32, hop_length=None, win_length=None, n_f
     Sf = items_to_rows(t.reshape(b, nb, T), _lib.SPEC_LD, out=torch.zeros((b * T, _lib.SPEC_LD), dtype=torch.float32, device=t.device))
     ph = _phase_to_internal(init_phase, b, T, t.device) if init_phase is not None else None
     seed = int(np.random.SeedSequence(random_state).generate_state(2, dtype=np.uint32).view(np.uint64)[0])
-    pitch = int(batch.out_sample_off()[1] - batch.out_sample_off()[0]) if b > 1 else L
-    y = torch.empty(max(batch.n_out_samples, b * pitch), dtype=torch.float32, device=t.device)
-    y = griffinlim_flat(Sf, batch, ctx, n_iter=n_iter, momentum=momentum, init_phase=ph, seed=seed, out=y)
-    return _ret(_unpack_items(y, b, L, pitch).view(*lead, L), was_numpy)
+    y = griffinlim_flat(Sf, batch, ctx, n_iter=n_iter, momentum=momentum, init_phase=ph, seed=seed)
+    return _ret(batch.output_items(y).view(*lead, L), was_numpy)
 
 
 def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_length=None, window="hann",
@@ -446,7 +437,6 @@ def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_len
     ctx = Context.get(t.device, sr=sr, n_mels=n_mels, fmin=fmin, fmax=fmax)
     L = (T - 1) * HOP if length is None else length
     batch = ctx.uniform_batch(b, T, with_chunks=True, out_len=length)
-    pitch = int(batch.out_sample_off()[1] - batch.out_sample_off()[0]) if b > 1 else L
     tm = items_to_rows(t.reshape(b, n_mels, T)).view(-1)                  # frame-major -> tensor-core GEMM
     S = mel_to_mag_flat(tm, batch, ctx, layout=0, is_log=is_log)
     ph = _phase_to_internal(init_phase, b, T, t.device) if init_phase is not None else None
@@ -454,9 +444,8 @@ def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_len
     out = {}
 
     def run_gl():
-        if "y" not in out:
-            out["y"] = torch.empty(max(batch.n_out_samples, b * pitch), dtype=torch.float32, device=t.device)
-        griffinlim_flat(S, batch, ctx, n_iter=n_iter, momentum=momentum, init_phase=ph, seed=seed, out=out["y"])
+        out["y"] = griffinlim_flat(S, batch, ctx, n_iter=n_iter, momentum=momentum, init_phase=ph, seed=seed,
+                                   out=out.get("y"))
     if nnls == "librosa" and b * T > 0:
         # Griffin-Lim is enqueued on the warm start while the host fetches the screening result; in the (rare: short
         # utterances, short remainder blocks) case that librosa's solver iterates, S is refined and the loop redone
@@ -464,4 +453,4 @@ def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_len
             run_gl()
     else:
         run_gl()
-    return _ret(_unpack_items(out["y"], b, L, pitch).view(*lead, L), was_numpy)
+    return _ret(batch.output_items(out["y"]).view(*lead, L), was_numpy)

@@ -20,7 +20,7 @@ def header_symbols():
     return sorted(set(re.findall(r"SPEV_API\s+[\w\s\*]+?\b(spev_\w+)\s*\(", src)))
 
 
-def test_library_builds_and_exports_header_symbols():
+def test_library_builds_exports_header_symbols_abi_2():
     import spev_tts_b200 as sp
     from spev_tts_b200 import build
     build.build()
@@ -33,7 +33,7 @@ def test_library_builds_and_exports_header_symbols():
     out = subprocess.check_output(["nm", "-D", "--defined-only", sp.LIB_PATH], text=True)
     exported = sorted(l.split()[-1] for l in out.splitlines() if " T " in l)
     assert exported == syms, "library exports symbols outside the header (or misses some)"
-    assert lib.spev_abi_version() == 1 and lib.spev_tile_chunks() == lib.spev_tile_frames() - 3
+    assert lib.spev_abi_version() == 2 and lib.spev_tile_chunks() == lib.spev_tile_frames() - 3
 
 
 def test_sass_is_sm100a():
@@ -56,36 +56,41 @@ def test_host_constants_match_oracle():
         assert np.linalg.norm(p - op) / np.linalg.norm(op) < 1e-6
 
 
-def test_plan_tiles_c_vs_numpy():
-    """spev_plan_frame_tiles / spev_plan_chunk_tiles (C) == the vectorised numpy twins."""
+def test_plan_tiles_count_query_and_closed_forms():
+    """spev_plan_frame_tiles / spev_plan_chunk_tiles: the count query (out == NULL) equals the number of tiles the fill
+    writes, for both frame layouts and both chunk layouts, and the counts are sum ceil(T/32), sum ceil((T-1)/29) and
+    sum ceil(ceil(L/256)/29)."""
     import spev_tts_b200 as sp
     from spev_tts_b200 import batch as B
     lib = sp.load()
+    tf, tc = lib.spev_tile_frames(), lib.spev_tile_chunks()
     rng = np.random.default_rng(0)
     ns = rng.integers(0, 200 * 256, 50).astype(np.int64)
     ns[:4] = [0, 255, 256, 32 * 256]
     frames = 1 + ns // 256
-    starts = np.concatenate([[0], np.cumsum((ns + 3) // 4 * 4)])[:-1].astype(np.int64)
+    starts = B.aligned_offsets(ns)[:-1]
+    out_len = rng.integers(0, 260 * 200, 50).astype(np.int64)
+    out_len[:4] = [0, 1, 256, 29 * 256 + 1]
+    out_off = B.out_layout(frames, out_len)[0]
+
+    def ptr(a):
+        return None if a is None else a.ctypes.data
+
+    def count_and_fill(fn, a, b):
+        cnt = fn(ptr(frames), ptr(a), ptr(b), len(frames), None)
+        out = np.zeros(cnt + 1, dtype=B.TILE_DTYPE)           # one spare record, which the fill must not touch
+        assert fn(ptr(frames), ptr(a), ptr(b), len(frames), out.ctypes.data) == cnt
+        assert out[cnt:].tobytes() == bytes(B.TILE_DTYPE.itemsize)
+        return cnt
     for lo, n in ((starts, ns), (None, None)):
-        cnt = lib.spev_plan_frame_tiles(frames.ctypes.data, lo.ctypes.data if lo is not None else None,
-                                        n.ctypes.data if n is not None else None, len(frames), None)
-        out = np.zeros(cnt, dtype=B.TILE_DTYPE)
-        assert lib.spev_plan_frame_tiles(frames.ctypes.data, lo.ctypes.data if lo is not None else None,
-                                         n.ctypes.data if n is not None else None, len(frames),
-                                         out.ctypes.data) == cnt
-        tf = lib.spev_tile_frames()
-        ref = B.plan_frame_tiles(frames, lo, n, tf)
-        assert cnt == len(ref) == int(((frames + tf - 1) // tf).sum())
-        assert out.tobytes() == ref.tobytes()
-    cnt = lib.spev_plan_chunk_tiles(frames.ctypes.data, len(frames), None)
-    out = np.zeros(cnt, dtype=B.TILE_DTYPE)
-    assert lib.spev_plan_chunk_tiles(frames.ctypes.data, len(frames), out.ctypes.data) == cnt
-    tc = lib.spev_tile_chunks()
-    ref = B.plan_chunk_tiles(frames, tc)
-    assert out.tobytes() == ref.tobytes() and cnt == int(((frames - 1 + tc - 1) // tc).sum())
+        assert count_and_fill(lib.spev_plan_frame_tiles, lo, n) == int(((frames + tf - 1) // tf).sum())
+    assert count_and_fill(lib.spev_plan_chunk_tiles, None, None) == int(((frames - 1 + tc - 1) // tc).sum())
+    nc = (out_len + 255) // 256
+    assert count_and_fill(lib.spev_plan_chunk_tiles, out_off, out_len) == int(((nc + tc - 1) // tc).sum())
     # every frame / chunk covered exactly once
     assert B.plan_frame_tiles(frames)["n"].sum() == frames.sum()
-    assert ref["n"].sum() == (frames - 1).sum()
+    assert B.plan_chunk_tiles(frames)["n"].sum() == (frames - 1).sum()
+    assert B.plan_chunk_tiles(frames, out_off=out_off, out_len=out_len)["n"].sum() == nc.sum()
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure mode")
@@ -146,11 +151,18 @@ def test_header_is_valid_c99_and_struct_layout():
         assert f"USE({sym})" in src, sym
 
 
-def test_host_entry_points_reject_bad_arguments():
+def test_host_entry_points_and_planners_reject_bad_arguments():
     import spev_tts_b200 as sp
     lib = sp.load()
     assert lib.spev_plan_frame_tiles(None, None, None, 3, None) == -1
-    assert lib.spev_plan_chunk_tiles(None, 3, None) == -1
+    assert lib.spev_plan_chunk_tiles(None, None, None, 3, None) == -1
+    frames, off, lens = (np.array(v, dtype=np.int64) for v in ([3, 3], [0, 1024], [512, -1]))
+    assert lib.spev_plan_chunk_tiles(frames.ctypes.data, off.ctypes.data, None, 2, None) == -1    # out_off, no out_len
+    assert lib.spev_plan_chunk_tiles(frames.ctypes.data, off.ctypes.data, lens.ctypes.data, 2, None) == -1
+    assert b"out_len[1]" in lib.spev_last_error()
+    from spev_tts_b200 import batch as B
+    with pytest.raises(ValueError, match="out_len"):
+        B.plan_chunk_tiles(frames, out_off=off, out_len=lens)
     assert lib.spev_host_mel_basis(0, 1024, 80, 0.0, 0.0, None) == -1
     assert lib.spev_griffinlim_workspace_bytes(-5) == 0
     assert lib.spev_griffinlim_workspace_bytes(10) >= 10 * 520 * 16

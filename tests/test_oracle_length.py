@@ -75,7 +75,14 @@ def test_griffinlim_length_of_whole_chunks_is_the_default():
     assert not np.array_equal(tail[: 40 * 256], plain)         # the tail is re-analysed in every iteration
 
 
-def test_length_planner_covers_every_sample_once():
+@pytest.fixture(scope="module")
+def built():
+    """The tile planners are the library's (spev_plan_*_tiles): build it first."""
+    from spev_tts_b200 import build
+    build.build()
+
+
+def test_c_length_planner_covers_every_sample_once(built):
     rng = np.random.default_rng(5)
     for trial in range(20):
         n = int(rng.integers(1, 12))
@@ -89,7 +96,7 @@ def test_length_planner_covers_every_sample_once():
         else:
             off, L = B.out_layout(frames, lens)
             assert (off % 4 == 0).all() and off[0] == 0
-        tiles = B.plan_chunk_tiles(frames, 29, out_off=off, out_len=L)
+        tiles = B.plan_chunk_tiles(frames, out_off=off, out_len=L)
         end = int((off + L).max(initial=0)) + 300
         count = np.zeros(end + 29 * 256, dtype=np.int64)
         for t in tiles:
@@ -109,9 +116,8 @@ def test_length_planner_covers_every_sample_once():
         assert not (full[1:] & ~full[:-1]).any()               # full tiles first
         ft = B.plan_frame_tiles(frames, off, L)
         assert np.array_equal(ft["lo"], off[ft["item"]]) and np.array_equal(ft["hi"], (off + L)[ft["item"]])
-    # without a layout: byte-identical to the plain planner (lo = hi = 0)
+    # without a layout: the plain planner (lo = hi = 0)
     frames = np.array([800, 33, 1, 2, 64])
-    assert B.plan_chunk_tiles(frames, 29).tobytes() == B.plan_chunk_tiles(frames).tobytes()
     assert not B.plan_chunk_tiles(frames)["hi"].any()
 
 
@@ -123,6 +129,33 @@ def test_out_layout_rejects_bad_layouts():
     with pytest.raises(ValueError):
         B.out_layout([3, 3], [600, 600], [0])
     assert B.out_layout([3, 3, 3], 513)[0].tolist() == [0, 516, 1032]
+
+
+def test_output_items_of_the_flat_output_layout():
+    """``FlatBatch.output_items``: a view of back-to-back items, a copy of items whose starts are padded to 4 samples,
+    from a buffer of exactly ``n_out_samples``; unequal lengths or spacing are refused."""
+    def host_batch(frames, out_len=None, out_off=None):
+        frames = np.asarray(frames, dtype=np.int64)
+        if out_len is not None:
+            out_off, out_len = B.out_layout(frames, out_len, out_off)
+        fo = np.concatenate([[0], np.cumsum(frames)])
+        return B.FlatBatch(len(frames), int(fo[-1]), frames, None, fo, 0, 0, None, None, torch.device("cpu"),
+                           out_off=out_off, out_len=out_len)
+    for out_len, back_to_back in ((None, True), (99 * 256 + 8, True), (99 * 256 + 5, False), (0, True)):
+        fb = host_batch([100] * 3, None if out_len is None else [out_len] * 3)
+        L = 99 * 256 if out_len is None else out_len
+        y = torch.arange(fb.n_out_samples, dtype=torch.float32)
+        items = fb.output_items(y)
+        pitch = L if back_to_back else (L + 3) // 4 * 4
+        assert items.shape == (3, L) and items.is_contiguous()
+        assert torch.equal(items, torch.stack([y[i * pitch: i * pitch + L] for i in range(3)]))
+        assert (items.data_ptr() == y.data_ptr()) == back_to_back
+    for fb in (host_batch([100, 99]), host_batch([100] * 3, [512] * 3, [0, 512, 1200])):
+        with pytest.raises(ValueError, match="one length at one spacing"):
+            fb.output_items(torch.zeros(fb.n_out_samples))
+    fb = host_batch([100] * 2, [600] * 2)
+    with pytest.raises(ValueError):
+        fb.output_items(torch.zeros(fb.n_out_samples - 1))
 
 
 def test_griffinlim_length_outside_the_frame_range_is_a_value_error():

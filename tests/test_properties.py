@@ -2,9 +2,18 @@
 frame / chunk exactly once; the vectorised LengthRegulator restatement equals a literal
 transcription of the reference loop for arbitrary durations."""
 import numpy as np
+import pytest
 from hypothesis import given, settings, strategies as st
 
 from oracle import librosa_restated as lr
+
+
+@pytest.fixture(scope="module")
+def planners():
+    """The tile planners are the library's (spev_plan_*_tiles): build it first."""
+    from spev_tts_b200 import batch, build
+    build.build()
+    return batch
 
 
 def literal_lr(x, dur):
@@ -46,26 +55,35 @@ def test_lr_restatement_equals_literal_loop(B, T, H, seed, as_float):
 
 @settings(max_examples=80, deadline=None)
 @given(st.lists(st.integers(0, 40000), min_size=1, max_size=30))
-def test_tiles_cover_everything_once(n_samples):
-    from spev_tts_b200 import batch as B
+def test_c_planned_tiles_cover_everything_once_in_order(planners, n_samples):
+    B = planners
     ns = np.asarray(n_samples, dtype=np.int64)
     frames = 1 + ns // 256
     starts = np.concatenate([[0], np.cumsum((ns + 3) // 4 * 4)])[:-1]
-    ft = B.plan_frame_tiles(frames, starts, ns, 32)
+    ft = B.plan_frame_tiles(frames, starts, ns)
     fo = np.concatenate([[0], np.cumsum(frames)])
+    # item order, 32-frame steps within an item
+    assert np.array_equal(ft["item"], np.repeat(np.arange(len(frames)), (frames + 31) // 32))
+    assert (np.diff(ft["row0"]) > 0).all()
     covered = np.zeros(fo[-1], dtype=np.int32)
     for t in ft:
-        assert 1 <= t["n"] <= 32 and t["T"] == frames[t["item"]]
+        assert 1 <= t["n"] <= 32 and t["T"] == frames[t["item"]] and t["t0"] % 32 == 0
         assert t["row0"] == fo[t["item"]] + t["t0"]
         assert t["src0"] == starts[t["item"]] + 256 * t["t0"] - 512
         assert t["lo"] == starts[t["item"]] and t["hi"] == t["lo"] + ns[t["item"]]
         covered[t["row0"]: t["row0"] + t["n"]] += 1
     assert np.all(covered == 1)
-    ct = B.plan_chunk_tiles(frames, 29)
+    ct = B.plan_chunk_tiles(frames)
     yo = (fo - np.arange(len(fo))) * 256
     cov = np.zeros(yo[-1] // 256, dtype=np.int32)
     for t in ct:
-        assert 1 <= t["n"] <= 29
+        assert 1 <= t["n"] <= 29 and t["t0"] % 29 == 0
+        assert t["lo"] == t["hi"] == 0 and t["T"] == frames[t["item"]]
         assert t["src0"] == yo[t["item"]] + 256 * t["t0"] and t["row0"] == fo[t["item"]] + t["t0"] - 1
         cov[t["src0"] // 256: t["src0"] // 256 + t["n"]] += 1
     assert np.all(cov == 1)
+    # full tiles first, then the partial ones; each group in item order
+    full = ct["n"] == 29
+    assert not (full[1:] & ~full[:-1]).any()
+    for group in (ct[full], ct[~full]):
+        assert (np.lexsort((group["t0"], group["item"])) == np.arange(len(group))).all()
