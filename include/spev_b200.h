@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define SPEV_ABI_VERSION 2
+#define SPEV_ABI_VERSION 3
 
 #if defined(__GNUC__)
 #define SPEV_API __attribute__((visibility("default")))
@@ -59,18 +59,17 @@ typedef struct spev_ctx spev_ctx;
  *     src0 = absolute index in y of the first output sample of chunk t0
  *     row0 = global row of item frame (t0 - 1): the first of the n+3 frames the tile gathers
  *            (one before the item's first row when t0 == 0; never dereferenced then)
- *     lo, hi = 0, 0 (what spev_plan_chunk_tiles writes without out_off / out_len): whole chunks,
- *            the item's output is (T-1)*hop samples.  hi > lo: absolute bounds of the item's output
- *            in y; the ISTFT kernels write every sample of [lo, hi) and nothing outside it.
+ *     lo, hi = absolute bounds of the item's output in y; the ISTFT kernels write every sample
+ *            of [lo, hi) and nothing outside it.
  *
- * Output-length layout (librosa's istft / griffinlim `length=`): item i has L_i samples at
- * absolute offset out_off[i] of y.  Its chunk tiles (spev_plan_chunk_tiles with out_off,
- * out_len = L) cover chunks 0 .. ceil(L_i/hop)-1 with
+ * ISTFT output layout: item i has L_i samples at absolute offset out_off[i] of y.  librosa's
+ * istft / griffinlim give an item (T_i-1)*hop samples by default and exactly `length` with
+ * `length=`.  Its chunk tiles (spev_plan_chunk_tiles) cover chunks 0 .. ceil(L_i/hop)-1 with
  * src0 = out_off[i] + hop*t0, lo = out_off[i], hi = out_off[i] + L_i; only the last chunk can be
  * partial.  Chunk c sums the item frames c-1 .. c+2 that exist: chunk T-1 has frames T-2, T-1,
  * chunk T has frame T-1, later chunks have none and are written as 0 (librosa's zero padding).
  * The frame tiles of the same layout (spev_plan_frame_tiles with sample_lo = out_off,
- * n_samples = L) make spev_stft / spev_gl_phase_update / spev_griffinlim re-analyse exactly
+ * n_samples = L) make spev_stft / spev_gl_phase_update / spev_griffinlim analyse exactly
  * these samples.  Griffin-Lim needs 1 + L_i/hop == T_i, i.e. (T_i-1)*hop <= L_i < T_i*hop.
  * out_off[i] a multiple of 4 keeps the 16-byte load and store paths. */
 typedef struct spev_tile {
@@ -79,8 +78,8 @@ typedef struct spev_tile {
 } spev_tile;
 
 /* Flat batch descriptor.  Item i owns rows [frame_off[i], frame_off[i+1]) of every [F, .] array.
- * Framing is librosa center=True: an item of N samples has T = 1 + N / hop frames; an ISTFT
- * output item has (T-1)*hop samples at offset hop*(frame_off[i] - i). */
+ * Framing is librosa center=True: an item of N samples has T = 1 + N / hop frames.  Where an
+ * item's samples lie is told by the tiles' [lo, hi) bounds alone. */
 typedef struct spev_batch {
     int32_t n_items;
     int32_t n_ftiles;
@@ -121,14 +120,13 @@ SPEV_API int spev_host_pinv(const float* a, int m, int n, float* pinv);
 /* Host helpers that build the tile tables (call with out == NULL to get the count).
  *   frames[i]     : frames of item i
  *   sample_lo[i]  : absolute start of item i's samples in the flat buffer, n_samples[i] its
- *                   length (waveform batches: spev_logmel / spev_stft_power); pass NULL for both
- *                   to describe the implicit ISTFT-output layout (spev_stft, spev_gl_*, where
- *                   item i has (T_i-1)*hop samples at hop*(frame_off[i]-i)).
- *   out_off[i], out_len[i] : the output-length layout above (chunk tiles); pass NULL for both
- *                   for the implicit ISTFT-output layout.  Offsets must keep the items apart.
- * Chunk tiles are listed full tiles first, then the partial ones, each in item order.
- * Returns the tile count, or SPEV_E_INVALID (a null frames, n_items < 0, only one of a
- * pointer pair given, a negative out_len). */
+ *                   length: a waveform (spev_logmel / spev_stft_power) or an ISTFT output
+ *                   (spev_stft, spev_gl_*, spev_griffinlim: sample_lo = out_off, n_samples = out_len)
+ *   out_off[i], out_len[i] : the ISTFT output layout above (chunk tiles).  Offsets must keep
+ *                   the items apart.
+ * Every array is required.  Chunk tiles are listed full tiles first, then the partial ones,
+ * each in item order.  Returns the tile count, or SPEV_E_INVALID (a null array, n_items < 0,
+ * a negative n_samples or out_len). */
 SPEV_API int64_t spev_plan_frame_tiles(const int64_t* frames, const int64_t* sample_lo,
                                        const int64_t* n_samples, int n_items, spev_tile* out);
 SPEV_API int64_t spev_plan_chunk_tiles(const int64_t* frames, const int64_t* out_off,
@@ -195,9 +193,8 @@ SPEV_API int spev_nnls_objective(spev_ctx* ctx, const void* x, int x_mode, int64
                                  void* stream);
 
 /* ISTFT (irFFT-1024, Hann, gather overlap-add, window-sum-square normalisation).
- *   spec : dev float2 [n_frames, ld] ; y : dev float32, item i at 256*(frame_off[i]-i),
- *   length (T_i-1)*256 -- or, with bounded chunk tiles, the output-length layout above.
- *   Replaces librosa.istft inside griffinlim (:730-733). */
+ *   spec : dev float2 [n_frames, ld] ; y : dev float32 in the ISTFT output layout above (item i
+ *   is [lo, hi) of its chunk tiles).  Replaces librosa.istft inside griffinlim (:730-733). */
 SPEV_API int spev_istft(spev_ctx* ctx, const spev_batch* batch, const void* spec, int64_t ld, float* y,
                void* stream);
 
@@ -218,9 +215,9 @@ SPEV_API int spev_gl_phase_update(spev_ctx* ctx, const spev_batch* batch, const 
  * Same arithmetic per frame as spev_istft / spev_gl_phase_update, except that the phase normalisation uses a 2-ulp
  * rsqrt and the <= 4 overlap-add terms of a sample are summed pair by pair: agrees with those entry points to rounding.
  *   init_phase : dev float32 [n_frames, 513] radians, or NULL -> 2*pi*U[0,1) from `seed`
- *   y          : dev float32 [256*(n_frames - n_items)]; with bounded chunk tiles (and frame tiles of
- *                the same layout) item i is [out_off[i], out_off[i] + L_i) instead: librosa's
- *                griffinlim(length=L_i), every inner istft included; samples between items are not touched
+ *   y          : dev float32 in the ISTFT output layout above, chunk and frame tiles of the same layout:
+ *                item i is [out_off[i], out_off[i] + L_i), librosa's griffinlim(length=L_i), every inner
+ *                istft included; samples between items are not touched
  *   workspace  : dev, >= spev_griffinlim_workspace_bytes(n_frames)
  * Replaces librosa.griffinlim under spev_real_metrics.py:730-733 (n_iter default 32 there,
  * momentum 0.99). */

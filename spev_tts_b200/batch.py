@@ -27,14 +27,14 @@ TILE_DTYPE = np.dtype([("src0", "<i8"), ("lo", "<i8"), ("hi", "<i8"), ("row0", "
 assert TILE_DTYPE.itemsize == 48
 
 
-def _plan(fn, frames, pair):
-    """Count query, then fill, of a C tile planner ``fn(frames, a, b, n_items, out)``; ``pair`` is ``(a, b)``: two
-    per-item int64 arrays, or ``(None, None)`` for the implicit ISTFT-output layout."""
+def _plan(fn, frames, a, b):
+    """Count query, then fill, of a C tile planner ``fn(frames, a, b, n_items, out)``; ``a``, ``b``: per-item int64
+    arrays."""
     frames = np.ascontiguousarray(frames, dtype=np.int64).reshape(-1)
-    pair = [None if a is None else np.ascontiguousarray(a, dtype=np.int64).reshape(-1) for a in pair]
-    if any(a is not None and a.shape != frames.shape for a in pair):
+    a, b = (np.ascontiguousarray(x, dtype=np.int64).reshape(-1) for x in (a, b))
+    if a.shape != frames.shape or b.shape != frames.shape:
         raise ValueError(f"{fn.__name__}: needs one entry per item ({len(frames)}) in every array")
-    args = [frames.ctypes.data] + [None if a is None else a.ctypes.data for a in pair] + [len(frames)]
+    args = [frames.ctypes.data, a.ctypes.data, b.ctypes.data, len(frames)]
     n = fn(*args, None)
     if n < 0:
         raise ValueError(_lib.load().spev_last_error().decode(errors="replace"))
@@ -43,19 +43,17 @@ def _plan(fn, frames, pair):
     return out
 
 
-def plan_frame_tiles(frames, sample_lo=None, n_samples=None) -> np.ndarray:
-    """``spev_plan_frame_tiles``: one ``spev_tile`` per <=32-frame tile.  Item i's samples are ``n_samples[i]`` at
-    ``sample_lo[i]``, or, without both, its ISTFT output in the implicit layout."""
-    return _plan(_lib.load().spev_plan_frame_tiles, frames, (sample_lo, n_samples))
+def plan_frame_tiles(frames, sample_lo, n_samples) -> np.ndarray:
+    """``spev_plan_frame_tiles``: one ``spev_tile`` per <=32-frame tile; item i's samples are ``n_samples[i]`` at
+    ``sample_lo[i]``."""
+    return _plan(_lib.load().spev_plan_frame_tiles, frames, sample_lo, n_samples)
 
 
-def plan_chunk_tiles(frames, *, out_off=None, out_len=None) -> np.ndarray:
-    """``spev_plan_chunk_tiles``: one ``spev_tile`` per <=29-chunk ISTFT tile, full tiles first.
-
-    With ``out_off`` / ``out_len`` the tiles describe an explicit output layout instead (librosa's ``length=``): item i
-    writes ``out_len[i]`` samples at ``out_off[i]``, ``ceil(out_len[i] / 256)`` chunks, ``lo`` / ``hi`` set to those
-    bounds (see ``include/spev_b200.h``).  Without them ``lo = hi = 0``: the (T-1)*256-sample layout."""
-    return _plan(_lib.load().spev_plan_chunk_tiles, frames, (out_off, out_len))
+def plan_chunk_tiles(frames, *, out_off, out_len) -> np.ndarray:
+    """``spev_plan_chunk_tiles``: one ``spev_tile`` per <=29-chunk ISTFT tile, full tiles first.  Item i writes
+    ``out_len[i]`` samples at ``out_off[i]``, ``ceil(out_len[i] / 256)`` chunks, with ``lo`` / ``hi`` set to those
+    bounds (see ``include/spev_b200.h``)."""
+    return _plan(_lib.load().spev_plan_chunk_tiles, frames, out_off, out_len)
 
 
 def aligned_offsets(n_samples: Sequence[int], align: int = 4) -> np.ndarray:
@@ -67,11 +65,14 @@ def aligned_offsets(n_samples: Sequence[int], align: int = 4) -> np.ndarray:
     return np.concatenate([[0], np.cumsum(padded)]).astype(np.int64)
 
 
-def out_layout(frames, out_len, out_off=None):
-    """Output layout of a batch with explicit per-item output lengths -> (``out_off`` int64 [n_items], ``out_len`` int64
-    [n_items]).  ``out_len`` is one length per item (or one for all).  Default offsets pack the items in order, each
-    starting at a multiple of 4 samples (``aligned_offsets``); given offsets must keep the items apart."""
+def out_layout(frames, out_len=None, out_off=None):
+    """ISTFT output layout of a spectrogram batch -> (``out_off`` int64 [n_items], ``out_len`` int64 [n_items]).
+    ``out_len`` is one length per item (or one for all; librosa's ``length=``), by default ``256 * max(T - 1, 0)``.
+    Default offsets pack the items in order, each starting at a multiple of 4 samples (``aligned_offsets``); given
+    offsets must keep the items apart."""
     frames = np.asarray(frames, dtype=np.int64).reshape(-1)
+    if out_len is None:
+        out_len = np.maximum(frames - 1, 0) * HOP
     lens = np.broadcast_to(np.asarray(out_len, dtype=np.int64), frames.shape).copy()
     if (lens < 0).any():
         raise ValueError("output lengths must be >= 0")
@@ -130,15 +131,15 @@ class Context:
                       out_len: Optional[int] = None) -> "FlatBatch":
         """Descriptor of ``n_items`` equal-length spectrogram items, cached: the vocoder is called over and over with
         the same shapes, and planning + pinned staging + upload cost more than the kernels of a short utterance.
-        ``out_len``: output samples per item (librosa's ``length=``; default layout when None)."""
-        key = (int(n_items), int(n_frames), bool(with_chunks), None if out_len is None else int(out_len))
+        ``out_len``: output samples per item (librosa's ``length=``; ``out_layout``'s default when None)."""
+        out_len = int(out_layout([n_frames], out_len)[1][0])
+        key = (int(n_items), int(n_frames), bool(with_chunks), out_len)
         cache = self.__dict__.setdefault("_uniform", {})
         fb = cache.get(key)
         if fb is None:
             if len(cache) >= 64:
                 cache.pop(next(iter(cache)))
-            fb = cache[key] = make_batch(self, n_frames=[n_frames] * n_items, with_chunks=with_chunks,
-                                         out_len=None if out_len is None else [out_len] * n_items)
+            fb = cache[key] = make_batch(self, n_frames=[n_frames] * n_items, with_chunks=with_chunks, out_len=out_len)
         return fb
 
     def side_stream(self) -> "torch.cuda.Stream":
@@ -193,29 +194,22 @@ class FlatBatch:
     table: torch.Tensor         # device uint8 buffer holding frame_off + tile tables
     desc: _lib.SpevBatch
     device: torch.device
-    out_off: Optional[np.ndarray] = None   # int64 [n_items] ISTFT output starts (explicit output layout), else None
-    out_len: Optional[np.ndarray] = None   # int64 [n_items] ISTFT output lengths (explicit output layout), else None
+    out_off: np.ndarray         # int64 [n_items] ISTFT output starts (``out_layout``)
+    out_len: np.ndarray         # int64 [n_items] ISTFT output lengths (``out_layout``)
 
     @property
     def n_out_samples(self) -> int:
-        """size of the flat ISTFT output buffer: sum (T_i - 1) * hop, or the end of the last item of an explicit
-        output layout"""
-        if self.out_len is not None:
-            return int((self.out_off + self.out_len).max(initial=0))
-        return int((self.n_frames - self.n_items) * HOP)
+        """size of the flat ISTFT output buffer: the end of the last item"""
+        return int((self.out_off + self.out_len).max(initial=0))
 
     def out_sample_off(self) -> np.ndarray:
-        """[n_items + 1]: item i's output starts at entry i; the last entry is ``n_out_samples``.  Items are back to
-        back in the default layout; an explicit layout (``out_len``) may leave gaps, which no kernel writes."""
-        if self.out_len is not None:
-            return np.append(self.out_off, self.n_out_samples).astype(np.int64)
-        return (self.frame_off - np.arange(self.n_items + 1)) * HOP
+        """[n_items + 1]: item i's output starts at entry i; the last entry is ``n_out_samples``.  Items may have gaps
+        between them (starts rounded up to 4 samples, or given offsets), which no kernel writes."""
+        return np.append(self.out_off, self.n_out_samples).astype(np.int64)
 
     def out_lengths(self) -> np.ndarray:
-        """[n_items] ISTFT output samples per item: (T_i - 1) * hop, or the explicit lengths."""
-        if self.out_len is not None:
-            return self.out_len.copy()
-        return np.maximum(self.frames - 1, 0) * HOP
+        """[n_items] ISTFT output samples per item."""
+        return self.out_len.copy()
 
     def output_items(self, y: torch.Tensor) -> torch.Tensor:
         """``[n_items, L]`` items of an equal-length batch from its flat ISTFT output ``y`` (``n_out_samples``
@@ -236,17 +230,16 @@ def make_batch(ctx: Context, *, n_samples: Optional[Sequence[int]] = None,
                with_chunks: bool = False, pinned: bool = True, out_len=None,
                out_off: Optional[Sequence[int]] = None) -> FlatBatch:
     """Build the descriptor for items given by sample counts (waveform inputs) or frame counts
-    (spectrogram inputs; sample tiles then describe the implicit ISTFT-output layout).
+    (spectrogram inputs; frame tiles then describe their ISTFT outputs).
     ``sample_off[i]`` is the absolute start of item i in the flat sample buffer (default: items
     packed back to back).  Starts that are multiples of 4 samples take the 16-byte cp.async path;
     whatever lies between items is never read as signal (explicit [lo, hi) bounds per item).
-    ``out_len`` (spectrogram inputs only): item i's ISTFT output has ``out_len[i]`` samples at ``out_off[i]``
-    (librosa's ``length=``; see ``out_layout`` for the default offsets); frame and chunk tiles follow that layout."""
+    ``out_len`` / ``out_off`` (spectrogram inputs only): item i's ISTFT output has ``out_len[i]`` samples at
+    ``out_off[i]`` (librosa's ``length=``; see ``out_layout`` for the defaults); frame and chunk tiles follow that
+    layout."""
     dev = torch.device("cuda", ctx.device)
-    if out_off is not None and out_len is None:
-        raise ValueError("out_off needs out_len")
-    if out_len is not None and n_samples is not None:
-        raise ValueError("out_len describes ISTFT outputs: give n_frames, not n_samples")
+    if n_samples is not None and (out_len is not None or out_off is not None):
+        raise ValueError("out_len / out_off describe ISTFT outputs: give n_frames, not n_samples")
     if n_samples is not None:
         ns = np.asarray(n_samples, dtype=np.int64).reshape(-1)
         frames = 1 + ns // HOP
@@ -255,11 +248,11 @@ def make_batch(ctx: Context, *, n_samples: Optional[Sequence[int]] = None,
         else:
             sample_off = np.asarray(sample_off, dtype=np.int64).reshape(-1)[: len(ns)]
         ftiles = plan_frame_tiles(frames, sample_off, ns)
+        out_off, out_len = out_layout(frames)
     else:
         frames = np.asarray(n_frames, dtype=np.int64).reshape(-1)
         sample_off = None
-        if out_len is not None:
-            out_off, out_len = out_layout(frames, out_len, out_off)
+        out_off, out_len = out_layout(frames, out_len, out_off)
         ftiles = plan_frame_tiles(frames, out_off, out_len)
     n_items = int(len(frames))
     frame_off = np.concatenate([[0], np.cumsum(frames)]).astype(np.int64)

@@ -404,14 +404,13 @@ int spev_tile_chunks(void) { return kTileChunks; }
 int64_t spev_plan_frame_tiles(const int64_t* frames, const int64_t* sample_lo, const int64_t* n_samples,
                               int n_items, spev_tile* out) {
     SPEV_REQUIRE(frames && n_items >= 0, SPEV_E_INVALID, "spev_plan_frame_tiles: frames is null or n_items < 0");
-    SPEV_REQUIRE((sample_lo == nullptr) == (n_samples == nullptr), SPEV_E_INVALID,
-                 "spev_plan_frame_tiles: sample_lo and n_samples go together");
+    SPEV_REQUIRE(sample_lo && n_samples, SPEV_E_INVALID, "spev_plan_frame_tiles: sample_lo or n_samples is null");
+    for (int i = 0; i < n_items; ++i)
+        SPEV_REQUIRE(n_samples[i] >= 0, SPEV_E_INVALID, "spev_plan_frame_tiles: n_samples[%d] = %lld < 0", i,
+                     static_cast<long long>(n_samples[i]));
     int64_t nt = 0, fo = 0;
     for (int i = 0; i < n_items; ++i) {
-        const int64_t T = frames[i];
-        // implicit layout: the ISTFT output of item i, (T-1)*hop samples at hop*(frame_off - i)
-        const int64_t lo = sample_lo ? sample_lo[i] : kHop * (fo - i);
-        const int64_t hi = lo + (n_samples ? n_samples[i] : (T - 1) * kHop);
+        const int64_t T = frames[i], lo = sample_lo[i], hi = lo + n_samples[i];
         for (int64_t t0 = 0; t0 < T; t0 += kTileFrames, ++nt) {
             if (!out) continue;
             spev_tile& d = out[nt];
@@ -427,9 +426,8 @@ int64_t spev_plan_frame_tiles(const int64_t* frames, const int64_t* sample_lo, c
 int64_t spev_plan_chunk_tiles(const int64_t* frames, const int64_t* out_off, const int64_t* out_len, int n_items,
                               spev_tile* out) {
     SPEV_REQUIRE(frames && n_items >= 0, SPEV_E_INVALID, "spev_plan_chunk_tiles: frames is null or n_items < 0");
-    SPEV_REQUIRE((out_off == nullptr) == (out_len == nullptr), SPEV_E_INVALID,
-                 "spev_plan_chunk_tiles: out_off and out_len go together");
-    for (int i = 0; out_len && i < n_items; ++i)
+    SPEV_REQUIRE(out_off && out_len, SPEV_E_INVALID, "spev_plan_chunk_tiles: out_off or out_len is null");
+    for (int i = 0; i < n_items; ++i)
         SPEV_REQUIRE(out_len[i] >= 0, SPEV_E_INVALID, "spev_plan_chunk_tiles: out_len[%d] = %lld < 0", i,
                      static_cast<long long>(out_len[i]));
     // Full tiles first, then the (at most one per item) partial tiles: the persistent kernels hand tile j to CTA
@@ -438,18 +436,15 @@ int64_t spev_plan_chunk_tiles(const int64_t* frames, const int64_t* out_off, con
     for (int pass = 0; pass < 2; ++pass) {
         int64_t fo = 0;
         for (int i = 0; i < n_items; ++i) {
-            // implicit layout: (T-1) whole chunks at hop*(frame_off - i), lo = hi = 0;
-            // output-length layout: ceil(out_len/hop) chunks at out_off, bounded by [lo, hi)
-            const int64_t T = frames[i];
-            const int64_t nc = out_len ? (out_len[i] + kHop - 1) / kHop : T - 1;
-            const int64_t start = out_off ? out_off[i] : kHop * (fo - i);
-            const int64_t lo = out_off ? start : 0, hi = out_len ? start + out_len[i] : 0;
+            // ceil(out_len/hop) chunks at out_off, bounded by [lo, hi)
+            const int64_t T = frames[i], lo = out_off[i], hi = lo + out_len[i];
+            const int64_t nc = (out_len[i] + kHop - 1) / kHop;
             for (int64_t c0 = 0; c0 < nc; c0 += kTileChunks) {
                 const int64_t n = std::min<int64_t>(kTileChunks, nc - c0);
                 if ((n == kTileChunks) != (pass == 0)) continue;
                 if (out) {
                     spev_tile& d = out[nt];
-                    d.src0 = start + kHop * c0; d.lo = lo; d.hi = hi; d.row0 = fo + c0 - 1;
+                    d.src0 = lo + kHop * c0; d.lo = lo; d.hi = hi; d.row0 = fo + c0 - 1;
                     d.n = static_cast<int32_t>(n);
                     d.t0 = static_cast<int32_t>(c0); d.T = static_cast<int32_t>(T); d.item = i;
                 }

@@ -8,7 +8,7 @@
 //                   gather overlap-add (each output sample owner sums its <= 4 frames in
 //                   ascending frame order, no atomics) fused with window-sum-square
 //                   normalisation.            Replaces librosa.istft under :730-733.
-//                   Chunk tiles with hi > lo bound the output explicitly (librosa's istft(length=)):
+//                   Chunk tiles carry each item's output bounds [lo, hi) (librosa's istft(length=)):
 //                   every sample of [lo, hi) is written, nothing outside it.
 // K5 k_stft_phase_w : STFT of the rebuilt signal fused with Griffin-Lim's momentum / phase
 //                   normalisation update, one frame pair per warp.  Replaces librosa.stft + the angle
@@ -729,9 +729,9 @@ k_gl_fused(BatchView bv, const float* __restrict__ y, const float* __restrict__ 
 // ---------------------------------------------------------------------------------------
 // K4: ISTFT with gather overlap-add and window-sum-square normalisation
 //
-// Output chunk c (samples [256c, 256c + 256) of the item) sums frames c-1 .. c+2 that exist.  Without an explicit
-// bound an item has chunks 0 .. T-2.  With one (hi > lo: librosa's istft(length=L), ceil(L / 256) chunks) it may also
-// have chunk T-1 (frames T-2, T-1), chunk T (frame T-1) and later chunks with no frame, written as 0; all of them take
+// Output chunk c (samples [256c, 256c + 256) of the item) sums frames c-1 .. c+2 that exist.  An item of L = hi - lo
+// samples (librosa's istft(length=L)) has ceil(L / 256) chunks: 0 .. T-2 for the default L = (T-1)*256, and beyond
+// that chunk T-1 (frames T-2, T-1), chunk T (frame T-1) and later chunks with no frame, written as 0; all of these take
 // the per-sample edge normalisation.  Only the item's last chunk can be partial, and only its stores are masked.
 // ---------------------------------------------------------------------------------------
 // BULK: a warp's two spectrum rows (8,272 B) arrive in its region by ONE bulk asynchronous copy instead of 34 scattered
@@ -852,13 +852,12 @@ k_istft(BatchView bv, const float2* __restrict__ spec, int64_t ld, float* __rest
             });
         }
         __syncthreads();
-        // gather: chunk c = c0 + cl receives frames c-1, c, c+1, c+2 (ascending), local cl..cl+3.  An explicit output
-        // bound (hi > lo) may end inside the item's last chunk: only that chunk stores fewer than kHop samples.
+        // gather: chunk c = c0 + cl receives frames c-1, c, c+1, c+2 (ascending), local cl..cl+3.  The item's output
+        // bound hi may end inside its last chunk: only that chunk stores fewer than kHop samples.
         for (int cl = warp; cl < nchunks; cl += kWarps) {
             const int c = c0 + cl;
             float* yo_c = y + d.src0 + static_cast<int64_t>(cl) * kHop;
-            const int nv = d.hi > d.lo ? static_cast<int>(min(static_cast<int64_t>(kHop), d.hi - d.src0 - static_cast<int64_t>(cl) * kHop))
-                                       : kHop;
+            const int nv = static_cast<int>(min(static_cast<int64_t>(kHop), d.hi - d.src0 - static_cast<int64_t>(cl) * kHop));
             if (c >= 1 && c + 2 < T) {   // all four frames exist: table-driven normalisation
                 const float* f0 = s_x + (cl >> 1) * kWarpRegionWords + (cl & 1) * kNfft + lane;
                 const float* f1 = s_x + ((cl + 1) >> 1) * kWarpRegionWords + ((cl + 1) & 1) * kNfft + lane;
@@ -902,9 +901,9 @@ k_istft(BatchView bv, const float2* __restrict__ spec, int64_t ld, float* __rest
 // j with 0 <= q - 2j <= 4 -- two or three of them --, summed here in ascending pair order and normalised by the
 // window-sum-square exactly as k_istft does (table for interior chunks, per-sample sum over the existing frames at
 // the item edges).  One warp per chunk, 16-byte loads and stores, no shared-memory staging: a pure streaming kernel.
-// With an explicit output bound (chunk tiles with hi > lo) an item may also have chunk T-1 (frames T-2, T-1: pairs
-// covering them are selected by the same rule, a lone last frame included) and chunk T (frame T-1 alone); later chunks
-// meet no segment and are written as 0.  Only the item's last chunk can be partial; it stores sample by sample.
+// An item longer than (T-1)*256 samples (chunk tile bound hi) also has chunk T-1 (frames T-2, T-1: pairs covering
+// them are selected by the same rule, a lone last frame included) and chunk T (frame T-1 alone); later chunks meet no
+// segment and are written as 0.  Only the item's last chunk can be partial; it stores sample by sample.
 // ---------------------------------------------------------------------------------------
 constexpr int kOlaWarps = 8;
 constexpr int kOlaPerWarp = 1;                                           // chunks per warp (2 measured: no gain)
@@ -924,10 +923,9 @@ k_ola_pairs(BatchView bv, const float* __restrict__ seg, int64_t ld_f, float* __
     const int64_t item_row = __ldg(&d->row0) - t0 + 1;
     const int64_t src0 = __ldg(&d->src0);
     float* yo0 = y + src0;
-    // an explicit output bound (hi > lo) that ends inside this warp's chunks: kept as one predicate, the exact count is
-    // re-read from the descriptor only on that path
-    const bool bounded_tail = __ldg(&d->hi) > __ldg(&d->lo) &&
-                              __ldg(&d->hi) - src0 - static_cast<int64_t>(cl0) * kHop < kOlaPerWarp * kHop;
+    // the item's output bound hi ends inside this warp's chunks: kept as one predicate, the exact count is re-read from
+    // the descriptor only on that path
+    const bool bounded_tail = __ldg(&d->hi) - src0 - static_cast<int64_t>(cl0) * kHop < kOlaPerWarp * kHop;
     const int n_pairs = (T + 1) >> 1;
     const int s0 = 4 * lane, s1 = 128 + 4 * lane;
     pdl_wait();   // the segments come from the previous kernel

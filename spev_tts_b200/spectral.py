@@ -213,13 +213,13 @@ def istft(X: ArrayLike, *, hop_length=None, win_length=None, n_fft=None, window=
     lead, T = t.shape[:-2], t.shape[-1]
     b = int(np.prod(lead)) if lead else 1
     ctx = Context.get(t.device)
-    L = (T - 1) * HOP if length is None else length
-    batch = make_batch(ctx, n_frames=[T] * b, with_chunks=True, out_len=None if length is None else [L] * b)
+    batch = make_batch(ctx, n_frames=[T] * b, with_chunks=True, out_len=length)
     spec = _spec_to_internal(t.reshape(b, nb, T))
     y = torch.empty(batch.n_out_samples, dtype=torch.float32, device=t.device)
     _lib.check(ctx.lib.spev_istft(ctx.handle, batch.desc, spec.data_ptr(), _lib.SPEC_LD, y.data_ptr(),
                                   stream_ptr(t.device)), "spev_istft")
-    return _ret(batch.output_items(y).view(*lead, L), was_numpy)
+    items = batch.output_items(y)
+    return _ret(items.view(*lead, items.shape[1]), was_numpy)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -365,14 +365,13 @@ def griffinlim_flat(S: torch.Tensor, batch: FlatBatch, ctx: Context, *, n_iter=3
                     out: Optional[torch.Tensor] = None, workspace: Optional[torch.Tensor] = None):
     """``S``: ``[F, 520]`` float32 magnitudes; ``init_phase``: ``[F, 513]`` float32 radians or None.
     Returns the flat waveform buffer (item i at ``batch.out_sample_off()[i]``, ``batch.out_lengths()[i]`` samples).
-    A batch built with ``out_len`` runs librosa's ``griffinlim(length=out_len[i])`` per item: every inner ISTFT writes
-    those samples and the next STFT re-analyses them; each length must satisfy ``1 + out_len[i] // 256 == T_i``."""
+    Item i runs librosa's ``griffinlim(length=out_len[i])`` (``make_batch(..., out_len=)``): every inner ISTFT writes
+    those samples and the next STFT re-analyses them; items with frames must satisfy ``1 + out_len[i] // 256 == T_i``."""
     lib = ctx.lib
-    if batch.out_len is not None:
-        bad = np.flatnonzero(1 + batch.out_len // HOP != batch.frames)
-        if len(bad):
-            i = int(bad[0])
-            _gl_length(int(batch.out_len[i]), int(batch.frames[i]))      # raises, naming the valid range
+    bad = np.flatnonzero((batch.frames >= 1) & (1 + batch.out_len // HOP != batch.frames))
+    if len(bad):
+        i = int(bad[0])
+        _gl_length(int(batch.out_len[i]), int(batch.frames[i]))      # raises, naming the valid range
     need = lib.spev_griffinlim_workspace_bytes(batch.n_frames)
     if workspace is None or workspace.numel() < need:
         workspace = torch.empty(need, dtype=torch.uint8, device=S.device)
@@ -409,13 +408,12 @@ def griffinlim(S: ArrayLike, *, n_iter=32, hop_length=None, win_length=None, n_f
     lead, T = t.shape[:-2], t.shape[-1]
     b = int(np.prod(lead)) if lead else 1
     ctx = Context.get(t.device)
-    L = (T - 1) * HOP if length is None else length
-    batch = make_batch(ctx, n_frames=[T] * b, with_chunks=True, out_len=None if length is None else [L] * b)
+    batch = make_batch(ctx, n_frames=[T] * b, with_chunks=True, out_len=length)
     Sf = items_to_rows(t.reshape(b, nb, T), _lib.SPEC_LD, out=torch.zeros((b * T, _lib.SPEC_LD), dtype=torch.float32, device=t.device))
     ph = _phase_to_internal(init_phase, b, T, t.device) if init_phase is not None else None
     seed = int(np.random.SeedSequence(random_state).generate_state(2, dtype=np.uint32).view(np.uint64)[0])
-    y = griffinlim_flat(Sf, batch, ctx, n_iter=n_iter, momentum=momentum, init_phase=ph, seed=seed)
-    return _ret(batch.output_items(y).view(*lead, L), was_numpy)
+    items = batch.output_items(griffinlim_flat(Sf, batch, ctx, n_iter=n_iter, momentum=momentum, init_phase=ph, seed=seed))
+    return _ret(items.view(*lead, items.shape[1]), was_numpy)
 
 
 def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_length=None, window="hann",
@@ -435,7 +433,6 @@ def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_len
     lead, n_mels, T = t.shape[:-2], t.shape[-2], t.shape[-1]
     b = int(np.prod(lead)) if lead else 1
     ctx = Context.get(t.device, sr=sr, n_mels=n_mels, fmin=fmin, fmax=fmax)
-    L = (T - 1) * HOP if length is None else length
     batch = ctx.uniform_batch(b, T, with_chunks=True, out_len=length)
     tm = items_to_rows(t.reshape(b, n_mels, T)).view(-1)                  # frame-major -> tensor-core GEMM
     S = mel_to_mag_flat(tm, batch, ctx, layout=0, is_log=is_log)
@@ -453,4 +450,5 @@ def mel_to_audio(M: ArrayLike, *, sr=22050, n_fft=2048, hop_length=None, win_len
             run_gl()
     else:
         run_gl()
-    return _ret(batch.output_items(out["y"]).view(*lead, L), was_numpy)
+    items = batch.output_items(out["y"])
+    return _ret(items.view(*lead, items.shape[1]), was_numpy)

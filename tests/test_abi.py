@@ -20,7 +20,7 @@ def header_symbols():
     return sorted(set(re.findall(r"SPEV_API\s+[\w\s\*]+?\b(spev_\w+)\s*\(", src)))
 
 
-def test_library_builds_exports_header_symbols_abi_2():
+def test_library_builds_exports_header_symbols_abi_3():
     import spev_tts_b200 as sp
     from spev_tts_b200 import build
     build.build()
@@ -33,7 +33,7 @@ def test_library_builds_exports_header_symbols_abi_2():
     out = subprocess.check_output(["nm", "-D", "--defined-only", sp.LIB_PATH], text=True)
     exported = sorted(l.split()[-1] for l in out.splitlines() if " T " in l)
     assert exported == syms, "library exports symbols outside the header (or misses some)"
-    assert lib.spev_abi_version() == 2 and lib.spev_tile_chunks() == lib.spev_tile_frames() - 3
+    assert lib.spev_abi_version() == 3 and lib.spev_tile_chunks() == lib.spev_tile_frames() - 3
 
 
 def test_sass_is_sm100a():
@@ -58,8 +58,8 @@ def test_host_constants_match_oracle():
 
 def test_plan_tiles_count_query_and_closed_forms():
     """spev_plan_frame_tiles / spev_plan_chunk_tiles: the count query (out == NULL) equals the number of tiles the fill
-    writes, for both frame layouts and both chunk layouts, and the counts are sum ceil(T/32), sum ceil((T-1)/29) and
-    sum ceil(ceil(L/256)/29)."""
+    writes, for waveform and ISTFT-output frame tiles and for default and explicit output lengths, and the counts are
+    sum ceil(T/32), sum ceil((T-1)/29) and sum ceil(ceil(L/256)/29)."""
     import spev_tts_b200 as sp
     from spev_tts_b200 import batch as B
     lib = sp.load()
@@ -72,24 +72,22 @@ def test_plan_tiles_count_query_and_closed_forms():
     out_len = rng.integers(0, 260 * 200, 50).astype(np.int64)
     out_len[:4] = [0, 1, 256, 29 * 256 + 1]
     out_off = B.out_layout(frames, out_len)[0]
-
-    def ptr(a):
-        return None if a is None else a.ctypes.data
+    def_off, def_len = B.out_layout(frames)
 
     def count_and_fill(fn, a, b):
-        cnt = fn(ptr(frames), ptr(a), ptr(b), len(frames), None)
+        cnt = fn(frames.ctypes.data, a.ctypes.data, b.ctypes.data, len(frames), None)
         out = np.zeros(cnt + 1, dtype=B.TILE_DTYPE)           # one spare record, which the fill must not touch
-        assert fn(ptr(frames), ptr(a), ptr(b), len(frames), out.ctypes.data) == cnt
+        assert fn(frames.ctypes.data, a.ctypes.data, b.ctypes.data, len(frames), out.ctypes.data) == cnt
         assert out[cnt:].tobytes() == bytes(B.TILE_DTYPE.itemsize)
         return cnt
-    for lo, n in ((starts, ns), (None, None)):
+    for lo, n in ((starts, ns), (def_off, def_len)):
         assert count_and_fill(lib.spev_plan_frame_tiles, lo, n) == int(((frames + tf - 1) // tf).sum())
-    assert count_and_fill(lib.spev_plan_chunk_tiles, None, None) == int(((frames - 1 + tc - 1) // tc).sum())
+    assert count_and_fill(lib.spev_plan_chunk_tiles, def_off, def_len) == int(((frames - 1 + tc - 1) // tc).sum())
     nc = (out_len + 255) // 256
     assert count_and_fill(lib.spev_plan_chunk_tiles, out_off, out_len) == int(((nc + tc - 1) // tc).sum())
     # every frame / chunk covered exactly once
-    assert B.plan_frame_tiles(frames)["n"].sum() == frames.sum()
-    assert B.plan_chunk_tiles(frames)["n"].sum() == (frames - 1).sum()
+    assert B.plan_frame_tiles(frames, def_off, def_len)["n"].sum() == frames.sum()
+    assert B.plan_chunk_tiles(frames, out_off=def_off, out_len=def_len)["n"].sum() == (frames - 1).sum()
     assert B.plan_chunk_tiles(frames, out_off=out_off, out_len=out_len)["n"].sum() == nc.sum()
 
 
@@ -158,11 +156,19 @@ def test_host_entry_points_and_planners_reject_bad_arguments():
     assert lib.spev_plan_chunk_tiles(None, None, None, 3, None) == -1
     frames, off, lens = (np.array(v, dtype=np.int64) for v in ([3, 3], [0, 1024], [512, -1]))
     assert lib.spev_plan_chunk_tiles(frames.ctypes.data, off.ctypes.data, None, 2, None) == -1    # out_off, no out_len
+    assert b"out_len is null" in lib.spev_last_error()
+    assert lib.spev_plan_chunk_tiles(frames.ctypes.data, None, None, 2, None) == -1
     assert lib.spev_plan_chunk_tiles(frames.ctypes.data, off.ctypes.data, lens.ctypes.data, 2, None) == -1
     assert b"out_len[1]" in lib.spev_last_error()
+    assert lib.spev_plan_frame_tiles(frames.ctypes.data, None, lens.ctypes.data, 2, None) == -1   # no sample_lo
+    assert b"sample_lo or n_samples is null" in lib.spev_last_error()
+    assert lib.spev_plan_frame_tiles(frames.ctypes.data, off.ctypes.data, lens.ctypes.data, 2, None) == -1
+    assert b"n_samples[1]" in lib.spev_last_error()
     from spev_tts_b200 import batch as B
     with pytest.raises(ValueError, match="out_len"):
         B.plan_chunk_tiles(frames, out_off=off, out_len=lens)
+    with pytest.raises(ValueError, match="n_samples"):
+        B.plan_frame_tiles(frames, off, lens)
     assert lib.spev_host_mel_basis(0, 1024, 80, 0.0, 0.0, None) == -1
     assert lib.spev_griffinlim_workspace_bytes(-5) == 0
     assert lib.spev_griffinlim_workspace_bytes(10) >= 10 * 520 * 16

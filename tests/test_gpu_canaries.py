@@ -56,7 +56,7 @@ def test_forward_kernels_stay_in_bounds(cuda, lens):
     assert bool(torch.isfinite(r.check("rms")).all()) and bool(torch.isfinite(c.check("centroid")).all())
 
 
-@pytest.mark.parametrize("frames", [[1], [2, 3], [29, 30, 31, 32, 33], [100, 1, 64]])
+@pytest.mark.parametrize("frames", [[1], [2, 3], [29, 30, 31, 32, 33], [100, 1, 64], [0, 5], [3, 0, 0, 40]])
 def test_griffinlim_kernels_stay_in_bounds(cuda, frames):
     import spev_tts_b200 as sp
     from spev_tts_b200 import _lib

@@ -1,6 +1,6 @@
 """GPU: exact-length inverse transforms (librosa's ``length=``) for istft, griffinlim and mel_to_audio.
-Chunk tiles with hi > lo bound each item's output explicitly; the ISTFT kernels (k_istft, k_ola_pairs) write every
-sample of [lo, hi) and nothing else, and the fused Griffin-Lim iteration re-analyses exactly those samples."""
+Chunk tiles bound each item's output by [lo, hi); the ISTFT kernels (k_istft, k_ola_pairs) write every sample of it
+and nothing else, and the fused Griffin-Lim iteration re-analyses exactly those samples."""
 import numpy as np
 import pytest
 import torch

@@ -116,9 +116,30 @@ def test_c_length_planner_covers_every_sample_once(built):
         assert not (full[1:] & ~full[:-1]).any()               # full tiles first
         ft = B.plan_frame_tiles(frames, off, L)
         assert np.array_equal(ft["lo"], off[ft["item"]]) and np.array_equal(ft["hi"], (off + L)[ft["item"]])
-    # without a layout: the plain planner (lo = hi = 0)
+    # the default layout: (T-1)*256 samples per item, bounded like any other
     frames = np.array([800, 33, 1, 2, 64])
-    assert not B.plan_chunk_tiles(frames)["hi"].any()
+    off, L = B.out_layout(frames)
+    assert np.array_equal(L, (frames - 1) * 256) and np.array_equal(off, np.concatenate([[0], np.cumsum(L)[:-1]]))
+    tiles = B.plan_chunk_tiles(frames, out_off=off, out_len=L)
+    assert np.array_equal(tiles["lo"], off[tiles["item"]]) and np.array_equal(tiles["hi"], (off + L)[tiles["item"]])
+
+
+def test_default_layout_of_items_without_frames(built):
+    """Items with T = 0 take no output samples, leading or in the middle: every bound and chunk start is >= 0, the
+    items are disjoint, and the buffer ends at the last item's end."""
+    for frames in ([0, 5], [3, 0, 0, 40], [0, 0, 2, 0, 33, 0]):
+        frames = np.array(frames)
+        off, L = B.out_layout(frames)
+        assert np.array_equal(L, np.maximum(frames - 1, 0) * 256)
+        order = np.argsort(off, kind="stable")
+        assert (off >= 0).all() and (off[order][1:] >= (off + L)[order][:-1]).all()
+        ft = B.plan_frame_tiles(frames, off, L)
+        ct = B.plan_chunk_tiles(frames, out_off=off, out_len=L)
+        for t in (ft, ct):
+            assert (t["lo"] >= 0).all() and np.array_equal(t["hi"], (off + L)[t["item"]])
+        assert (ct["src0"] >= 0).all() and (ct["src0"] + 256 * ct["n"] <= ct["hi"]).all()
+        assert set(ft["item"]) == set(np.flatnonzero(frames >= 1)) and set(ct["item"]) == set(np.flatnonzero(frames >= 2))
+        assert int((off + L).max()) == int(L.sum())                # [0, 5]: the 1,024 samples item 1 needs
 
 
 def test_out_layout_rejects_bad_layouts():
@@ -136,8 +157,7 @@ def test_output_items_of_the_flat_output_layout():
     from a buffer of exactly ``n_out_samples``; unequal lengths or spacing are refused."""
     def host_batch(frames, out_len=None, out_off=None):
         frames = np.asarray(frames, dtype=np.int64)
-        if out_len is not None:
-            out_off, out_len = B.out_layout(frames, out_len, out_off)
+        out_off, out_len = B.out_layout(frames, out_len, out_off)
         fo = np.concatenate([[0], np.cumsum(frames)])
         return B.FlatBatch(len(frames), int(fo[-1]), frames, None, fo, 0, 0, None, None, torch.device("cpu"),
                            out_off=out_off, out_len=out_len)

@@ -73,12 +73,15 @@ def test_c_planned_tiles_cover_everything_once_in_order(planners, n_samples):
         assert t["lo"] == starts[t["item"]] and t["hi"] == t["lo"] + ns[t["item"]]
         covered[t["row0"]: t["row0"] + t["n"]] += 1
     assert np.all(covered == 1)
-    ct = B.plan_chunk_tiles(frames)
+    # the default ISTFT output layout: (T-1)*256 samples per item, back to back
+    off, L = B.out_layout(frames)
     yo = (fo - np.arange(len(fo))) * 256
+    assert np.array_equal(off, yo[:-1]) and np.array_equal(L, np.diff(yo))
+    ct = B.plan_chunk_tiles(frames, out_off=off, out_len=L)
     cov = np.zeros(yo[-1] // 256, dtype=np.int32)
     for t in ct:
         assert 1 <= t["n"] <= 29 and t["t0"] % 29 == 0
-        assert t["lo"] == t["hi"] == 0 and t["T"] == frames[t["item"]]
+        assert t["lo"] == yo[t["item"]] and t["hi"] == yo[t["item"] + 1] and t["T"] == frames[t["item"]]
         assert t["src0"] == yo[t["item"]] + 256 * t["t0"] and t["row0"] == fo[t["item"]] + t["t0"] - 1
         cov[t["src0"] // 256: t["src0"] // 256 + t["n"]] += 1
     assert np.all(cov == 1)

@@ -6,7 +6,8 @@ cfg3 is 16 items x 800 frames, 60 iterations, with seeded magnitudes and initial
 back-to-back calls with device events, once per variant, the variants alternating round by round:
   default  : no length, this build ((T-1)*256 = 204,544 samples per item)
   length   : length = 204,799 per item (T*256 - 1: the worst case, a 255-sample tail re-analysed every iteration)
-  parent   : no length, another build of the library (--parent-lib, e.g. the parent commit's), for outputs and time.
+  parent   : no length, another build of the library (--parent-lib, e.g. the parent commit's), for outputs and time,
+             on tile tables planned by that build's own planners.
 The default output must be bit-identical to the parent's.  The card name and power limit are printed with the numbers.
 Prints one JSON line; --out also writes it to DIR/gl_length_bench.json.
 """
@@ -16,6 +17,7 @@ import json
 import os
 import subprocess
 import sys
+import types
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np  # noqa: E402
@@ -36,7 +38,8 @@ class Lib:
             self.lib = _lib.load()
         else:
             self.lib = C.CDLL(os.path.abspath(path))
-            for name in ("spev_create", "spev_destroy", "spev_griffinlim", "spev_griffinlim_workspace_bytes", "spev_last_error"):
+            for name in ("spev_abi_version", "spev_create", "spev_destroy", "spev_griffinlim",
+                         "spev_griffinlim_workspace_bytes", "spev_last_error", "spev_plan_frame_tiles", "spev_plan_chunk_tiles"):
                 res, args = _lib._SIGS[name]
                 getattr(self.lib, name).restype = res
                 getattr(self.lib, name).argtypes = args
@@ -47,6 +50,25 @@ class Lib:
     def _check(self, rc):
         if rc != 0:
             raise RuntimeError(f"spev call failed ({rc}): {self.lib.spev_last_error().decode(errors='replace')}")
+
+    def replan(self, fb, dev):
+        """The batch ``fb`` with tile tables from this build's own planners.  Builds before ABI 3 plan the default
+        output layout from NULL layout arrays (chunk tiles with lo = hi = 0)."""
+        layout = [fb.out_off, fb.out_len] if self.lib.spev_abi_version() >= 3 else [None, None]
+        args = [fb.frames.ctypes.data] + [None if a is None else a.ctypes.data for a in layout] + [fb.n_items]
+        tables = []
+        for fn in (self.lib.spev_plan_frame_tiles, self.lib.spev_plan_chunk_tiles):
+            n = fn(*args, None)
+            if n < 0:
+                self._check(n)
+            tables.append(np.empty(n, dtype=sp.batch.TILE_DTYPE))
+            fn(*args, tables[-1].ctypes.data)
+        ft, ct = tables
+        table = torch.from_numpy(np.concatenate([ft.view(np.uint8), ct.view(np.uint8), fb.frame_off.view(np.uint8)])).to(dev)
+        d = _lib.SpevBatch()
+        d.n_items, d.n_frames, d.n_ftiles, d.n_ctiles = fb.n_items, fb.n_frames, len(ft), len(ct)
+        d.ftiles, d.ctiles, d.frame_off = table.data_ptr(), table.data_ptr() + ft.nbytes, table.data_ptr() + ft.nbytes + ct.nbytes
+        return types.SimpleNamespace(desc=d, table=table, n_out_samples=fb.n_out_samples)
 
     def griffinlim(self, fb, S, ph, y, ws, st):
         self._check(self.lib.spev_griffinlim(self.handle, fb.desc, S.data_ptr(), S.shape[1], ph.data_ptr(), 7, N_ITER, 0.99,
@@ -74,7 +96,8 @@ def main():
     cur = Lib(None, dev)
     libs = {"default": (cur, fb_def), "length": (cur, fb_len)}
     if a.parent_lib:
-        libs["parent"] = (Lib(a.parent_lib, dev), fb_def)
+        parent = Lib(a.parent_lib, dev)
+        libs["parent"] = (parent, parent.replan(fb_def, dev))
     ys = {k: torch.empty(fb.n_out_samples, device=dev) for k, (_, fb) in libs.items()}
 
     def run(k, n):
