@@ -53,31 +53,6 @@ k_pad_ragged(PadParams p) {
     }
 }
 
-int launch_collate(const spev_pad_array* arrays, int n_arrays, const int64_t* frame_off, const int64_t* phone_off,
-                   const int64_t* sel, int B, int64_t t_max, int64_t p_max, cudaStream_t st) {
-    SPEV_REQUIRE(n_arrays >= 0 && n_arrays <= kMaxPadArrays && B >= 0 && t_max >= 0 && p_max >= 0, SPEV_E_INVALID,
-                 "collate: bad sizes (at most %d arrays)", kMaxPadArrays);
-    if (n_arrays == 0 || B == 0) return SPEV_OK;
-    SPEV_REQUIRE(arrays && B <= 65535, SPEV_E_INVALID, "collate: null arrays or B > 65535");
-    PadParams p{};
-    p.n_arrays = n_arrays; p.B = B; p.t_max = t_max; p.p_max = p_max;
-    p.frame_off = frame_off; p.phone_off = phone_off; p.sel = sel;
-    int64_t max_bytes = 0;
-    for (int i = 0; i < n_arrays; ++i) {
-        SPEV_REQUIRE(arrays[i].src && arrays[i].dst && arrays[i].row_bytes > 0, SPEV_E_INVALID, "collate: array %d incomplete", i);
-        SPEV_REQUIRE(arrays[i].per_phone ? phone_off != nullptr : frame_off != nullptr, SPEV_E_INVALID,
-                     "collate: array %d needs an offset table that was not given", i);
-        p.a[i] = arrays[i];
-        max_bytes = std::max(max_bytes, (arrays[i].per_phone ? p_max : t_max) * arrays[i].row_bytes);
-    }
-    if (max_bytes == 0) return SPEV_OK;
-    dim3 grid(static_cast<unsigned>((max_bytes + kPadBytesPerCta - 1) / kPadBytesPerCta), static_cast<unsigned>(B),
-              static_cast<unsigned>(n_arrays));
-    k_pad_ragged<<<grid, kPadThreads, 0, st>>>(p);
-    SPEV_CUDA(cudaGetLastError());
-    return SPEV_OK;
-}
-
 // ---- segmented copy: dst[dst_off[i] .. +nbytes[i]) = src[src_off[i] .. +nbytes[i]) -------------------------------
 // Re-orders a gathered cache (rank-major rows) into corpus order, or packs scattered utterances into a shard: each
 // segment is a contiguous run of rows.  CTA <-> 16 KB piece of one segment (binary search in the piece prefix table).
@@ -109,18 +84,6 @@ k_copy_segments(const unsigned char* __restrict__ src, unsigned char* __restrict
     }
 }
 
-int launch_copy_segments(const void* src, void* dst, const int64_t* src_off, const int64_t* dst_off, const int64_t* nbytes,
-                         const int64_t* piece_off, int n_seg, int64_t n_pieces, cudaStream_t st) {
-    SPEV_REQUIRE(n_seg >= 0 && n_pieces >= 0, SPEV_E_INVALID, "copy_segments: negative sizes");
-    if (n_seg == 0 || n_pieces == 0) return SPEV_OK;
-    SPEV_REQUIRE(src && dst && src_off && dst_off && nbytes && piece_off, SPEV_E_INVALID, "copy_segments: null buffer");
-    const int grid = static_cast<int>(std::min<int64_t>(n_pieces, 148 * 32));
-    k_copy_segments<<<grid, kPadThreads, 0, st>>>(static_cast<const unsigned char*>(src), static_cast<unsigned char*>(dst),
-                                                  src_off, dst_off, nbytes, piece_off, n_seg, n_pieces);
-    SPEV_CUDA(cudaGetLastError());
-    return SPEV_OK;
-}
-
 // ---- batched 2-D transpose: dst[b][c][r] = src[b][r][c] -------------------------------------------------------------
 // librosa lays spectra and mels out as [..., bins, T]; the kernels here work on frame-major rows [F, pitch].  This is
 // the layout change between the two (32 x 32 tiles through padded shared memory, coalesced on both sides), for 4-byte
@@ -149,14 +112,46 @@ k_transpose(const T* __restrict__ src, T* __restrict__ dst, int rows, int cols, 
     }
 }
 
-int launch_transpose(const void* src, void* dst, int elem_bytes, int64_t batches, int rows, int cols, int64_t src_pitch,
-                     int64_t src_batch, int64_t dst_pitch, int64_t dst_batch, cudaStream_t st) {
+}  // namespace spev
+
+using namespace spev;
+
+extern "C" {
+
+int spev_collate(const spev_pad_array* arrays, int n_arrays, const int64_t* frame_off, const int64_t* phone_off,
+                 const int64_t* sel, int B, int64_t t_max, int64_t p_max, void* stream) {
+    SPEV_REQUIRE(n_arrays >= 0 && n_arrays <= kMaxPadArrays && B >= 0 && t_max >= 0 && p_max >= 0, SPEV_E_INVALID,
+                 "collate: bad sizes (at most %d arrays)", kMaxPadArrays);
+    if (n_arrays == 0 || B == 0) return SPEV_OK;
+    SPEV_REQUIRE(arrays && B <= 65535, SPEV_E_INVALID, "collate: null arrays or B > 65535");
+    PadParams p{};
+    p.n_arrays = n_arrays; p.B = B; p.t_max = t_max; p.p_max = p_max;
+    p.frame_off = frame_off; p.phone_off = phone_off; p.sel = sel;
+    int64_t max_bytes = 0;
+    for (int i = 0; i < n_arrays; ++i) {
+        SPEV_REQUIRE(arrays[i].src && arrays[i].dst && arrays[i].row_bytes > 0, SPEV_E_INVALID, "collate: array %d incomplete", i);
+        SPEV_REQUIRE(arrays[i].per_phone ? phone_off != nullptr : frame_off != nullptr, SPEV_E_INVALID,
+                     "collate: array %d needs an offset table that was not given", i);
+        p.a[i] = arrays[i];
+        max_bytes = std::max(max_bytes, (arrays[i].per_phone ? p_max : t_max) * arrays[i].row_bytes);
+    }
+    if (max_bytes == 0) return SPEV_OK;
+    dim3 grid(static_cast<unsigned>((max_bytes + kPadBytesPerCta - 1) / kPadBytesPerCta), static_cast<unsigned>(B),
+              static_cast<unsigned>(n_arrays));
+    k_pad_ragged<<<grid, kPadThreads, 0, static_cast<cudaStream_t>(stream)>>>(p);
+    SPEV_CUDA(cudaGetLastError());
+    return SPEV_OK;
+}
+
+int spev_transpose_batched(const void* src, void* dst, int elem_bytes, int64_t batches, int rows, int cols, int64_t src_pitch,
+                           int64_t src_batch, int64_t dst_pitch, int64_t dst_batch, void* stream) {
     SPEV_REQUIRE(batches >= 0 && rows >= 0 && cols >= 0, SPEV_E_INVALID, "transpose: negative shape");
     if (batches == 0 || rows == 0 || cols == 0) return SPEV_OK;
     SPEV_REQUIRE(src && dst && src_pitch >= cols && dst_pitch >= rows, SPEV_E_INVALID, "transpose: null buffer or pitch < extent");
     SPEV_REQUIRE(elem_bytes == 4 || elem_bytes == 8, SPEV_E_UNSUPPORTED, "transpose: 4- or 8-byte elements only");
     SPEV_REQUIRE(batches <= 65535, SPEV_E_UNSUPPORTED, "transpose: more than 65535 batches");
     dim3 grid(static_cast<unsigned>((cols + 31) / 32), static_cast<unsigned>((rows + 31) / 32), static_cast<unsigned>(batches));
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (elem_bytes == 4)
         k_transpose<float><<<grid, 256, 0, st>>>(static_cast<const float*>(src), static_cast<float*>(dst), rows, cols, src_pitch,
                                                 src_batch, dst_pitch, dst_batch);
@@ -167,4 +162,18 @@ int launch_transpose(const void* src, void* dst, int elem_bytes, int64_t batches
     return SPEV_OK;
 }
 
-}  // namespace spev
+int spev_copy_segments_piece_bytes(void) { return kPadBytesPerCta; }
+
+int spev_copy_segments(const void* src, void* dst, const int64_t* src_off, const int64_t* dst_off, const int64_t* nbytes,
+                       const int64_t* piece_off, int n_seg, int64_t n_pieces, void* stream) {
+    SPEV_REQUIRE(n_seg >= 0 && n_pieces >= 0, SPEV_E_INVALID, "copy_segments: negative sizes");
+    if (n_seg == 0 || n_pieces == 0) return SPEV_OK;
+    SPEV_REQUIRE(src && dst && src_off && dst_off && nbytes && piece_off, SPEV_E_INVALID, "copy_segments: null buffer");
+    const int grid = static_cast<int>(std::min<int64_t>(n_pieces, 148 * 32));
+    k_copy_segments<<<grid, kPadThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+        static_cast<const unsigned char*>(src), static_cast<unsigned char*>(dst), src_off, dst_off, nbytes, piece_off, n_seg, n_pieces);
+    SPEV_CUDA(cudaGetLastError());
+    return SPEV_OK;
+}
+
+}  // extern "C"

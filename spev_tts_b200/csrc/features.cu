@@ -12,6 +12,7 @@
 //     sigma, lo, hi) -- the e / bri (and, with mu=1, sigma=-1, the br) lines of :400-417.  One warp
 //     per utterance: warp-scan of the durations, then one lane per phoneme.
 #include <algorithm>
+#include <cmath>
 #include "spev_internal.cuh"
 #include "tile_pipe.cuh"
 
@@ -162,40 +163,69 @@ __global__ void k_segment_pool(const float* __restrict__ curve, const int64_t* _
     }
 }
 
-// ---- launchers -----------------------------------------------------------------------------------
-int launch_frame_features(spev_ctx* ctx, const spev_batch* b, const float* samples, float* rms, float* centroid,
-                          cudaStream_t st) {
-    SPEV_REQUIRE(ctx && b, SPEV_E_INVALID, "null ctx or batch");
-    if (b->n_ftiles == 0) return SPEV_OK;
-    SPEV_REQUIRE(samples && rms && centroid && b->ftiles, SPEV_E_INVALID, "frame_features: null buffer");
-    const size_t smem = sizeof(float2) * (1024 + 1024 + 512) + sizeof(spev_tile) * kRing + sizeof(float) * kFeatStage +
-                        sizeof(float) * kWarps * kWarpRegionWords;
-    SPEV_CUDA(cudaFuncSetAttribute(k_frame_features, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    const int grid = std::min<int64_t>(b->n_ftiles, ctx->num_sms);
-    BatchView bv = view_of(b);
-    k_frame_features<<<grid, kThreads, smem, st>>>(bv, samples, rms, centroid, ctx->d_tw, ctx->d_win2048, ctx->d_tw2048,
-                                                   static_cast<float>(static_cast<double>(ctx->sr) / kFeatFft));
-    SPEV_CUDA(cudaGetLastError());
-    return SPEV_OK;
+// ---- host side ---------------------------------------------------------------------------------
+// 0.5 * periodic Hann-2048 as (w[2n], w[2n+1]) pairs and the post-twiddles w2048^k, float64 -> float32
+int features_init(spev_ctx* c) {
+    std::vector<float2> win2048(1024), tw2048(512);
+    for (int n = 0; n < 1024; ++n) {
+        const double w0 = 0.5 - 0.5 * std::cos(2.0 * M_PI * (2 * n) / 2048.0), w1 = 0.5 - 0.5 * std::cos(2.0 * M_PI * (2 * n + 1) / 2048.0);
+        win2048[n] = make_float2(0.5f * static_cast<float>(w0), 0.5f * static_cast<float>(w1));
+    }
+    for (int k = 0; k < 512; ++k) {
+        const double a = -2.0 * M_PI * k / 2048.0;
+        tw2048[k] = make_float2(static_cast<float>(std::cos(a)), static_cast<float>(std::sin(a)));
+    }
+    int rc = upload(&c->d_win2048, win2048);
+    return rc ? rc : upload(&c->d_tw2048, tw2048);
 }
 
-int launch_segment_pool(const float* curve, const int64_t* frame_off, const int64_t* durs, const int64_t* phone_off,
-                        int U, float mu, float sigma, float lo, float hi, int take_log, float log_eps, float* out,
-                        cudaStream_t st) {
+template <bool LOG>
+static int segment_pool(const float* curve, const int64_t* frame_off, const int64_t* durs, const int64_t* phone_off,
+                        int U, float mu, float sigma, float lo, float hi, float log_eps, float* out, cudaStream_t st) {
     SPEV_REQUIRE(U >= 0, SPEV_E_INVALID, "segment_pool: U < 0");
     if (U == 0) return SPEV_OK;
     SPEV_REQUIRE(curve && frame_off && durs && phone_off && out, SPEV_E_INVALID, "segment_pool: null buffer");
     SPEV_REQUIRE(sigma != 0.f, SPEV_E_INVALID, "segment_pool: sigma == 0");
     const int wpb = 4;
     const int grid = std::min((U + wpb - 1) / wpb, 148 * 16);
-    if (take_log)
-        k_segment_pool<true><<<grid, wpb * 32, 0, st>>>(curve, frame_off, reinterpret_cast<const long long*>(durs), phone_off,
-                                                        U, mu, sigma, lo, hi, log_eps, out);
-    else
-        k_segment_pool<false><<<grid, wpb * 32, 0, st>>>(curve, frame_off, reinterpret_cast<const long long*>(durs), phone_off,
-                                                         U, mu, sigma, lo, hi, 0.f, out);
+    k_segment_pool<LOG><<<grid, wpb * 32, 0, st>>>(curve, frame_off, reinterpret_cast<const long long*>(durs), phone_off,
+                                                   U, mu, sigma, lo, hi, log_eps, out);
     SPEV_CUDA(cudaGetLastError());
     return SPEV_OK;
 }
 
 }  // namespace spev
+
+using namespace spev;
+
+extern "C" {
+
+int spev_frame_features(spev_ctx* c, const spev_batch* b, const float* samples, float* rms, float* centroid, void* stream) {
+    SPEV_ON_CTX_DEVICE(c);
+    SPEV_REQUIRE(b, SPEV_E_INVALID, "null ctx or batch");
+    if (b->n_ftiles == 0) return SPEV_OK;
+    SPEV_REQUIRE(samples && rms && centroid && b->ftiles, SPEV_E_INVALID, "frame_features: null buffer");
+    const size_t smem = sizeof(float2) * (1024 + 1024 + 512) + sizeof(spev_tile) * kRing + sizeof(float) * kFeatStage +
+                        sizeof(float) * kWarps * kWarpRegionWords;
+    SPEV_CUDA(cudaFuncSetAttribute(k_frame_features, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    const int grid = std::min<int64_t>(b->n_ftiles, c->num_sms);
+    k_frame_features<<<grid, kThreads, smem, static_cast<cudaStream_t>(stream)>>>(
+        view_of(b), samples, rms, centroid, c->d_tw, c->d_win2048, c->d_tw2048, static_cast<float>(static_cast<double>(c->sr) / kFeatFft));
+    SPEV_CUDA(cudaGetLastError());
+    return SPEV_OK;
+}
+
+int spev_segment_pool(const float* curve, const int64_t* frame_off, const int64_t* durs, const int64_t* phone_off,
+                      int n_items, float mu, float sigma, float lo, float hi, float* out, void* stream) {
+    return segment_pool<false>(curve, frame_off, durs, phone_off, n_items, mu, sigma, lo, hi, 0.f, out,
+                               static_cast<cudaStream_t>(stream));
+}
+
+int spev_segment_pool_log(const float* curve, float log_eps, const int64_t* frame_off, const int64_t* durs,
+                          const int64_t* phone_off, int n_items, float mu, float sigma, float lo, float hi, float* out,
+                          void* stream) {
+    return segment_pool<true>(curve, frame_off, durs, phone_off, n_items, mu, sigma, lo, hi, log_eps, out,
+                              static_cast<cudaStream_t>(stream));
+}
+
+}  // extern "C"

@@ -355,6 +355,7 @@ static float tf32_hi(float x) {
     return x;
 }
 
+// The tf32 hi / residual splits of both B operands: the mel basis zero padded to [n_mels, 520] and pinv [513, n_mels].
 int gemm_tc_init(spev_ctx* c) {
     TcState* st = new TcState();
     c->tma = st;
@@ -363,20 +364,25 @@ int gemm_tc_init(spev_ctx* c) {
     SPEV_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
     SPEV_REQUIRE(fn && qres == cudaDriverEntryPointSuccess, SPEV_E_CUDA, "cuTensorMapEncodeTiled not available");
     st->encode = reinterpret_cast<EncodeTiledFn>(fn);
-    // pinv as the K-major B operand [513, n_mels], split into tf32 hi / residual
     const int nm = c->n_mels;
-    std::vector<float> hi(c->h_pinv.size()), lo(c->h_pinv.size());
-    for (size_t i = 0; i < hi.size(); ++i) { hi[i] = tf32_hi(c->h_pinv[i]); lo[i] = c->h_pinv[i] - hi[i]; }
-    SPEV_CUDA(cudaMalloc(reinterpret_cast<void**>(&c->d_pinv_hi), hi.size() * sizeof(float)));
-    SPEV_CUDA(cudaMalloc(reinterpret_cast<void**>(&c->d_pinv_lo), lo.size() * sizeof(float)));
-    SPEV_CUDA(cudaMemcpy(c->d_pinv_hi, hi.data(), hi.size() * sizeof(float), cudaMemcpyHostToDevice));
-    SPEV_CUDA(cudaMemcpy(c->d_pinv_lo, lo.data(), lo.size() * sizeof(float), cudaMemcpyHostToDevice));
+    std::vector<float> b_hi(static_cast<size_t>(nm) * kSpecLd, 0.f), b_lo(b_hi.size(), 0.f);
+    for (int m = 0; m < nm; ++m)
+        for (int k = 0; k < kBins; ++k) {
+            const float v = c->h_basis[static_cast<size_t>(m) * kBins + k];
+            const size_t i = static_cast<size_t>(m) * kSpecLd + k;
+            b_hi[i] = tf32_hi(v); b_lo[i] = v - b_hi[i];
+        }
+    std::vector<float> p_hi(c->h_pinv.size()), p_lo(c->h_pinv.size());
+    for (size_t i = 0; i < p_hi.size(); ++i) { p_hi[i] = tf32_hi(c->h_pinv[i]); p_lo[i] = c->h_pinv[i] - p_hi[i]; }
+    int rc;
+    if ((rc = upload(&c->d_basis_hi, b_hi)) || (rc = upload(&c->d_basis_lo, b_lo)) || (rc = upload(&c->d_pinv_hi, p_hi)) ||
+        (rc = upload(&c->d_pinv_lo, p_lo)))
+        return rc;
     SPEV_CUDA(cudaFuncSetAttribute(k_gemm_tf32x3<80, EPI_MEL, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    static_cast<int>(TcSmem<80, 3>::kTotal)));
     SPEV_CUDA(cudaFuncSetAttribute(k_gemm_tf32x3<176, EPI_MAG, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    static_cast<int>(TcSmem<176, 1>::kTotal)));
     if (nm % 4 != 0) return SPEV_OK;   // TMA needs 16-byte row pitches; the TC path is then unavailable
-    int rc;
     if ((rc = encode_2d(st, &st->mel_bhi, c->d_basis_hi, nm, kBins, kSpecLd, 80))) return rc;
     if ((rc = encode_2d(st, &st->mel_blo, c->d_basis_lo, nm, kBins, kSpecLd, 80))) return rc;
     if ((rc = encode_2d(st, &st->pinv_bhi, c->d_pinv_hi, kBins, nm, nm, 176))) return rc;
@@ -400,8 +406,30 @@ static int launch_tc(const CUtensorMap& ma, const CUtensorMap& mbh, const CUtens
     return SPEV_OK;
 }
 
-int launch_mel_project_tc(spev_ctx* c, const float* power, int64_t n_frames, float* out, int mode, float floor_v,
-                          float lo, float hi, cudaStream_t stm) {
+// mel [F, n_mels] frame-major (layout 0) -> S [F, ld_s]
+int mel_to_mag_tc(spev_ctx* c, const float* mel, int64_t n_frames, int is_log, float* S, int64_t ld_s, cudaStream_t stm) {
+    TcState* st = static_cast<TcState*>(c->tma);
+    SPEV_REQUIRE(st && st->encode, SPEV_E_UNSUPPORTED, "tensor-core path unavailable");
+    SPEV_REQUIRE(n_frames < (1ll << 31), SPEV_E_INVALID, "mel_to_mag (tc): need ld_s >= 520, multiple of 4");
+    CUtensorMap ma;
+    int rc = encode_2d(st, &ma, mel, static_cast<uint64_t>(n_frames), c->n_mels, c->n_mels, kBM);
+    if (rc) return rc;
+    TcParams p{};
+    p.m_total = static_cast<int>(n_frames); p.k_chunks = (c->n_mels + kBK - 1) / kBK; p.n_valid = kSpecLd; p.ld_out = ld_s;
+    p.a_exp = is_log; p.log_mode = 0;
+    return launch_tc<176, EPI_MAG, 1>(ma, st->pinv_bhi, st->pinv_blo, S, p, 3, stm);
+}
+
+}  // namespace spev
+
+using namespace spev;
+
+extern "C" {
+
+int spev_mel_project(spev_ctx* c, const float* power, int64_t n_frames, float* out, int mode, float floor_v, float lo,
+                     float hi, void* stream) {
+    SPEV_ON_CTX_DEVICE(c);
+    SPEV_REQUIRE(mode == 0 || mode == 1, SPEV_E_INVALID, "spev_mel_project: mode must be 0 or 1");
     TcState* st = static_cast<TcState*>(c->tma);
     SPEV_REQUIRE(st && st->encode, SPEV_E_UNSUPPORTED, "tensor-core path unavailable");
     SPEV_REQUIRE(c->n_mels == 80, SPEV_E_UNSUPPORTED, "spev_mel_project: tensor-core path is built for n_mels=80");
@@ -415,25 +443,7 @@ int launch_mel_project_tc(spev_ctx* c, const float* power, int64_t n_frames, flo
     TcParams p{};
     p.m_total = static_cast<int>(n_frames); p.k_chunks = (kBins + kBK - 1) / kBK; p.n_valid = 80; p.ld_out = 80;
     p.a_exp = 0; p.log_mode = mode; p.floor_v = floor_v; p.lo = lo; p.hi = hi;
-    return launch_tc<80, EPI_MEL, 3>(ma, st->mel_bhi, st->mel_blo, out, p, 1, stm);
+    return launch_tc<80, EPI_MEL, 3>(ma, st->mel_bhi, st->mel_blo, out, p, 1, static_cast<cudaStream_t>(stream));
 }
 
-// mel [F, n_mels] frame-major (layout 0) -> S [F, ld_s]
-int launch_mel_to_mag_tc(spev_ctx* c, const float* mel, int64_t n_frames, int is_log, float* S, int64_t ld_s,
-                         cudaStream_t stm) {
-    TcState* st = static_cast<TcState*>(c->tma);
-    SPEV_REQUIRE(st && st->encode && c->n_mels % 4 == 0, SPEV_E_UNSUPPORTED, "tensor-core path unavailable");
-    SPEV_REQUIRE(n_frames > 0 && n_frames < (1ll << 31) && ld_s >= kSpecLd && ld_s % 4 == 0, SPEV_E_INVALID,
-                 "mel_to_mag (tc): need ld_s >= 520, multiple of 4");
-    SPEV_REQUIRE((reinterpret_cast<uintptr_t>(mel) & 15) == 0 && (reinterpret_cast<uintptr_t>(S) & 15) == 0, SPEV_E_INVALID,
-                 "mel_to_mag (tc): unaligned buffer");
-    CUtensorMap ma;
-    int rc = encode_2d(st, &ma, mel, static_cast<uint64_t>(n_frames), c->n_mels, c->n_mels, kBM);
-    if (rc) return rc;
-    TcParams p{};
-    p.m_total = static_cast<int>(n_frames); p.k_chunks = (c->n_mels + kBK - 1) / kBK; p.n_valid = kSpecLd; p.ld_out = ld_s;
-    p.a_exp = is_log; p.log_mode = 0;
-    return launch_tc<176, EPI_MAG, 1>(ma, st->pinv_bhi, st->pinv_blo, S, p, 3, stm);
-}
-
-}  // namespace spev
+}  // extern "C"

@@ -561,22 +561,62 @@ __global__ void k_pcm16_to_f32(const short* __restrict__ in, int64_t n, float* _
 }
 
 // ---------------------------------------------------------------------------------------
-// launchers
+// host side
 // ---------------------------------------------------------------------------------------
-int launch_pcm16_to_f32(const int16_t* in, int64_t n, float* out, cudaStream_t st) {
-    SPEV_REQUIRE(n >= 0, SPEV_E_INVALID, "pcm16_to_f32: n < 0");
-    if (n == 0) return SPEV_OK;
-    SPEV_REQUIRE(in && out, SPEV_E_INVALID, "pcm16_to_f32: null buffer");
-    const int grid = static_cast<int>(std::min<int64_t>((n / 8 + 255) / 256 + 1, 148 * 16));
-    k_pcm16_to_f32<<<grid, 256, 0, st>>>(reinterpret_cast<const short*>(in), n, out);
+static void fill_clamp(ClampParams& cp, int n_feat, const float* clamp_lo, const float* clamp_hi) {
+    cp.enabled = (n_feat > 0 && clamp_lo && clamp_hi) ? 1 : 0;
+    for (int j = 0; j < kMaxFeat; ++j) {
+        cp.lo[j] = (cp.enabled && j < n_feat) ? clamp_lo[j] : 0.f;
+        cp.hi[j] = (cp.enabled && j < n_feat) ? clamp_hi[j] : 0.f;
+    }
+}
+
+static int grid_for(int64_t n, int block) {
+    return static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((n + block - 1) / block, 148 * 16)));
+}
+
+static int va_bwd_grid(int B, int64_t max_len) {
+    const int64_t tiles = static_cast<int64_t>(B) * ((max_len + kVaFrames - 1) / kVaFrames);
+    return static_cast<int>(std::max<int64_t>(1, std::min<int64_t>(tiles, 148 * 2)));
+}
+
+template <int NF>
+static int launch_va_bwd(const float* grad_out, const float* feats, const ClampParams& cp, const float* conv_w,
+                         const int32_t* cumsum, int B, int T, int H, int64_t max_len, float* grad_cv, float* partials,
+                         int grid, cudaStream_t st) {
+    const int threads = (H + 31) & ~31;
+    const int kF = kVaFrames + 2;
+    const size_t smem = sizeof(int) * (kF + 2) + sizeof(float) * NF * kF + ((NF * kF + 15) & ~15) +
+                        sizeof(float) * 16 * kF + sizeof(float) * kF * (threads / 32) * 16;
+    SPEV_CUDA(cudaFuncSetAttribute(k_variance_fuse_bwd<NF>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    const int tiles_per_row = static_cast<int>((max_len + kVaFrames - 1) / kVaFrames);
+    k_variance_fuse_bwd<NF><<<grid, threads, smem, st>>>(grad_out, feats, cp, conv_w, cumsum, B, T, H, max_len, tiles_per_row,
+                                                         grad_cv, partials);
     SPEV_CUDA(cudaGetLastError());
     return SPEV_OK;
 }
 
-int launch_lr_plan(const void* dur, int dur_dtype, int B, int T, int32_t* cumsum, int64_t* mel_lens,
-                   int64_t* max_len_dev, int64_t* max_len_host, cudaStream_t st) {
+}  // namespace spev
+
+using namespace spev;
+
+extern "C" {
+
+int spev_pcm16_to_f32(const int16_t* pcm, int64_t n, float* out, void* stream) {
+    SPEV_REQUIRE(n >= 0, SPEV_E_INVALID, "pcm16_to_f32: n < 0");
+    if (n == 0) return SPEV_OK;
+    SPEV_REQUIRE(pcm && out, SPEV_E_INVALID, "pcm16_to_f32: null buffer");
+    const int grid = static_cast<int>(std::min<int64_t>((n / 8 + 255) / 256 + 1, 148 * 16));
+    k_pcm16_to_f32<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(reinterpret_cast<const short*>(pcm), n, out);
+    SPEV_CUDA(cudaGetLastError());
+    return SPEV_OK;
+}
+
+int spev_lr_plan(const void* dur, int dur_dtype, int B, int T, int32_t* cumsum, int64_t* mel_lens,
+                 int64_t* max_len_dev, int64_t* max_len_host, void* stream) {
     SPEV_REQUIRE(B >= 0 && T >= 0, SPEV_E_INVALID, "lr_plan: negative shape");
     SPEV_REQUIRE(max_len_dev, SPEV_E_INVALID, "lr_plan: max_len_dev is null");
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
     SPEV_CUDA(cudaMemsetAsync(max_len_dev, 0, sizeof(int64_t), st));
     if (B > 0) {
         SPEV_REQUIRE(mel_lens && (T == 0 || (dur && cumsum)), SPEV_E_INVALID, "lr_plan: null buffer");
@@ -600,9 +640,9 @@ int launch_lr_plan(const void* dur, int dur_dtype, int B, int T, int32_t* cumsum
     return SPEV_OK;
 }
 
-int launch_lr_expand(const void* x, int64_t row_bytes, const float* feats, int n_feat,
-                     const float* clamp_lo, const float* clamp_hi, const int32_t* cumsum, int B, int T,
-                     void* out, float* feats_out, int64_t max_len, cudaStream_t st) {
+int spev_lr_expand_fused(const void* x, int64_t row_bytes, const float* feats, int n_feat,
+                         const float* clamp_lo_host, const float* clamp_hi_host, const int32_t* cumsum,
+                         int B, int T, void* out, float* feats_out, int64_t max_len, void* stream) {
     SPEV_REQUIRE(B >= 0 && T >= 0 && max_len >= 0 && n_feat >= 0 && n_feat <= 16, SPEV_E_INVALID,
                  "lr_expand: bad shape");
     if (B == 0 || max_len == 0) return SPEV_OK;
@@ -611,22 +651,24 @@ int launch_lr_expand(const void* x, int64_t row_bytes, const float* feats, int n
     SPEV_REQUIRE(!x || (out && row_bytes > 0), SPEV_E_INVALID, "lr_expand: x given but out/row_bytes missing");
     SPEV_REQUIRE(n_feat == 0 || (feats && feats_out), SPEV_E_INVALID, "lr_expand: feats buffers missing");
     ClampParams cp;
-    cp.enabled = (n_feat > 0 && clamp_lo && clamp_hi) ? 1 : 0;
-    for (int j = 0; j < kMaxFeat; ++j) {
-        cp.lo[j] = (cp.enabled && j < n_feat) ? clamp_lo[j] : 0.f;
-        cp.hi[j] = (cp.enabled && j < n_feat) ? clamp_hi[j] : 0.f;
-    }
+    fill_clamp(cp, n_feat, clamp_lo_host, clamp_hi_host);
     dim3 grid(static_cast<unsigned>((max_len + kLrFrames - 1) / kLrFrames), static_cast<unsigned>(B));
-    k_lr_expand<<<grid, kLrThreads, 0, st>>>(static_cast<const unsigned char*>(x), row_bytes, feats, n_feat,
-                                             cp, cumsum, B, T, static_cast<unsigned char*>(out),
-                                             feats_out, max_len);
+    k_lr_expand<<<grid, kLrThreads, 0, static_cast<cudaStream_t>(stream)>>>(static_cast<const unsigned char*>(x), row_bytes,
+                                                                            feats, n_feat, cp, cumsum, B, T,
+                                                                            static_cast<unsigned char*>(out), feats_out, max_len);
     SPEV_CUDA(cudaGetLastError());
     return SPEV_OK;
 }
 
-int launch_variance_fuse(const float* x, const float* feats, int n_feat, const float* clamp_lo, const float* clamp_hi,
-                         const float* conv_w, const float* conv_b, const int32_t* cumsum, int B, int T, int H, float* out,
-                         float* feats_out, int64_t max_len, cudaStream_t st) {
+int spev_lr_expand(const void* x, int64_t row_bytes, const int32_t* cumsum, int B, int T, void* out,
+                   int64_t max_len, void* stream) {
+    SPEV_REQUIRE(x && out, SPEV_E_INVALID, "spev_lr_expand: null x/out");
+    return spev_lr_expand_fused(x, row_bytes, nullptr, 0, nullptr, nullptr, cumsum, B, T, out, nullptr, max_len, stream);
+}
+
+int spev_variance_fuse(const float* x, const float* feats, int n_feat, const float* clamp_lo_host, const float* clamp_hi_host,
+                       const float* conv_w, const float* conv_b, const int32_t* cumsum, int B, int T, int H, float* out,
+                       float* feats_out, int64_t max_len, void* stream) {
     SPEV_REQUIRE(B >= 0 && T >= 0 && H > 0 && max_len >= 0 && n_feat >= 0 && n_feat <= kVaMaxFeat, SPEV_E_INVALID,
                  "variance_fuse: bad shape (n_feat <= %d)", kVaMaxFeat);
     if (B == 0 || max_len == 0) return SPEV_OK;
@@ -634,40 +676,27 @@ int launch_variance_fuse(const float* x, const float* feats, int n_feat, const f
     SPEV_REQUIRE(x && out && (T == 0 || cumsum) && (n_feat == 0 || (feats && conv_w && conv_b)), SPEV_E_INVALID,
                  "variance_fuse: null buffer");
     ClampParams cp;
-    cp.enabled = (n_feat > 0 && clamp_lo && clamp_hi) ? 1 : 0;
-    for (int j = 0; j < kMaxFeat; ++j) {
-        cp.lo[j] = (cp.enabled && j < n_feat) ? clamp_lo[j] : 0.f;
-        cp.hi[j] = (cp.enabled && j < n_feat) ? clamp_hi[j] : 0.f;
-    }
+    fill_clamp(cp, n_feat, clamp_lo_host, clamp_hi_host);
     dim3 grid(static_cast<unsigned>((max_len + kVaFrames - 1) / kVaFrames), static_cast<unsigned>(B));
-    k_variance_fuse<<<grid, 256, 0, st>>>(x, feats, n_feat, cp, conv_w, conv_b, cumsum, B, T, H, out, feats_out, max_len);
+    k_variance_fuse<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(x, feats, n_feat, cp, conv_w, conv_b, cumsum, B, T, H,
+                                                                         out, feats_out, max_len);
     SPEV_CUDA(cudaGetLastError());
     return SPEV_OK;
 }
 
-static void fill_clamp(ClampParams& cp, int n_feat, const float* clamp_lo, const float* clamp_hi) {
-    cp.enabled = (n_feat > 0 && clamp_lo && clamp_hi) ? 1 : 0;
-    for (int j = 0; j < kMaxFeat; ++j) {
-        cp.lo[j] = (cp.enabled && j < n_feat) ? clamp_lo[j] : 0.f;
-        cp.hi[j] = (cp.enabled && j < n_feat) ? clamp_hi[j] : 0.f;
-    }
-}
-
-static int grid_for(int64_t n, int block) {
-    return static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((n + block - 1) / block, 148 * 16)));
-}
-
-int launch_lr_expand_backward(const void* grad_out, int dtype, int H, const float* grad_feats_out, int n_feat,
-                              const float* feats, const float* clamp_lo, const float* clamp_hi, const int32_t* cumsum,
-                              int B, int T, int64_t max_len, void* grad_x, float* grad_feats, cudaStream_t st) {
+int spev_lr_expand_backward(const void* grad_out, int dtype, int H, const float* grad_feats_out, int n_feat,
+                            const float* feats, const float* clamp_lo_host, const float* clamp_hi_host,
+                            const int32_t* cumsum, int B, int T, int64_t max_len, void* grad_x, float* grad_feats,
+                            void* stream) {
     SPEV_REQUIRE(B >= 0 && T >= 0 && max_len >= 0 && H >= 0 && n_feat >= 0 && n_feat <= kMaxFeat, SPEV_E_INVALID,
                  "lr_expand_backward: bad shape");
     if (B == 0 || T == 0) return SPEV_OK;
     SPEV_REQUIRE(cumsum, SPEV_E_INVALID, "lr_expand_backward: cumsum is null");
     SPEV_REQUIRE((grad_out == nullptr) == (grad_x == nullptr), SPEV_E_INVALID, "lr_expand_backward: grad_out/grad_x must come together");
     SPEV_REQUIRE(n_feat == 0 || (grad_feats_out && grad_feats), SPEV_E_INVALID, "lr_expand_backward: curve gradients missing");
-    SPEV_REQUIRE(!(clamp_lo && clamp_hi) || n_feat == 0 || feats, SPEV_E_INVALID,
+    SPEV_REQUIRE(!(clamp_lo_host && clamp_hi_host) || n_feat == 0 || feats, SPEV_E_INVALID,
                  "lr_expand_backward: the clamp mask needs the forward's feats");
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (grad_out && H > 0) {
         const int64_t n = static_cast<int64_t>(B) * T * H;
         const bool f4 = dtype == 0 && H % 4 == 0 && (reinterpret_cast<uintptr_t>(grad_out) & 15) == 0 &&
@@ -689,7 +718,7 @@ int launch_lr_expand_backward(const void* grad_out, int dtype, int H, const floa
     }
     if (n_feat > 0) {
         ClampParams cp;
-        fill_clamp(cp, n_feat, clamp_lo, clamp_hi);
+        fill_clamp(cp, n_feat, clamp_lo_host, clamp_hi_host);
         const int64_t n = static_cast<int64_t>(n_feat) * B * T;
         k_lr_curves_bwd<<<grid_for(n, 256), 256, 0, st>>>(grad_feats_out, feats, n_feat, cp, cumsum, B, T, max_len, grad_feats);
         SPEV_CUDA(cudaGetLastError());
@@ -697,60 +726,40 @@ int launch_lr_expand_backward(const void* grad_out, int dtype, int H, const floa
     return SPEV_OK;
 }
 
-static int va_bwd_grid(int B, int64_t max_len) {
-    const int64_t tiles = static_cast<int64_t>(B) * ((max_len + kVaFrames - 1) / kVaFrames);
-    return static_cast<int>(std::max<int64_t>(1, std::min<int64_t>(tiles, 148 * 2)));
-}
-
-size_t variance_fuse_backward_workspace_bytes(int n_feat, int B, int H, int64_t max_len) {
+size_t spev_variance_fuse_backward_workspace_bytes(int n_feat, int B, int H, int64_t max_len) {
     if (n_feat < 0 || B < 0 || H < 0 || max_len < 0) return 0;
     const size_t gcv = static_cast<size_t>(n_feat) * B * max_len * sizeof(float);
     const size_t part = static_cast<size_t>(va_bwd_grid(B, max_len)) * H * (3 * n_feat + 1) * sizeof(float);
     return ((gcv + 255) & ~static_cast<size_t>(255)) + part + 256;
 }
 
-template <int NF>
-static int launch_va_bwd(const float* grad_out, const float* feats, const ClampParams& cp, const float* conv_w,
-                         const int32_t* cumsum, int B, int T, int H, int64_t max_len, float* grad_cv, float* partials,
-                         int grid, cudaStream_t st) {
-    const int threads = (H + 31) & ~31;
-    const int kF = kVaFrames + 2;
-    const size_t smem = sizeof(int) * (kF + 2) + sizeof(float) * NF * kF + ((NF * kF + 15) & ~15) +
-                        sizeof(float) * 16 * kF + sizeof(float) * kF * (threads / 32) * 16;
-    SPEV_CUDA(cudaFuncSetAttribute(k_variance_fuse_bwd<NF>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    const int tiles_per_row = static_cast<int>((max_len + kVaFrames - 1) / kVaFrames);
-    k_variance_fuse_bwd<NF><<<grid, threads, smem, st>>>(grad_out, feats, cp, conv_w, cumsum, B, T, H, max_len, tiles_per_row,
-                                                         grad_cv, partials);
-    SPEV_CUDA(cudaGetLastError());
-    return SPEV_OK;
-}
-
-int launch_variance_fuse_backward(const float* grad_out, const float* feats, int n_feat, const float* clamp_lo,
-                                  const float* clamp_hi, const float* conv_w, const int32_t* cumsum, int B, int T, int H,
-                                  int64_t max_len, float* grad_x, float* grad_feats, float* grad_w, float* grad_b,
-                                  void* workspace, size_t ws_bytes, cudaStream_t st) {
+int spev_variance_fuse_backward(const float* grad_out, const float* feats, int n_feat, const float* clamp_lo_host,
+                                const float* clamp_hi_host, const float* conv_w, const int32_t* cumsum, int B, int T,
+                                int H, int64_t max_len, float* grad_x, float* grad_feats, float* grad_w, float* grad_b,
+                                void* workspace, size_t workspace_bytes, void* stream) {
     SPEV_REQUIRE(B >= 0 && T >= 0 && H > 0 && max_len >= 0 && n_feat >= 0, SPEV_E_INVALID, "variance_fuse_backward: bad shape");
     SPEV_REQUIRE(n_feat <= 5 && H <= 1024, SPEV_E_UNSUPPORTED,
                  "variance_fuse_backward: at most 5 curves and H <= 1024 (got n_feat=%d, H=%d)", n_feat, H);
     if (B == 0 || max_len == 0) return SPEV_OK;
     SPEV_REQUIRE(grad_out && (T == 0 || cumsum), SPEV_E_INVALID, "variance_fuse_backward: null buffer");
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
     int rc = SPEV_OK;
     if (grad_x && T > 0) {
-        rc = launch_lr_expand_backward(grad_out, 0, H, nullptr, 0, nullptr, nullptr, nullptr, cumsum, B, T, max_len, grad_x,
-                                       nullptr, st);
+        rc = spev_lr_expand_backward(grad_out, 0, H, nullptr, 0, nullptr, nullptr, nullptr, cumsum, B, T, max_len, grad_x,
+                                     nullptr, stream);
         if (rc) return rc;
     }
     if (n_feat == 0 || !(grad_feats || grad_w || grad_b)) return SPEV_OK;
     SPEV_REQUIRE(feats && conv_w, SPEV_E_INVALID, "variance_fuse_backward: feats / conv_w missing");
-    SPEV_REQUIRE(workspace && ws_bytes >= variance_fuse_backward_workspace_bytes(n_feat, B, H, max_len), SPEV_E_WORKSPACE,
-                 "variance_fuse_backward: workspace too small (%zu < %zu)", ws_bytes,
-                 variance_fuse_backward_workspace_bytes(n_feat, B, H, max_len));
+    const size_t need = spev_variance_fuse_backward_workspace_bytes(n_feat, B, H, max_len);
+    SPEV_REQUIRE(workspace && workspace_bytes >= need, SPEV_E_WORKSPACE,
+                 "variance_fuse_backward: workspace too small (%zu < %zu)", workspace_bytes, need);
     uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~static_cast<uintptr_t>(255);
     float* grad_cv = reinterpret_cast<float*>(base);
     const size_t gcv = static_cast<size_t>(n_feat) * B * max_len * sizeof(float);
     float* partials = reinterpret_cast<float*>(base + ((gcv + 255) & ~static_cast<size_t>(255)));
     ClampParams cp;
-    fill_clamp(cp, n_feat, clamp_lo, clamp_hi);
+    fill_clamp(cp, n_feat, clamp_lo_host, clamp_hi_host);
     const int grid = va_bwd_grid(B, max_len);
     switch (n_feat) {
         case 1: rc = launch_va_bwd<1>(grad_out, feats, cp, conv_w, cumsum, B, T, H, max_len, grad_cv, partials, grid, st); break;
@@ -776,31 +785,29 @@ int launch_variance_fuse_backward(const float* grad_out, const float* feats, int
     return SPEV_OK;
 }
 
-int launch_duration_rule(const float* ld, int64_t n, float d_control, int64_t* dur, cudaStream_t st) {
+int spev_duration_rule(const float* log_dur, int64_t n, float d_control, int64_t* dur, void* stream) {
     SPEV_REQUIRE(n >= 0, SPEV_E_INVALID, "duration_rule: n < 0");
     if (n == 0) return SPEV_OK;
-    SPEV_REQUIRE(ld && dur, SPEV_E_INVALID, "duration_rule: null buffer");
+    SPEV_REQUIRE(log_dur && dur, SPEV_E_INVALID, "duration_rule: null buffer");
     const int grid = static_cast<int>(std::min<int64_t>((n + 255) / 256, 148 * 8));
-    k_duration_rule<<<grid, 256, 0, st>>>(ld, n, d_control, reinterpret_cast<long long*>(dur));
+    k_duration_rule<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(log_dur, n, d_control, reinterpret_cast<long long*>(dur));
     SPEV_CUDA(cudaGetLastError());
     return SPEV_OK;
 }
 
-int launch_bucketize_embed(const float* v, int64_t n, const float* bnd, int nb, int right,
-                           const float* table, int H, int64_t* idx_out, float* out, int accumulate,
-                           cudaStream_t st) {
-    SPEV_REQUIRE(n >= 0 && nb >= 0 && nb <= 12000, SPEV_E_INVALID, "bucketize: bad sizes (n_boundaries <= 12000)");
+int spev_bucketize_embed(const float* v, int64_t n, const float* boundaries, int n_boundaries, int right,
+                         const float* table, int H, int64_t* idx_out, float* out, int accumulate, void* stream) {
+    SPEV_REQUIRE(n >= 0 && n_boundaries >= 0 && n_boundaries <= 12000, SPEV_E_INVALID, "bucketize: bad sizes (n_boundaries <= 12000)");
     if (n == 0) return SPEV_OK;
-    SPEV_REQUIRE(v && (nb == 0 || bnd), SPEV_E_INVALID, "bucketize: null input");
+    SPEV_REQUIRE(v && (n_boundaries == 0 || boundaries), SPEV_E_INVALID, "bucketize: null input");
     SPEV_REQUIRE(!out || (table && H > 0), SPEV_E_INVALID, "bucketize: out given but table/H missing");
     const int wpb = 8;
     const int64_t groups = (n + 31) / 32;
     const int grid = static_cast<int>(std::min<int64_t>((groups + wpb - 1) / wpb, 148 * 8));
-    k_bucketize_embed<<<grid, wpb * 32, sizeof(float) * nb, st>>>(v, n, bnd, nb, right, table, H,
-                                                                  reinterpret_cast<long long*>(idx_out),
-                                                                  out, accumulate);
+    k_bucketize_embed<<<grid, wpb * 32, sizeof(float) * n_boundaries, static_cast<cudaStream_t>(stream)>>>(
+        v, n, boundaries, n_boundaries, right, table, H, reinterpret_cast<long long*>(idx_out), out, accumulate);
     SPEV_CUDA(cudaGetLastError());
     return SPEV_OK;
 }
 
-}  // namespace spev
+}  // extern "C"

@@ -140,36 +140,69 @@ k_nnls_screen(const float* __restrict__ S, int64_t ld_x, const float* __restrict
     if (lane == 0) { pg_max[col] = pg; value_parts[col] = 0.5 * inv_size * v; }
 }
 
-int launch_nnls_objective(spev_ctx* ctx, const void* x, int x_mode, int64_t ld_x, const float* mel, int is_log, int L,
-                          int64_t T, int64_t t0, int tb, int size_cols, double* value_parts, double* grad, double* pg_max, cudaStream_t st) {
-    SPEV_REQUIRE(ctx && x && mel && value_parts && pg_max, SPEV_E_INVALID, "nnls_objective: null argument");
+// The dense basis both kernels read and the banded view of it the screening kernel walks: per band its run of non-zero
+// bins (first bin, count), then per bin the bands that cover it (first band, last band).
+int nnls_init(spev_ctx* c) {
+    const int n_mels = c->n_mels;
+    const std::vector<float>& basis = c->h_basis;
+    std::vector<int> rng(2 * static_cast<size_t>(n_mels) + 2 * kBins);
+    for (int m = 0; m < n_mels; ++m) {
+        int lo = kBins, hi = -1;
+        for (int k = 0; k < kBins; ++k)
+            if (basis[static_cast<size_t>(m) * kBins + k] != 0.f) { lo = std::min(lo, k); hi = std::max(hi, k); }
+        rng[2 * m] = hi >= lo ? lo : 0;
+        rng[2 * m + 1] = hi >= lo ? hi - lo + 1 : 0;
+    }
+    for (int k = 0; k < kBins; ++k) {
+        int lo = n_mels, hi = -1;
+        for (int m = 0; m < n_mels; ++m)
+            if (basis[static_cast<size_t>(m) * kBins + k] != 0.f) { lo = std::min(lo, m); hi = std::max(hi, m); }
+        rng[2 * n_mels + 2 * k] = hi >= lo ? lo : 0;
+        rng[2 * n_mels + 2 * k + 1] = hi >= lo ? hi : -1;
+    }
+    int rc = upload(&c->d_basis, basis);
+    return rc ? rc : upload(&c->d_nnls_rng, rng);
+}
+
+}  // namespace spev
+
+using namespace spev;
+
+extern "C" {
+
+int spev_nnls_objective(spev_ctx* c, const void* x, int x_mode, int64_t ld_x, const float* mel, int is_log, int L, int64_t T,
+                        int64_t t0, int tb, int size_cols, double* value_parts, double* grad, double* pg_max, void* stream) {
+    SPEV_ON_CTX_DEVICE(c);
+    SPEV_REQUIRE(x_mode >= 0 && x_mode <= 2, SPEV_E_INVALID, "spev_nnls_objective: x_mode must be 0, 1 or 2");
+    SPEV_REQUIRE(x && mel && value_parts && pg_max, SPEV_E_INVALID, "nnls_objective: null argument");
     SPEV_REQUIRE(L > 0 && tb > 0 && t0 >= 0 && t0 + tb <= T, SPEV_E_INVALID, "nnls_objective: bad block [%lld, %lld) of %lld",
                  static_cast<long long>(t0), static_cast<long long>(t0 + tb), static_cast<long long>(T));
     const int x_is_f32_rows = x_mode != 0;            // 1: float64 arithmetic, 2: float32 screening pass
     SPEV_REQUIRE(!x_is_f32_rows || ld_x >= kBins, SPEV_E_INVALID, "nnls_objective: ld_x < 513");
     SPEV_REQUIRE(size_cols >= 0, SPEV_E_INVALID, "nnls_objective: size_cols < 0");
-    const double inv_size = 1.0 / (static_cast<double>(L) * ctx->n_mels * (size_cols > 0 ? size_cols : tb));      // 1 / B.size
-    const size_t smem = sizeof(double) * (kBins + 1 + ctx->n_mels);
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const double inv_size = 1.0 / (static_cast<double>(L) * c->n_mels * (size_cols > 0 ? size_cols : tb));      // 1 / B.size
+    const size_t smem = sizeof(double) * (kBins + 1 + c->n_mels);
     const int grid = L * tb;
-    if (x_mode == 2 && !grad && ctx->d_nnls_rng) {
-        const int n_pad = (ctx->n_mels + 3) & ~3;
+    if (x_mode == 2 && !grad && c->d_nnls_rng) {
+        const int n_pad = (c->n_mels + 3) & ~3;
         const int64_t n_cols = static_cast<int64_t>(L) * tb;
         const size_t sm = sizeof(float) * kScreenWarps * (kScreenX + n_pad);
-        const int2* rng = reinterpret_cast<const int2*>(ctx->d_nnls_rng);
+        const int2* rng = reinterpret_cast<const int2*>(c->d_nnls_rng);
         k_nnls_screen<<<static_cast<unsigned>((n_cols + kScreenWarps - 1) / kScreenWarps), kScreenWarps * 32, sm, st>>>(
-            static_cast<const float*>(x), ld_x, mel, is_log, ctx->d_basis, rng, rng + ctx->n_mels, ctx->n_mels, n_pad, n_cols, T, t0, tb,
+            static_cast<const float*>(x), ld_x, mel, is_log, c->d_basis, rng, rng + c->n_mels, c->n_mels, n_pad, n_cols, T, t0, tb,
             inv_size, value_parts, pg_max);
     } else if (x_mode == 2)
-        k_nnls_objective<1, float><<<grid, kNnlsThreads, smem, st>>>(x, ld_x, mel, is_log, ctx->d_basis, ctx->n_mels, L, T, t0, tb,
+        k_nnls_objective<1, float><<<grid, kNnlsThreads, smem, st>>>(x, ld_x, mel, is_log, c->d_basis, c->n_mels, L, T, t0, tb,
                                                                     inv_size, value_parts, grad, pg_max);
     else if (x_mode == 1)
-        k_nnls_objective<1, double><<<grid, kNnlsThreads, smem, st>>>(x, ld_x, mel, is_log, ctx->d_basis, ctx->n_mels, L, T, t0, tb,
+        k_nnls_objective<1, double><<<grid, kNnlsThreads, smem, st>>>(x, ld_x, mel, is_log, c->d_basis, c->n_mels, L, T, t0, tb,
                                                                      inv_size, value_parts, grad, pg_max);
     else
-        k_nnls_objective<0, double><<<grid, kNnlsThreads, smem, st>>>(x, 0, mel, is_log, ctx->d_basis, ctx->n_mels, L, T, t0, tb,
+        k_nnls_objective<0, double><<<grid, kNnlsThreads, smem, st>>>(x, 0, mel, is_log, c->d_basis, c->n_mels, L, T, t0, tb,
                                                                      inv_size, value_parts, grad, pg_max);
     SPEV_CUDA(cudaGetLastError());
     return SPEV_OK;
 }
 
-}  // namespace spev
+}  // extern "C"

@@ -747,13 +747,6 @@ static double beta_cdf_int(double x, int a, int b) {
     return upper ? 1.0 - s : s;
 }
 
-template <class T>
-static int up(T** dst, const std::vector<T>& src) {
-    SPEV_CUDA(cudaMalloc(reinterpret_cast<void**>(dst), std::max<size_t>(1, src.size()) * sizeof(T)));
-    if (!src.empty()) SPEV_CUDA(cudaMemcpy(*dst, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice));
-    return SPEV_OK;
-}
-
 extern "C" {
 
 int spev_pyin_create(spev_pyin** out, int device, int sr, int hop_length, float fmin, float fmax,
@@ -841,9 +834,9 @@ int spev_pyin_create(spev_pyin** out, int device, int sr, int hop_length, float 
     std::vector<double> logf(nb);
     for (int i = 0; i < nb; ++i) logf[i] = std::log(c->h_freqs[i] + 1e-8);
     int rc;
-    if ((rc = up(&c->d_thresholds, thr)) || (rc = up(&c->d_beta_probs, bp)) || (rc = up(&c->d_beta_cum, bc)) ||
-        (rc = up(&c->d_boltz_exp, bexp)) || (rc = up(&c->d_boltz_fact, bfact)) || (rc = up(&c->d_ltrans, ab)) ||
-        (rc = up(&c->d_freqs, c->h_freqs)) || (rc = up(&c->d_logf, logf))) {
+    if ((rc = upload(&c->d_thresholds, thr)) || (rc = upload(&c->d_beta_probs, bp)) || (rc = upload(&c->d_beta_cum, bc)) ||
+        (rc = upload(&c->d_boltz_exp, bexp)) || (rc = upload(&c->d_boltz_fact, bfact)) || (rc = upload(&c->d_ltrans, ab)) ||
+        (rc = upload(&c->d_freqs, c->h_freqs)) || (rc = upload(&c->d_logf, logf))) {
         spev_pyin_destroy(c);
         return rc;
     }

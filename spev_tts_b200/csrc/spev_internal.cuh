@@ -1,6 +1,7 @@
 // spev_internal.cuh -- ctx layout, error plumbing and launch helpers shared by the .cu files.
 #pragma once
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
@@ -35,17 +36,6 @@ int cuda_fail(cudaError_t e, const char* what);
         }                                                                      \
     } while (0)
 
-// Mel projection of the fused kernels as a per-warp band list built on the host: warp w owns the nb bands
-// hdr[w*nb .. w*nb+nb) (LPT-balanced; unused slots have mel = -1).  A band is a run of float4 weight groups over
-// consecutive bins starting at a multiple of 4: hdr = (first group in gw, first bin, group count, mel index).
-struct MelProgram {
-    int n_mels;
-    int nb;              // bands per warp = ceil(n_mels / 16)
-    int n_groups;        // float4 groups in gw
-    const float4* gw;    // dev [n_groups]
-    const int4* hdr;     // dev [16*nb]
-};
-
 }  // namespace spev
 
 struct spev_ctx {
@@ -59,23 +49,61 @@ struct spev_ctx {
     std::vector<float> h_window;     // [1024]
     // device constants
     float2* d_tw;        // [32*32] exp(-2 pi i k1 l / 1024)
-    float* d_window;     // [1024] periodic Hann
+    float* d_window;     // [1024] periodic Hann, then [256] 1 / window-sum-square of interior ISTFT chunks
     float2* d_win2048;   // [1024] 0.5 * periodic Hann-2048 as (w[2n], w[2n+1])  (features.cu)
     float2* d_tw2048;    // [512]  exp(-2 pi i k / 2048)
     float* d_basis;      // [n_mels, 513] dense float32 basis (NNLS objective)
     int* d_nnls_rng;     // banded view of the basis for the NNLS screening kernel: [n_mels] (first bin, count) then [513] (first band, last band)
-    float* d_basis_pad;  // [n_mels, 520] zero padded (K-major B operand of the mel GEMM)
-    float* d_basis_hi;   // tf32-truncated part, same shape
-    float* d_basis_lo;   // residual, same shape
+    float* d_basis_hi;   // [n_mels, 520] zero padded basis (K-major B operand of the mel GEMM), tf32 hi
+    float* d_basis_lo;   //   residual
     float* d_pinv_t;     // [n_mels, 520]: pinv transposed (pinv_t[m][k] = pinv[k][m])
-    float* d_pinv_hi;    // [528, n_mels_pad]: pinv rows (K-major B operand), tf32 hi
+    float* d_pinv_hi;    // [513, n_mels]: pinv rows (K-major B operand of the mel->magnitude GEMM), tf32 hi
     float* d_pinv_lo;    //   residual
-    float4* d_prog_w;    // mel program of the fused kernel (MelProgram)
+    float4* d_prog_w;    // mel program of the fused kernel (MelProgram, spectral.cu)
     int4* d_prog_h;
-    int prog_gmax;       // most groups any warp runs (diagnostics)
     int prog_nb, prog_groups;
-    int band_nnz;        // nnz of the basis (diagnostics)
-    int band_max_len;
     void* tma;           // opaque: tensor-map cache (gemm_tc.cu)
     int use_tc;          // mel->magnitude on frame-major input uses the tcgen05 GEMM
 };
+
+namespace spev {
+
+// Entry points that take a ctx run on the ctx's device and leave the caller's current device as they found it.
+struct DeviceGuard {
+    int prev = -1, rc = SPEV_OK;
+    explicit DeviceGuard(const spev_ctx* c) {
+        if (!c) { set_error("ctx is null"); rc = SPEV_E_INVALID; return; }
+        cudaError_t e = cudaGetDevice(&prev);
+        if (e == cudaSuccess && prev != c->device) e = cudaSetDevice(c->device); else if (e == cudaSuccess) prev = -1;
+        if (e != cudaSuccess) { rc = cuda_fail(e, "cudaSetDevice(ctx->device)"); prev = -1; }
+    }
+    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
+    DeviceGuard(const DeviceGuard&) = delete;
+    DeviceGuard& operator=(const DeviceGuard&) = delete;
+};
+#define SPEV_ON_CTX_DEVICE(c)      \
+    ::spev::DeviceGuard _guard(c); \
+    if (_guard.rc) return _guard.rc
+
+// Copy a host table to a new device allocation (at least one element, so an empty table still gets a valid pointer).
+template <class T>
+int upload(T** dst, const std::vector<T>& src) {
+    SPEV_CUDA(cudaMalloc(reinterpret_cast<void**>(dst), std::max<size_t>(1, src.size()) * sizeof(T)));
+    if (!src.empty())
+        SPEV_CUDA(cudaMemcpy(*dst, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice));
+    return SPEV_OK;
+}
+
+// Per-file parts of spev_create: each builds and uploads the ctx tables only its own kernels read, from h_basis,
+// h_pinv and h_window.  spev_destroy frees them.
+int spectral_init(spev_ctx* c);
+int gemm_tc_init(spev_ctx* c);
+void gemm_tc_destroy(spev_ctx* c);
+int nnls_init(spev_ctx* c);
+int features_init(spev_ctx* c);
+
+// spev_mel_to_mag on frame-major input (gemm_tc.cu).  The caller has checked n_mels % 4 == 0, n_frames > 0,
+// ld_s >= 520 with ld_s % 4 == 0, and 16-byte aligned mel and S.
+int mel_to_mag_tc(spev_ctx* c, const float* mel, int64_t n_frames, int is_log, float* S, int64_t ld_s, cudaStream_t st);
+
+}  // namespace spev

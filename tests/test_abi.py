@@ -177,3 +177,61 @@ def test_host_entry_points_and_planners_reject_bad_arguments():
     assert lib.spev_create(None, 0, 22050, 1024, 256, 1024, 80, 0.0, 0.0) == -1
     assert lib.spev_logmel(None, None, None, None, 1, 1e-5, -10.0, 2.0, None) == -1             # null ctx
     assert b"ctx is null" in lib.spev_last_error()
+
+
+# One bad call per entry point, each rejected before any CUDA call (so no device is needed): (name, args, rc, message).
+# Dummy non-null pointers (16) stand in for buffers the check never reaches.
+_P = 16
+_NULL_CTX = [
+    ("spev_logmel", (None, None, None, None, 0, 0.0, 0.0, 0.0, None)),
+    ("spev_stft_power", (None, None, None, None, None)),
+    ("spev_mel_project", (None, None, 1, None, 0, 0.0, 0.0, 0.0, None)),
+    ("spev_mel_to_mag", (None, None, None, 0, 0, None, 520, None)),
+    ("spev_nnls_objective", (None, None, 0, 0, None, 0, 1, 1, 0, 1, 0, None, None, None, None)),
+    ("spev_istft", (None, None, None, 520, None, None)),
+    ("spev_stft", (None, None, None, None, 520, None)),
+    ("spev_gl_phase_update", (None, None, None, None, 520, None, None, 520, 0.5, 0, None)),
+    ("spev_griffinlim", (None, None, None, 520, None, 0, 1, 0.99, None, None, 0, None)),
+    ("spev_frame_features", (None, None, None, None, None, None)),
+    ("spev_set_sm_limit", (None, 0)),
+    ("spev_set_tensor_core", (None, 1)),
+]
+_BAD_CALLS = [(name, args, -1, b"ctx is null") for name, args in _NULL_CTX] + [
+    ("spev_transpose_batched", (_P, _P, 4, 1, -1, 4, 4, 16, 4, 16, None), -1, b"transpose: negative shape"),
+    ("spev_transpose_batched", (_P, _P, 3, 1, 4, 4, 4, 16, 4, 16, None), -2, b"4- or 8-byte elements only"),
+    ("spev_collate", (_P, 13, _P, _P, None, 2, 4, 4, None), -1, b"at most 12 arrays"),
+    ("spev_copy_segments", (_P, _P, _P, _P, _P, _P, -1, 1, None), -1, b"copy_segments: negative sizes"),
+    ("spev_segment_pool", (_P, _P, _P, _P, 2, 0.0, 0.0, -3.0, 3.0, _P, None), -1, b"segment_pool: sigma == 0"),
+    ("spev_segment_pool_log", (_P, 1e-5, _P, _P, _P, 2, 0.0, 0.0, -3.0, 3.0, _P, None), -1,
+     b"segment_pool: sigma == 0"),
+    ("spev_lr_plan", (_P, 0, -1, 4, _P, _P, _P, None, None), -1, b"lr_plan: negative shape"),
+    ("spev_lr_expand", (None, 16, _P, 2, 4, _P, 8, None), -1, b"spev_lr_expand: null x/out"),
+    ("spev_lr_expand_fused", (_P, 16, _P, 17, None, None, _P, 2, 4, _P, _P, 8, None), -1, b"lr_expand: bad shape"),
+    ("spev_pcm16_to_f32", (_P, -1, _P, None), -1, b"pcm16_to_f32: n < 0"),
+    ("spev_variance_fuse", (_P, _P, 1, None, None, _P, _P, _P, 2, 4, 0, _P, _P, 8, None), -1,
+     b"variance_fuse: bad shape"),
+    ("spev_lr_expand_backward", (_P, 0, 4, None, 0, None, None, None, _P, -1, 4, 8, _P, None, None), -1,
+     b"lr_expand_backward: bad shape"),
+    ("spev_variance_fuse_backward", (_P, _P, 6, None, None, _P, _P, 2, 4, 8, 8, _P, _P, _P, _P, _P, 1 << 20, None),
+     -2, b"at most 5 curves"),
+    ("spev_duration_rule", (_P, -1, 1.0, _P, None), -1, b"duration_rule: n < 0"),
+    ("spev_bucketize_embed", (_P, 8, _P, 12001, 0, None, 0, _P, None, 0, None), -1, b"n_boundaries <= 12000"),
+]
+
+
+@pytest.mark.parametrize("name,args,rc,msg", _BAD_CALLS, ids=[f"{c[0]}-{i}" for i, c in enumerate(_BAD_CALLS)])
+def test_entry_points_reject_bad_arguments_before_any_cuda_call(name, args, rc, msg):
+    import spev_tts_b200 as sp
+    lib = sp.load()
+    assert getattr(lib, name)(*args) == rc
+    assert msg in lib.spev_last_error()
+
+
+def test_workspace_queries_and_piece_size():
+    import spev_tts_b200 as sp
+    lib = sp.load()
+    assert lib.spev_griffinlim_workspace_bytes(-1) == 0
+    for bad in ((-1, 2, 8, 8), (1, -1, 8, 8), (1, 2, -1, 8), (1, 2, 8, -1)):
+        assert lib.spev_variance_fuse_backward_workspace_bytes(*bad) == 0
+    assert lib.spev_variance_fuse_backward_workspace_bytes(1, 2, 8, 8) > 0
+    assert lib.spev_copy_segments_piece_bytes() == 16384
