@@ -236,9 +236,11 @@ SPEV_API int spev_frame_features(spev_ctx* ctx, const spev_batch* batch, const f
 
 /* Per-phoneme pooling of a frame-level curve: for phoneme p of item i with duration d_p frames,
  *   out[p] = clamp((mean(curve[frame_off[i] + start_p .. + d_p)) - mu) / sigma, lo, hi)
- * where start_p is the running sum of the item's earlier durations.  durs: dev int64 flat, item i
- * owns [phone_off[i], phone_off[i+1]).  Replaces the e / bri (and, with mu=1, sigma=-1, br) lines of
- * the per-phone loop, spev_real_metrics.py:400-417. */
+ * where start_p is the running sum of the item's earlier durations.  The mean covers only the phone's
+ * frames inside the item (numpy's mean of the slice cut at the item's end); a phone with no frame there
+ * (duration 0, or starting at or after the item's end) gives NaN.  Negative durations count as 0.
+ * durs: dev int64 flat, item i owns [phone_off[i], phone_off[i+1]).  Replaces the e / bri (and, with
+ * mu=1, sigma=-1, br) lines of the per-phone loop, spev_real_metrics.py:400-417. */
 SPEV_API int spev_segment_pool(const float* curve, const int64_t* frame_off, const int64_t* durs,
                                const int64_t* phone_off, int n_items, float mu, float sigma, float lo, float hi,
                                float* out, void* stream);
@@ -409,6 +411,8 @@ SPEV_API int spev_pyin_decode(spev_pyin* ctx, const float* logobs, const float* 
  *   f0_log = log(f0 + 1e-8) on voiced frames (state < n_bins); unvoiced frames are masked (the reference's
  *   log(1e-8 + 1e-8) < -5 test);  pitch[p] = clip((mean - p_mean) / p_std, lo, hi), or clip(0) without voiced
  *   frames;  rough[p] = clip(population std, 0, rough_hi), 0 without voiced frames.
+ *   Only the phone's frames inside the item count: a phone past the item's end has no voiced frame there.
+ *   Negative durations count as 0.
  *   states int32 [F]; frame_off / phone_off int64 [n_items+1]; durs int64 [P]; pitch, rough f32 [P]. */
 SPEV_API int spev_pitch_pool(const spev_pyin* ctx, const int32_t* states, const int64_t* frame_off, const int64_t* durs,
                              const int64_t* phone_off, int n_items, double p_mean, double p_std, float lo, float hi,

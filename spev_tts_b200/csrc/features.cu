@@ -10,7 +10,9 @@
 //     __shfl_sync (fetch_mirror).  Only two scalars per frame leave the SM.
 // K10 k_segment_pool   : per phoneme p with duration d_p (frames): clip((mean(curve[seg_p]) - mu) /
 //     sigma, lo, hi) -- the e / bri (and, with mu=1, sigma=-1, the br) lines of :400-417.  One warp
-//     per utterance: warp-scan of the durations, then one lane per phoneme.
+//     per utterance: warp-scan of the durations, then one lane per phoneme.  The mean covers the
+//     phone's frames inside the item (numpy's slice); a phone with none gives NaN.  Negative
+//     durations count as 0.
 #include <algorithm>
 #include <cmath>
 #include "spev_internal.cuh"
@@ -152,11 +154,12 @@ __global__ void k_segment_pool(const float* __restrict__ curve, const int64_t* _
             if (p < p1) {
                 float acc = 0.f;
                 const long long end = min(static_cast<long long>(T), start + dd);
+                const long long n = max(0LL, end - start);   // frames of the phone inside the item
                 for (long long t = start; t < end; ++t) acc += LOG ? logf(c[t] + log_eps) : c[t];
-                // numpy: mean of an empty slice is NaN
-                const float m = dd > 0 ? acc / static_cast<float>(dd) : __int_as_float(0x7fc00000);
+                // numpy: the mean of a slice cut at the item's end; the mean of an empty slice is NaN
+                const float m = n > 0 ? acc / static_cast<float>(n) : __int_as_float(0x7fc00000);
                 // np.clip propagates the NaN of an empty phone; fminf/fmaxf would swallow it
-                out[p] = dd > 0 ? fminf(fmaxf((m - mu) / sigma, lo), hi) : m;
+                out[p] = n > 0 ? fminf(fmaxf((m - mu) / sigma, lo), hi) : m;
             }
             carry += __shfl_sync(0xffffffffu, incl, 31);
         }
